@@ -1,6 +1,6 @@
 """Golden vectors of BSS Eval v4 and the ideal-mask systems, produced by RUNNING THE REFERENCE ITSELF
-(/root/reference/bsseval_v4.py, /root/reference/oracle_systems.py: pure numpy / scipy, importable here with the
-``np.float`` alias that NumPy >= 1.24 removed).  Run in the build container:  python tests/golden/make_bsseval_golden.py
+(bsseval_v4.py, oracle_systems.py of SamArgt/AudioSourceSep: pure numpy / scipy, importable with the ``np.float``
+alias that NumPy >= 1.24 removed).   python tests/golden/make_bsseval_golden.py <reference checkout>
 """
 import os
 import sys
@@ -9,7 +9,7 @@ import types
 import numpy as np
 
 np.float = float                                      # bsseval_v4.py:507, oracle_systems.py use the removed alias
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, sys.argv[1])
 import bsseval_v4 as bv  # noqa: E402
 
 HERE = os.path.dirname(os.path.abspath(__file__))

@@ -7,15 +7,20 @@ GPU tests compare against these committed vectors instead of re-running the orac
 NOT stored: the tests regenerate them from the same seeded generators (audiosourcesep_b200.synthetic,
 weights.init_glow_params), so a drift of either generator fails the test loudly.
 
-    python tests/golden/make_glow_k40_golden.py            (build container, ~45 min on 8 cores)
+    python tests/golden/make_glow_k40_golden.py            (CPU, ~45 min on 8 cores)
 
-Writes tests/golden/glow_k40.npz:
-  grad1, grad2  float32 [30,96,64]   oracle (float64) grad_log_prob of prior 1 at x1 / prior 2 at x2
+Writes tests/golden/glow_k40.npz, a fixed sample of the oracle outputs that keeps the file under 1 MB:
+  keep          uint8 packbits of a bool [30,96,64] mask: a seeded half of the score elements (every patch, row
+                and column is represented)
+  grad1, grad2  float32 [keep.sum()] oracle (float64) grad_log_prob of prior 1 at x1 / prior 2 at x2, at the
+                                      elements of ``keep`` in C order
   logp1, logp2  float64 [30]         oracle (float64) log_prob
-  traj_x1, traj_x2  float32 [11,2,96,64]  oracle (float32, "as-TF") Langevin states of the first 2 segments at the
-                                      LAST noise level (sigma index 9) after 0,10,...,100 steps with injected noise
+  traj_steps    int64 [2]            50, 100
+  traj_x1, traj_x2  float32 [2,2,96,64]  oracle (float32, "as-TF") Langevin states of the first 2 segments at the
+                                      LAST noise level (sigma index 9) after ``traj_steps`` steps with injected noise
                                       (run_basis_sep.py:152-181)
-Seeds: weights 2 / 3 (mode "perturbed"), problem seeds 0 / 1, Langevin init 4, noise Generator(PCG64(3)).
+Seeds: weights 2 / 3 (mode "perturbed"), problem seeds 0 / 1, Langevin init 4, noise Generator(PCG64(3)),
+score sample Generator(PCG64(0)).
 """
 import os
 import sys
@@ -46,6 +51,15 @@ def problem():
 def traj_noise():
     rng = np.random.Generator(np.random.PCG64(3))
     return rng.standard_normal((T, 2, N_TRAJ, 96, 64, 1)).astype(np.float32)
+
+
+def sample(full):
+    """The stored subset of the full outputs: half of the score elements, the trajectory after 50 and 100 steps."""
+    keep = np.random.Generator(np.random.PCG64(0)).random(full["grad1"].shape) < 0.5
+    steps = np.array([50, 100])
+    return {"keep": np.packbits(keep), "grad1": full["grad1"][keep], "grad2": full["grad2"][keep],
+            "logp1": full["logp1"], "logp2": full["logp2"], "traj_steps": steps,
+            "traj_x1": full["traj_x1"][steps // 10], "traj_x2": full["traj_x2"][steps // 10]}
 
 
 def main():
@@ -79,6 +93,7 @@ def main():
             t2s.append(b[..., 0].copy())
             print(f"trajectory step {t + 1}, {time.time() - t0:.0f} s", flush=True)
     out["traj_x1"], out["traj_x2"] = np.stack(t1s), np.stack(t2s)
+    out = sample(out)
     np.savez_compressed(os.path.join(HERE, "glow_k40.npz"), **out)
     print("written", {k: v.shape for k, v in out.items()})
 

@@ -1,7 +1,5 @@
-"""Regenerates the fixtures of tests/golden/ from the READ-ONLY reference tree.
-
-Run in the build container only (``/root/reference`` does not exist on the GPU box):
-    python tests/golden/make_golden.py
+"""Regenerates the fixtures of tests/golden/ from a READ-ONLY checkout of the reference (SamArgt/AudioSourceSep):
+    python tests/golden/make_golden.py <reference checkout>
 Produces
   sigmas_v1.json     the noise schedule printed by the reference's own BASIS run
                      (basis_sep_results/beethoven_sonata_1_sep_1min/out.log:44-116)
@@ -13,15 +11,15 @@ Produces
 import json
 import os
 import re
+import sys
 
 import numpy as np
 
-REF = "/root/reference"
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
-def main():
-    run = os.path.join(REF, "basis_sep_results", "beethoven_sonata_1_sep_1min")
+def main(ref):
+    run = os.path.join(ref, "basis_sep_results", "beethoven_sonata_1_sep_1min")
     sig = []
     dur = None
     with open(os.path.join(run, "out.log")) as f:
@@ -38,7 +36,7 @@ def main():
                    "printed": sig, "duration_s": dur, "n_mixed": 30, "T": 100}, f, indent=1)
     d = np.load(os.path.join(run, "results.npz"))
     np.savez_compressed(os.path.join(HERE, "real_patches.npz"), **{k: d[k][:4] for k in ("gt1", "gt2", "mixed", "x1", "x2")})
-    with open(os.path.join(REF, "trained_ncsn", "ncsn_piano_192_32_dB_custom_loop", "out.log")) as f:
+    with open(os.path.join(ref, "trained_ncsn", "ncsn_piano_192_32_dB_custom_loop", "out.log")) as f:
         txt = f.read()
     m = re.search(r"([0-9][0-9,]{6,})", txt.split("\n")[34])
     with open(os.path.join(HERE, "param_counts.json"), "w") as f:
@@ -48,4 +46,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

@@ -1,5 +1,5 @@
 """GPU parity tests of BSS Eval v4 and the ideal masks against outputs of THE REFERENCE ITSELF
-(tests/golden/bsseval_v4.npz, written by tests/golden/make_bsseval_golden.py from /root/reference/bsseval_v4.py and
+(tests/golden/bsseval_v4.npz, written by tests/golden/make_bsseval_golden.py from the reference's bsseval_v4.py and
 oracle_systems.py) -- a reference-pinned oracle, not a restatement."""
 import os
 

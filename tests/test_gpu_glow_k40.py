@@ -2,7 +2,8 @@
 
 The oracle side is the committed fixture tests/golden/glow_k40.npz (generator: tests/golden/make_glow_k40_golden.py;
 one float64 oracle gradient of 30 patches costs minutes of CPU, a T=100 trajectory 200 evaluations).  The inputs are
-regenerated here from the same seeded generators, so the comparison is CUDA-vs-oracle on identical inputs.
+regenerated here from the same seeded generators, so the comparison is CUDA-vs-oracle on identical inputs.  The GPU
+computes every patch; scores are compared on the fixture's fixed half of the elements (``keep``).
 
 Reference: run_basis_sep.py:73-79 (compute_grad_logprob), :152-181 (basis_inner_loop), :478 (n_mixed = 30).
 Gates (BASELINE.json north_star): per-Langevin-step state relative error <= 1e-3, final SDR within 0.1 dB.
@@ -40,7 +41,8 @@ def problem():
     mixed, gt1, gt2 = synthetic.basis_problem(N_MIXED)
     x1, x2 = synthetic.langevin_init(N_MIXED, seed=4)
     gold = np.load(GOLD)
-    return dict(cfg=cfg, p1=p1, p2=p2, mixed=mixed, gt1=gt1, gt2=gt2, x1=x1, x2=x2, gold=gold)
+    keep = np.unpackbits(gold["keep"], count=N_MIXED * 96 * 64).reshape(N_MIXED, 96, 64).astype(bool)
+    return dict(cfg=cfg, p1=p1, p2=p2, mixed=mixed, gt1=gt1, gt2=gt2, x1=x1, x2=x2, gold=gold, keep=keep)
 
 
 _models = {}
@@ -65,14 +67,16 @@ GRAD_BOUND = {"fp32": 2e-3, "bf16": 0.1, "bf16x2": 0.1, "fp16x2": 0.08, "fp16x3"
 @pytest.mark.parametrize("precision", ["fp32", "bf16", "bf16x2", "fp16x2", "fp16x3"])
 def test_grad_log_prob_k40_n30_vs_oracle(problem, precision):
     m1, m2 = _pair(problem, precision)
-    gold = problem["gold"]
+    gold, keep = problem["gold"], problem["keep"]
     for k, (m, x) in enumerate(((m1, problem["x1"]), (m2, problem["x2"])), start=1):
         g, lp = m.grad_log_prob(torch.as_tensor(x), return_log_prob=True)
         g = _np(g)[..., 0].astype(np.float64)
-        ref = gold[f"grad{k}"].astype(np.float64)
+        ref = np.zeros_like(g)
+        ref[keep] = gold[f"grad{k}"]
         assert np.all(np.isfinite(g))
-        rel = np.linalg.norm(g - ref) / np.linalg.norm(ref)
-        per = np.linalg.norm((g - ref).reshape(N_MIXED, -1), axis=1) / np.linalg.norm(ref.reshape(N_MIXED, -1), axis=1)
+        err = np.where(keep, g - ref, 0.0)
+        rel = np.linalg.norm(err) / np.linalg.norm(ref)
+        per = np.linalg.norm(err.reshape(N_MIXED, -1), axis=1) / np.linalg.norm(ref.reshape(N_MIXED, -1), axis=1)
         dlp = np.max(np.abs(_np(lp).astype(np.float64) - gold[f"logp{k}"])) / problem["cfg"].dims
         print(f"[{precision}] prior {k}: K=40 N=30 score rel L2 err {rel:.3e} (worst patch {per.max():.3e}); "
               f"log_prob err {dlp:.3e} nats/dim")
@@ -105,17 +109,21 @@ def test_one_langevin_step_k40_n30_vs_oracle(problem, precision, sigma_idx):
     g, grad_g = bo.mixing_process("melspec", "dB")
     rng = np.random.Generator(np.random.PCG64(100 + sigma_idx))
     n1, n2 = (rng.standard_normal(problem["x1"].shape).astype(np.float32) for _ in range(2))
-    s1, s2 = gold["grad1"][..., None], gold["grad2"][..., None]
-    y1, y2 = bo.langevin_update(problem["x1"], problem["x2"], s1, s2, problem["mixed"], n1, n2, eta, lam, ns, g, grad_g)
+    # the update is element-wise: the expected state is known wherever the oracle score is stored
+    keep = problem["keep"][..., None]
+    x1, x2 = problem["x1"][keep], problem["x2"][keep]
+    y1, y2 = bo.langevin_update(x1, x2, gold["grad1"], gold["grad2"], problem["mixed"][keep], n1[keep], n2[keep],
+                                eta, lam, ns, g, grad_g)
     t1, t2 = torch.as_tensor(problem["x1"]).cuda(), torch.as_tensor(problem["x2"]).cuda()
     nan = torch.zeros(1, dtype=torch.int32, device="cuda")
     ops.basis_glow_inner(m1, m2, torch.as_tensor(problem["mixed"]), t1, t2, 1, float(eta), float(lam), float(ns),
                          noise1=torch.as_tensor(n1[None]), noise2=torch.as_tensor(n2[None]), nan_count=nan)
     worst = 0.0
-    for got, want, x0 in ((t1, y1, problem["x1"]), (t2, y2, problem["x2"])):
-        rel = float(np.linalg.norm(_np(got) - want) / np.linalg.norm(want))
+    for got, want, x0 in ((t1, y1, x1), (t2, y2, x2)):
+        got = _np(got)[keep]
+        rel = float(np.linalg.norm(got - want) / np.linalg.norm(want))
         # the same error relative to the size of the update itself (how much of the STEP is right)
-        upd = float(np.linalg.norm(_np(got) - want) / np.linalg.norm(want - x0))
+        upd = float(np.linalg.norm(got - want) / np.linalg.norm(want - x0))
         worst = max(worst, rel)
         print(f"[{precision}, sigma_idx={sigma_idx}] state rel err {rel:.3e}; relative to the update {upd:.3e}")
     assert nan.item() == 0
@@ -145,10 +153,10 @@ def test_t100_last_sigma_sdr_vs_oracle(problem, precision):
     for k, (got, key) in enumerate(((t1, "traj_x1"), (t2, "traj_x2"))):
         want = gold[key][-1]
         rel = float(np.linalg.norm(_np(got)[..., 0] - want) / np.linalg.norm(want))
-        drift = [float(np.linalg.norm(_np(dump[10 * i - 1, k])[..., 0] - gold[key][i]) / np.linalg.norm(gold[key][i]))
-                 for i in range(1, 11)]
+        drift = [float(np.linalg.norm(_np(dump[step - 1, k])[..., 0] - w) / np.linalg.norm(w))
+                 for step, w in zip(gold["traj_steps"], gold[key])]
         sdr_c, sdr_o = bo.sdr_db(gts[k], _np(got)[..., 0]), bo.sdr_db(gts[k], want)
-        print(f"[{precision}] source {k + 1}: final state rel err {rel:.3e} (every 10 steps: "
+        print(f"[{precision}] source {k + 1}: final state rel err {rel:.3e} (after steps {gold['traj_steps'].tolist()}: "
               f"{', '.join(f'{d:.1e}' for d in drift)}); SDR cuda {sdr_c:.4f} dB, oracle {sdr_o:.4f} dB")
         assert abs(sdr_c - sdr_o) <= 0.1, (sdr_c, sdr_o)
         assert rel <= 5e-3, rel
