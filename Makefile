@@ -3,7 +3,7 @@ NVCC      ?= /usr/local/cuda/bin/nvcc
 ARCH      := -gencode arch=compute_100a,code=sm_100a
 NVCCFLAGS := -O3 -std=c++17 -lineinfo $(ARCH) -Xcompiler -fPIC -Xcompiler -Wall -Iinclude --expt-relaxed-constexpr
 CSRC      := audiosourcesep_b200/csrc
-SRCS      := $(CSRC)/api.cu $(CSRC)/flow_kernels.cu $(CSRC)/langevin.cu $(CSRC)/nn_fp32.cu $(CSRC)/nn_tc.cu $(CSRC)/nn_tcx.cu $(CSRC)/glow_model.cu $(CSRC)/conv_tc.cu $(CSRC)/ncsn_kernels.cu $(CSRC)/ncsn_model.cu $(CSRC)/train_kernels.cu $(CSRC)/glow_train.cu $(CSRC)/wgrad_tc.cu $(CSRC)/ncsn_train_kernels.cu $(CSRC)/conv_wgrad_tc.cu $(CSRC)/ncsn_train.cu $(CSRC)/bsseval.cu $(CSRC)/mel_kernels.cu
+SRCS      := $(CSRC)/api.cu $(CSRC)/flow_kernels.cu $(CSRC)/langevin.cu $(CSRC)/nn_fp32.cu $(CSRC)/nn_tc.cu $(CSRC)/nn_tcx.cu $(CSRC)/glow_model.cu $(CSRC)/conv_tc.cu $(CSRC)/ncsn_kernels.cu $(CSRC)/ncsn_model.cu $(CSRC)/train_kernels.cu $(CSRC)/glow_train.cu $(CSRC)/wgrad_tc.cu $(CSRC)/ncsn_train_kernels.cu $(CSRC)/conv_wgrad_tc.cu $(CSRC)/ncsn_train.cu $(CSRC)/bsseval.cu $(CSRC)/mel_kernels.cu $(CSRC)/resample_kernels.cu
 OBJS      := $(SRCS:.cu=.o)
 LIB       := audiosourcesep_b200/libasep.so
 

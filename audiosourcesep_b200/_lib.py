@@ -127,6 +127,7 @@ _SIGNATURES = {
     "asep_stft_filter": [_P, _P, _P, _I, _V],
     "asep_istft": [_P, _I, _P, _V],
     "asep_griffinlim_update": [_P, _P, _P, _P, _F, _V],
+    "asep_resample": [_P, _P, _P, _P, ctypes.c_double, _I, _P, _V],
     "asep_basis_graphs": [_I],
     "asep_hbm_profile": [_I],
     "asep_hbm_profile_read": [_I, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_int64),

@@ -10,6 +10,7 @@
 #include "glow_model.h"
 #include "mel_kernels.h"
 #include "ncsn_model.h"
+#include "resample_kernels.h"
 
 namespace asep {
 
@@ -1192,6 +1193,27 @@ int asep_istft(const DLTensor* stft, int hop, DLTensor* audio, void* stream) {
     throw;
   }
   CUDA_CHECK(cudaFreeAsync(frames, s));
+  ASEP_API_END
+}
+
+// ------------------------------------------------------------------ resampling (resample_kernels.cu)
+int asep_resample(const DLTensor* audio, const DLTensor* time, const DLTensor* win, const DLTensor* delta, double scale, int step,
+                  DLTensor* out, void* stream) {
+  ASEP_API_BEGIN
+  ASEP_CHECK(g_device >= 0, ASEP_ERR_STATE, "asep_init() has not been called");
+  TView a = view_f32(audio, "audio", g_device), o = view_f32(out, "out", g_device);
+  TView tv = view_any(time, "time", g_device, false, kDLFloat, 64);
+  TView w = view_f32(win, "win", g_device), d = view_f32(delta, "delta", g_device);
+  ASEP_CHECK(a.ndim == 2, ASEP_ERR_BAD_SHAPE, "audio must be [N, L_in]");
+  ASEP_CHECK(tv.ndim == 1, ASEP_ERR_BAD_SHAPE, "time must be [L_out]");
+  ASEP_CHECK(w.ndim == 1 && w.numel >= 1, ASEP_ERR_BAD_SHAPE, "win must be a non-empty [nwin]");
+  expect_shape(d, "delta", {w.numel});
+  expect_shape(o, "out", {a.shape[0], tv.numel});
+  ASEP_CHECK(step >= 1, ASEP_ERR_BAD_ARG, "step must be >= 1 (got %d)", step);
+  ASEP_CHECK(scale > 0.0 && scale <= 1.0, ASEP_ERR_BAD_ARG, "scale must be in (0, 1] (got %g)", scale);
+  ASEP_CHECK(w.numel <= INT32_MAX && a.shape[0] <= INT32_MAX, ASEP_ERR_UNSUPPORTED, "resample: table or batch too large");
+  launch_resample(a.f32, static_cast<const double*>(tv.raw), w.f32, d.f32, o.f32, (int)a.shape[0], (long long)a.shape[1],
+                  (long long)tv.numel, (int)w.numel, scale, step, as_stream(stream));
   ASEP_API_END
 }
 

@@ -62,11 +62,44 @@ def synthetic_dataset(n: int, seed: int, H: int, W: int) -> np.ndarray:
     return synthetic.mel_patches_db(n, seed, H, W)
 
 
-def train(flow, optimizer, data: np.ndarray, args, sigma: float = 0.0, log=print, step_offset: int = 0):
+def held_out_mean(test: np.ndarray, batch: int, per_sample_loss) -> float:
+    """Mean of ``per_sample_loss(x, first)`` (a device vector of losses of the test patches ``x`` whose first global
+    index is ``first``) over every test patch.  Each rank evaluates one contiguous shard in chunks of ``batch``; the
+    float64 sums are all-reduced, so every rank returns the same value."""
+    world = dist.get_world_size() if dist.is_initialized() else 1
+    rank = dist.get_rank() if dist.is_initialized() else 0
+    n = test.shape[0]
+    lo, hi = rank * n // world, (rank + 1) * n // world
+    total = torch.zeros((1,), dtype=torch.float64, device=torch.device("cuda", torch.cuda.current_device()))
+    for c0 in range(lo, hi, max(1, int(batch))):
+        x = torch.as_tensor(test[c0: min(c0 + int(batch), hi)]).to(total.device)
+        total += per_sample_loss(x, c0).double().sum()
+    if world > 1:
+        dist.all_reduce(total, op=dist.ReduceOp.SUM)
+    return float(total.item()) / n
+
+
+def held_out_nll(flow, test: np.ndarray, batch: int, sigma: float = 0.0, seed: int = 0) -> float:
+    """Mean -log_prob over the test patches, the units of the train loss; at a noise level ``sigma`` the patches are
+    perturbed by sigma * N(0, 1) in raw data units, drawn from a fixed Philox key (seed, global sample index), so the
+    test loss of successive epochs is evaluated on the same perturbation."""
+    from . import ops
+
+    def nll(x, first):
+        if sigma > 0.0:
+            per = int(np.prod(x.shape[1:]))
+            x = x + float(sigma) * ops.philox_normal(tuple(x.shape), seed=seed, step=0, stream_id=4, elem_offset=first * per)
+        return -flow.log_prob(x)
+    return held_out_mean(test, batch, nll)
+
+
+def train(flow, optimizer, data: np.ndarray, args, sigma: float = 0.0, log=print, step_offset: int = 0,
+          test: Optional[np.ndarray] = None):
     """Epoch loop over a host dataset (reference: train_glow.py:88-181 without the TensorBoard / sample-grid side
     outputs); stops on a NaN / Inf loss like train_glow.py:115-118.  ``step_offset``: global step of the first
     iteration -- the noise of train_noisy_glow is keyed by (seed, global step, global sample), so successive calls
-    (one per noise level) must continue the count instead of redrawing the same sequence."""
+    (one per noise level) must continue the count instead of redrawing the same sequence.  ``test``: held-out patches;
+    when non-empty, ``Epoch NNN: Test Loss: ...`` (:func:`held_out_nll`) is logged after every epoch."""
     world = dist.get_world_size() if dist.is_initialized() else 1
     rank = dist.get_rank() if dist.is_initialized() else 0
     gb = int(args.batch_size)
@@ -93,6 +126,9 @@ def train(flow, optimizer, data: np.ndarray, args, sigma: float = 0.0, log=print
                 return history
             step += 1
         log("Epoch {:03d}: loss = {:.4f}  ({:.1f} s)".format(epoch, history[-1], time.time() - t0))
+        if test is not None and test.shape[0] > 0:
+            tl = held_out_nll(flow, test, local, sigma=sigma, seed=int(getattr(args, "seed", 0)))
+            log("Epoch {:03d}: Test Loss: {:.6f}".format(epoch, tl))
     return history
 
 
@@ -100,7 +136,10 @@ def build_parser():
     p = argparse.ArgumentParser(description="Train Glow (data-parallel, one process per GPU)")
     p.add_argument("--config", type=str, default=None)
     p.add_argument("--output", type=str, default="trained_glow")
-    p.add_argument("--n_train", type=int, default=256, help="synthetic training patches")
+    p.add_argument("--n_train", type=int, default=256, help="synthetic training patches (ignored with --dataset)")
+    p.add_argument("--dataset", type=str, default=None,
+                   help=".npz of dB mel patches written by audiosourcesep_b200.datasets.wav_to_spec: train on 'train', "
+                        "log the test loss of 'test' after every epoch")
     p.add_argument("--height", type=int, default=96)
     p.add_argument("--width", type=int, default=64)
     p.add_argument("--L", type=int, default=3)
@@ -131,7 +170,12 @@ def main(args):
     torch.cuda.set_device(local_rank)
     if world > 1 and not dist.is_initialized():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
-    data = synthetic_dataset(int(args.n_train), int(args.seed), args.height, args.width)
+    test = None
+    if getattr(args, "dataset", None):
+        from .datasets.wav_to_spec import load_patches
+        data, test = load_patches(args.dataset, args.height, args.width)
+    else:
+        data = synthetic_dataset(int(args.n_train), int(args.seed), args.height, args.width)
     minibatch = data[: int(args.batch_size)]                     # data-dependent ActNorm init batch (train_glow.py:300-306)
     flow = build_glow(minibatch, [args.height, args.width, 1], L=args.L, K=args.K, n_filters=args.n_filters,
                       learntop=args.learntop, l2_reg=None, data_type="melspec", minval=-100.0, maxval=20.0,
@@ -140,7 +184,7 @@ def main(args):
     optimizer = setUp_optimizer(None, args)
     log = print if rank == 0 else (lambda *a, **k: None)
     if not args.noisy:
-        hist = train(flow, optimizer, data, args, log=log)
+        hist = train(flow, optimizer, data, args, log=log, test=test)
         if rank == 0:
             flow.sync_host()
             os.makedirs(args.output, exist_ok=True)
@@ -151,7 +195,7 @@ def main(args):
     for sigma in sigmas:                                         # serial over noise levels, warm start (train_noisy_glow.py:309-358)
         log("Training at noise level sigma = {}".format(sigma))
         # noise is added in RAW data units (dB), train_noisy_glow.py:31-32
-        hist += train(flow, optimizer, data, args, sigma=float(sigma), log=log, step_offset=len(hist))
+        hist += train(flow, optimizer, data, args, sigma=float(sigma), log=log, step_offset=len(hist), test=test)
         if rank == 0:
             flow.sync_host()
             d = os.path.join(args.output, "sigma_" + str(round(float(sigma), 2)))

@@ -68,10 +68,33 @@ def shard(perm: np.ndarray, it: int, global_batch: int, rank: int, world: int) -
     return perm[it * global_batch + rank * local: it * global_batch + (rank + 1) * local]
 
 
-def train(model, optimizer, data: np.ndarray, args, log=print, ema_decay: Optional[float] = None):
+def held_out_dsm(model, sigmas, test: np.ndarray, batch: int, seed: int = 0) -> float:
+    """The denoising-score-matching loss of the (normalised) test patches in the units of the train loss, from forward
+    score evaluations only: one noise level per patch and z ~ N(0, 1), both drawn from fixed keys (seed, global sample
+    index), so every epoch is evaluated on the same perturbations.  Per patch 1/2 sum (score - target)^2 sigma^2 =
+    1/2 sum (score sigma + z)^2 (train_ncsn.py:26-44)."""
+    from . import ops
+    from .train_glow import held_out_mean
+    idx_all = np.random.default_rng(seed).integers(0, len(sigmas), test.shape[0]).astype(np.int32)
+    sig = torch.as_tensor(np.asarray(sigmas, dtype=np.float32), device=model.device)
+
+    def dsm(x, first):
+        idx = torch.as_tensor(idx_all[first: first + x.shape[0]], device=model.device)
+        per = int(np.prod(x.shape[1:]))
+        z = ops.philox_normal(tuple(x.shape), seed=seed, step=0, stream_id=5, elem_offset=first * per)
+        s = sig[idx.long()].reshape(-1, *([1] * (x.ndim - 1)))
+        score = model.score(x + s * z, idx)
+        return 0.5 * ((score * s + z) ** 2).sum(dim=tuple(range(1, x.ndim)))
+    return held_out_mean(test, batch, dsm)
+
+
+def train(model, optimizer, data: np.ndarray, args, log=print, ema_decay: Optional[float] = None,
+          test: Optional[np.ndarray] = None, sigmas=None):
     """Epoch loop over a host dataset of NORMALISED patches (reference: train_ncsn.py:95-160 without the TensorBoard /
     sample-grid side outputs); stops on a NaN / Inf loss (:113-117).  ``ema_decay``: tfa MovingAverage(0.999) of the
-    flat parameter vector (train_ncsn.py:327-329), returned as the second value."""
+    flat parameter vector (train_ncsn.py:327-329), returned as the second value.  ``test``: held-out normalised
+    patches; when non-empty, ``Epoch NNN: Test Loss: ...`` (:func:`held_out_dsm` at the noise levels ``sigmas``) is logged
+    after every epoch."""
     world = dist.get_world_size() if dist.is_initialized() else 1
     rank = dist.get_rank() if dist.is_initialized() else 0
     gb = int(args.batch_size)
@@ -97,6 +120,9 @@ def train(model, optimizer, data: np.ndarray, args, log=print, ema_decay: Option
                 log("Nan or Inf Loss: {}".format(loss))
                 return history, ema
         log("Epoch {:03d}: Train Loss: {:.3f}  ({:.1f} s)".format(epoch, float(np.mean(history[-steps_per_epoch:])), time.time() - t0))
+        if test is not None and test.shape[0] > 0:
+            tl = held_out_dsm(model, sigmas, test, gb // world, seed=int(getattr(args, "seed", 0)))
+            log("Epoch {:03d}: Test Loss: {:.6f}".format(epoch, tl))
     return history, ema
 
 
@@ -106,7 +132,10 @@ def build_parser():
     p.add_argument("--output", type=str, default="trained_ncsn")
     p.add_argument("--version", type=str, default="v2")
     p.add_argument("--ema", action="store_true")
-    p.add_argument("--n_train", type=int, default=256, help="synthetic training patches")
+    p.add_argument("--n_train", type=int, default=256, help="synthetic training patches (ignored with --dataset)")
+    p.add_argument("--dataset", type=str, default=None,
+                   help=".npz of dB mel patches written by audiosourcesep_b200.datasets.wav_to_spec: train on 'train' "
+                        "(normalised (x + 100) / 120), log the test loss of 'test' after every epoch")
     p.add_argument("--height", type=int, default=96)
     p.add_argument("--width", type=int, default=64)
     p.add_argument("--n_filters", type=int, default=192)
@@ -141,7 +170,13 @@ def main(args):
                      num_classes=int(args.num_classes), sigma1=float(args.sigma1), sigmaL=float(args.sigmaL),
                      progression=args.progression)
     sigmas = get_sigmas(cfg.sigma1, cfg.sigmaL, cfg.num_classes, progression=cfg.progression)
-    data = synthetic.normalise(synthetic.mel_patches_db(int(args.n_train), int(args.seed), cfg.H, cfg.W))
+    test = None
+    if getattr(args, "dataset", None):
+        from .datasets.wav_to_spec import load_patches
+        train_db, test_db = load_patches(args.dataset, cfg.H, cfg.W)
+        data, test = synthetic.normalise(train_db), synthetic.normalise(test_db)
+    else:
+        data = synthetic.normalise(synthetic.mel_patches_db(int(args.n_train), int(args.seed), cfg.H, cfg.W))
     model = ScoreModel(cfg, init_ncsn_params(cfg, seed=int(args.seed), mode="faithful"), sigmas=sigmas, device=local_rank,
                        precision=_lib.PREC_BF16X3 if args.exact else _lib.PREC_BF16)
     model.enable_training()
@@ -149,7 +184,7 @@ def main(args):
     log = print if rank == 0 else (lambda *a, **k: None)
     log("Total Trainable Variables: ", model.count_params())
     t0 = time.time()
-    hist, ema = train(model, optimizer, data, args, log=log, ema_decay=0.999 if args.ema else None)
+    hist, ema = train(model, optimizer, data, args, log=log, ema_decay=0.999 if args.ema else None, test=test, sigmas=sigmas)
     log("Training time: ", np.round(time.time() - t0, 2), " seconds")
     if rank == 0:
         if ema is not None:

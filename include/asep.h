@@ -296,6 +296,16 @@ int asep_istft(const DLTensor* stft, int hop, DLTensor* audio, void* stream);
 int asep_griffinlim_update(const DLTensor* mag, const DLTensor* rebuilt, DLTensor* tprev, DLTensor* next, float momentum,
                            void* stream);
 
+/* ------------------------------------------------------------------ resampling
+ * Replaces the resampler of librosa.load(path, sr=16000) (datasets/preprocessing.py:9-26; librosa's default
+ * res_type='kaiser_best' = resampy.resample): audio [N, L_in] fp32 -> out [N, L_out] fp32.  time [L_out] float64 is
+ * resampy's running time register (0, 1/ratio, 2/ratio, ... accumulated by repeated addition), shared by every row;
+ * win / delta [nwin] fp32 the interpolation table and its forward differences (built on the host,
+ * audiosourcesep_b200/resample.py); scale = min(1, ratio); step >= 1 the truncated table stride int(scale * 512).
+ * librosa's length fix (ceil(L_in * ratio) samples) and the equal-rate short-cut stay on the host. */
+int asep_resample(const DLTensor* audio, const DLTensor* time, const DLTensor* win, const DLTensor* delta, double scale, int step,
+                  DLTensor* out, void* stream);
+
 /* CUDA-graph replay of whole Langevin steps inside asep_basis_{glow,ncsn}_inner (on by default; steps 2..T of a call
  * with T >= 3 are replays of one captured step whose per-step scalars live in device memory).  0 = launch every step
  * eagerly (parity tests compare the two), and drop the cached graphs. */
