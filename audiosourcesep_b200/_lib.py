@@ -114,6 +114,14 @@ _SIGNATURES = {
                             ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_float), _U64, _U64, _P, _P, _V],
     "asep_basis_ncsn_run": [_V, _V, _P, _P, _P, _I, _I, ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_float),
                             ctypes.POINTER(ctypes.c_float), _U64, _U64, _P, _P, _V],
+    "asep_mixing_db_k": [_I, _P, _P, _P, _V],
+    "asep_langevin_step_k": [_I, _P, _P, _P, _P, _F, _F, _F, _U64, _U64, _U64, _P, _V],
+    "asep_basis_glow_inner_k": [_I, ctypes.POINTER(_V), _P, _P, _I, _F, _F, _F, _P, _U64, _U64, _U64, _P, _P, _V],
+    "asep_basis_ncsn_inner_k": [_I, ctypes.POINTER(_V), _P, _P, _I, _I, _F, _F, _F, _P, _U64, _U64, _U64, _P, _P, _V],
+    "asep_basis_glow_run_k": [_I, ctypes.POINTER(_V), _I, _P, _P, _I, _I, ctypes.POINTER(ctypes.c_float),
+                              ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_float), _U64, _U64, _P, _P, _V],
+    "asep_basis_ncsn_run_k": [_I, ctypes.POINTER(_V), _P, _P, _I, _I, ctypes.POINTER(ctypes.c_float),
+                              ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_float), _U64, _U64, _P, _P, _V],
     "asep_conv_profile": [_I],
     "asep_conv_profile_read": [ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_int64),
                                ctypes.POINTER(ctypes.c_double)],

@@ -522,6 +522,25 @@ int asep_squeeze(const DLTensor* x, DLTensor* y, int inverse, void* stream) {
 }
 
 // ------------------------------------------------------------------ Langevin
+static void check_sources(int K) {
+  ASEP_CHECK(K >= 2 && K <= kMaxSources, ASEP_ERR_BAD_ARG, "the number of sources K must be in [2, %d] (got %d)", kMaxSources, K);
+}
+
+// v = [lead..., *item.shape]: the stacked layout of the K-source entry points (source axis after the step / level axis)
+static void expect_stacked(const TView& v, const char* what, std::initializer_list<int64_t> lead, const TView& item) {
+  bool ok = v.ndim == (int)lead.size() + item.ndim;
+  int i = 0;
+  for (auto l : lead) ok = ok && v.shape[i++] == l;
+  for (int j = 0; ok && j < item.ndim; ++j) ok = v.shape[i + j] == item.shape[j];
+  if (!ok) {
+    std::string got = "[", want = "[";
+    for (int j = 0; j < v.ndim; ++j) got += std::to_string(v.shape[j]) + (j + 1 < v.ndim ? "," : "");
+    for (auto l : lead) want += std::to_string(l) + ",";
+    for (int j = 0; j < item.ndim; ++j) want += std::to_string(item.shape[j]) + (j + 1 < item.ndim ? "," : "");
+    throw Error(ASEP_ERR_BAD_SHAPE, strfmt("%s: shape %s], expected %s]", what, got.c_str(), want.c_str()));
+  }
+}
+
 int asep_langevin_step(DLTensor* x1, DLTensor* x2, const DLTensor* s1, const DLTensor* s2, const DLTensor* mixed,
                        const DLTensor* n1, const DLTensor* n2, float eta, float lambda, float noise_scale,
                        uint64_t seed, uint64_t step, uint64_t elem_offset, DLTensor* nan_count, void* stream) {
@@ -531,16 +550,44 @@ int asep_langevin_step(DLTensor* x1, DLTensor* x2, const DLTensor* s1, const DLT
   ASEP_CHECK(a.numel == b.numel && a.numel == sa.numel && a.numel == sb.numel && a.numel == mx.numel,
              ASEP_ERR_BAD_SHAPE, "langevin: all tensors must have the same number of elements");
   ASEP_CHECK((n1 == nullptr) == (n2 == nullptr), ASEP_ERR_BAD_ARG, "inject both noise tensors or neither");
-  const float *p1 = nullptr, *p2 = nullptr;
+  LangevinSources p{};
+  p.x[0] = a.f32; p.x[1] = b.f32;
+  p.s[0] = sa.f32; p.s[1] = sb.f32;
   if (n1) {
     TView na = view_f32(n1, "n1", g_device), nb = view_f32(n2, "n2", g_device);
     ASEP_CHECK(na.numel == a.numel && nb.numel == a.numel, ASEP_ERR_BAD_SHAPE, "noise shape mismatch");
-    p1 = na.f32; p2 = nb.f32;
+    p.n[0] = na.f32; p.n[1] = nb.f32;
   }
   int* nanp = nullptr;
   if (nan_count) nanp = static_cast<int*>(view_i32(nan_count, "nan_count", g_device).raw);
-  launch_langevin(a.f32, b.f32, sa.f32, sb.f32, mx.f32, p1, p2, eta, lambda, noise_scale, seed, step, elem_offset,
-                  nanp, a.numel, as_stream(stream));
+  launch_langevin(2, p, mx.f32, eta, lambda, noise_scale, seed, step, elem_offset, nanp, a.numel, as_stream(stream));
+  ASEP_API_END
+}
+
+int asep_langevin_step_k(int K, DLTensor* x, const DLTensor* score, const DLTensor* mixed, const DLTensor* noise, float eta,
+                         float lambda, float noise_scale, uint64_t seed, uint64_t step, uint64_t elem_offset,
+                         DLTensor* nan_count, void* stream) {
+  ASEP_API_BEGIN
+  check_sources(K);
+  TView mx = view_f32(mixed, "mixed", g_device), xv = view_f32(x, "x", g_device), sv = view_f32(score, "score", g_device);
+  expect_stacked(xv, "x", {K}, mx);
+  expect_stacked(sv, "score", {K}, mx);
+  const long long n = mx.numel;
+  ASEP_CHECK(n % 4 == 0, ASEP_ERR_BAD_SHAPE, "langevin: the element count of one source (%lld) must be a multiple of 4", n);
+  TView nv{};
+  if (noise) {
+    nv = view_f32(noise, "noise", g_device);
+    expect_stacked(nv, "noise", {K}, mx);
+  }
+  int* nanp = nullptr;
+  if (nan_count) nanp = static_cast<int*>(view_i32(nan_count, "nan_count", g_device).raw);
+  LangevinSources p{};
+  for (int k = 0; k < K; ++k) {
+    p.x[k] = xv.f32 + k * n;
+    p.s[k] = sv.f32 + k * n;
+    p.n[k] = noise ? nv.f32 + k * n : nullptr;
+  }
+  launch_langevin(K, p, mx.f32, eta, lambda, noise_scale, seed, step, elem_offset, nanp, n, as_stream(stream));
   ASEP_API_END
 }
 
@@ -550,7 +597,26 @@ int asep_mixing_db(const DLTensor* x1, const DLTensor* x2, DLTensor* g, DLTensor
   TView wa = view_f32(w1, "w1", g_device), wb = view_f32(w2, "w2", g_device);
   ASEP_CHECK(a.numel == b.numel && a.numel == gv.numel && a.numel == wa.numel && a.numel == wb.numel,
              ASEP_ERR_BAD_SHAPE, "mixing: element counts differ");
-  launch_mixing_db(a.f32, b.f32, gv.f32, wa.f32, wb.f32, a.numel, as_stream(stream));
+  MixingSources p{};
+  p.x[0] = a.f32; p.x[1] = b.f32;
+  p.w[0] = wa.f32; p.w[1] = wb.f32;
+  launch_mixing_db(2, p, gv.f32, a.numel, as_stream(stream));
+  ASEP_API_END
+}
+
+int asep_mixing_db_k(int K, const DLTensor* x, DLTensor* g, DLTensor* w, void* stream) {
+  ASEP_API_BEGIN
+  check_sources(K);
+  TView xv = view_f32(x, "x", g_device), gv = view_f32(g, "g", g_device), wv = view_f32(w, "w", g_device);
+  expect_stacked(xv, "x", {K}, gv);
+  expect_stacked(wv, "w", {K}, gv);
+  const long long n = gv.numel;
+  MixingSources p{};
+  for (int k = 0; k < K; ++k) {
+    p.x[k] = xv.f32 + k * n;
+    p.w[k] = wv.f32 + k * n;
+  }
+  launch_mixing_db(K, p, gv.f32, n, as_stream(stream));
   ASEP_API_END
 }
 
@@ -565,30 +631,34 @@ int asep_philox_normal(DLTensor* out, uint64_t seed, uint64_t step, uint64_t str
 }  // extern "C" (re-opened below)
 
 namespace {
-// ---- CUDA graphs of one whole BASIS Langevin step (both scores + the fused update), replayed for steps 2..T of a call.
-// A graph bakes in the state / noise / dump pointers of the call and the workspaces of both priors, so it is keyed by
-// all of them plus each prior's (uid, generation); per-step scalars are read from `dev` (LangevinDev).  The two score
-// evaluations are independent until the update: with two distinct handles they are captured as parallel branches (the
-// second on `side`), so the small HBM-bound launches of one prior overlap the tensor-core launches of the other.
+// ---- CUDA graphs of one whole BASIS Langevin step (every score + the fused update), replayed for steps 2..T of a call.
+// A graph bakes in the state / noise / dump pointers of the call and the workspaces of the priors, so it is keyed by
+// all of them plus each source's prior (uid, generation); per-step scalars are read from `dev` (LangevinDev).  The score
+// evaluations of distinct priors are independent until the update: each prior is captured as a branch of its own (the
+// first on `stream`, the others on `side[]`), so the small HBM-bound launches of one prior overlap the tensor-core
+// launches of the others.  A prior serving several sources evaluates them one after another on its branch.
 struct BasisGraphKey {
-  const void* p[9];
-  long long m1, m2, g1, g2;
+  const void* p[3 + 3 * kMaxSources];               // mixed, dump, NaN counter, then every source's state, score, noise
+  long long uid[kMaxSources], gen[kMaxSources];     // prior of every source
   unsigned long long seed, off;
-  int N, kind;                                      // kind: 0 Glow priors, 1 NCSN
+  long long noise_stride;
+  int N, kind, K, pad;                              // kind: 0 Glow priors, 1 NCSN
   bool operator<(const BasisGraphKey& o) const { return std::memcmp(this, &o, sizeof(*this)) < 0; }
 };
 struct BasisGraph { cudaGraphExec_t exec = nullptr; long long launches = 0; };
 struct BasisGraphs {
   std::map<BasisGraphKey, BasisGraph> graphs;
-  cudaStream_t stream = nullptr, side = nullptr;    // private: the caller's stream may be the legacy stream (not capturable)
-  cudaEvent_t ev_in = nullptr, ev_out = nullptr, ev_fork = nullptr, ev_join = nullptr;
+  cudaStream_t stream = nullptr;                    // private: the caller's stream may be the legacy stream (not capturable)
+  cudaStream_t side[kMaxSources - 1] = {};
+  cudaEvent_t ev_in = nullptr, ev_out = nullptr, ev_fork = nullptr, ev_join[kMaxSources - 1] = {};
   LangevinDev* dev = nullptr;
   bool enabled = true;
   void ensure() {
     if (stream) return;
     CUDA_CHECK(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-    CUDA_CHECK(cudaStreamCreateWithFlags(&side, cudaStreamNonBlocking));
-    for (cudaEvent_t* e : {&ev_in, &ev_out, &ev_fork, &ev_join}) CUDA_CHECK(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+    for (cudaStream_t& st : side) CUDA_CHECK(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
+    for (cudaEvent_t* e : {&ev_in, &ev_out, &ev_fork}) CUDA_CHECK(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+    for (cudaEvent_t& e : ev_join) CUDA_CHECK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     CUDA_CHECK(cudaMalloc(&dev, sizeof(LangevinDev)));
   }
   void clear() {
@@ -603,37 +673,65 @@ BasisGraphs& basis_graphs() {
   return g;
 }
 
+// One call of T Langevin steps over K sources.  src.n[k] is the base of source k's injected noise (step t at
+// src.n[k] + t * noise_stride) or NULL; dump the base of the [T, K, ...] per-step dump or NULL.
 struct BasisCall {
-  float *x1, *x2, *s1, *s2;
-  const float *mixed, *nz1, *nz2;
+  int K;
+  LangevinSources src;
+  long long noise_stride;
+  const float* mixed;
   float* dump;
   int* nanp;
-  long long numel;
+  long long numel;                                  // elements of one source
   int N, T;
   float eta, lambda, noise_scale;
   uint64_t seed, step0, elem_offset;
 };
 
-// score1(stream) / score2(stream) launch the score evaluation of source 1 / 2 into c.s1 / c.s2.
-// generations(key) fills key.g1 / key.g2; it is called after the first (eager) step has sized both workspaces.
-template <class F1, class F2, class FG>
-void run_basis_steps(const BasisCall& c, BasisGraphKey key, bool parallel, bool allow_graph, cudaStream_t s, F1&& score1,
-                     F2&& score2, FG&& generations) {
-  auto eager_step = [&](int t) {
-    score1(s);
-    score2(s);
-    launch_langevin(c.x1, c.x2, c.s1, c.s2, c.mixed, c.nz1 ? c.nz1 + (size_t)t * c.numel : nullptr,
-                    c.nz2 ? c.nz2 + (size_t)t * c.numel : nullptr, c.eta, c.lambda, c.noise_scale, c.seed, c.step0 + t,
-                    c.elem_offset, c.nanp, c.numel, s);
-    if (c.dump) {
-      CUDA_CHECK(cudaMemcpyAsync(c.dump + (size_t)(2 * t) * c.numel, c.x1, (size_t)c.numel * sizeof(float),
-                                 cudaMemcpyDeviceToDevice, s));
-      CUDA_CHECK(cudaMemcpyAsync(c.dump + (size_t)(2 * t + 1) * c.numel, c.x2, (size_t)c.numel * sizeof(float),
-                                 cudaMemcpyDeviceToDevice, s));
+// Sources grouped by prior handle, in order of first use.  The reference treats priors as plain callables
+// (run_basis_sep.py:166-175), so one handle may serve several sources: its score scratch then holds one tensor per source.
+template <class M>
+struct SourceGroups {
+  std::vector<M*> models;
+  std::vector<std::vector<int>> sources;
+};
+template <class M>
+SourceGroups<M> group_sources(BasisCall& c, M* const* m) {
+  SourceGroups<M> g;
+  for (int k = 0; k < c.K; ++k) {
+    size_t b = 0;
+    while (b < g.models.size() && g.models[b] != m[k]) ++b;
+    if (b == g.models.size()) {
+      g.models.push_back(m[k]);
+      g.sources.emplace_back();
     }
+    g.sources[b].push_back(k);
+  }
+  for (size_t b = 0; b < g.models.size(); ++b) {
+    float* buf = g.models[b]->score_scratch(c.N, (int)g.sources[b].size());
+    for (size_t j = 0; j < g.sources[b].size(); ++j) c.src.s[g.sources[b][j]] = buf + j * c.numel;
+  }
+  return g;
+}
+
+// score(b, stream) launches the score evaluations of branch b (one prior, every source it serves) into c.src.s.
+// generations(key) fills key.gen; it is called after the first (eager) step has sized every workspace.
+template <class FS, class FG>
+void run_basis_steps(const BasisCall& c, BasisGraphKey key, int branches, bool allow_graph, cudaStream_t s, FS&& score,
+                     FG&& generations) {
+  auto eager_step = [&](int t) {
+    for (int b = 0; b < branches; ++b) score(b, s);
+    LangevinSources p = c.src;
+    for (int k = 0; k < c.K; ++k)
+      if (p.n[k]) p.n[k] += (size_t)t * c.noise_stride;
+    launch_langevin(c.K, p, c.mixed, c.eta, c.lambda, c.noise_scale, c.seed, c.step0 + t, c.elem_offset, c.nanp, c.numel, s);
+    if (c.dump)
+      for (int k = 0; k < c.K; ++k)
+        CUDA_CHECK(cudaMemcpyAsync(c.dump + (size_t)(c.K * t + k) * c.numel, c.src.x[k], (size_t)c.numel * sizeof(float),
+                                   cudaMemcpyDeviceToDevice, s));
   };
-  // One Langevin step is 300-1200 small launches at the reference's n_mixed = 30: from the second step on the whole step
-  // is replayed as ONE CUDA graph whose per-step scalars live in device memory.
+  // One Langevin step is 300-1200 small launches per source at the reference's n_mixed = 30: from the second step on the
+  // whole step is replayed as ONE CUDA graph whose per-step scalars live in device memory.
   BasisGraphs& bg = basis_graphs();
   static const bool no_graph = getenv("ASEP_NO_GRAPH") != nullptr;
   const bool use_graph = c.T >= 3 && allow_graph && bg.enabled && !no_graph;
@@ -642,12 +740,16 @@ void run_basis_steps(const BasisCall& c, BasisGraphKey key, bool parallel, bool 
     return;
   }
   bg.ensure();
-  const void* ptrs[9] = {c.x1, c.x2, c.mixed, c.nz1, c.nz2, c.dump, c.nanp, c.s1, c.s2};
-  std::memcpy(key.p, ptrs, sizeof(ptrs));
-  key.N = c.N; key.seed = c.seed; key.off = c.elem_offset;
+  key.p[0] = c.mixed; key.p[1] = c.dump; key.p[2] = c.nanp;
+  for (int k = 0; k < c.K; ++k) {
+    key.p[3 + 3 * k] = c.src.x[k];
+    key.p[4 + 3 * k] = c.src.s[k];
+    key.p[5 + 3 * k] = c.src.n[k];
+  }
+  key.N = c.N; key.K = c.K; key.seed = c.seed; key.off = c.elem_offset; key.noise_stride = c.noise_stride;
   generations(key);
   auto it = bg.graphs.find(key);
-  // a cached graph means both workspaces already have this size: every step of the call is a replay.  Otherwise the
+  // a cached graph means every workspace already has this size: every step of the call is a replay.  Otherwise the
   // first step runs eagerly (it sizes the workspaces -- a capture may not allocate) and the rest replay the new graph.
   const int t_first = it != bg.graphs.end() ? 0 : 1;
   if (t_first == 1) eager_step(0);
@@ -662,19 +764,20 @@ void run_basis_steps(const BasisCall& c, BasisGraphKey key, bool parallel, bool 
     const long long c0 = g_launch_count.load();
     CUDA_CHECK(cudaStreamBeginCapture(bg.stream, cudaStreamCaptureModeRelaxed));
     try {
-      if (parallel) {
+      if (branches > 1) {
         CUDA_CHECK(cudaEventRecord(bg.ev_fork, bg.stream));
-        CUDA_CHECK(cudaStreamWaitEvent(bg.side, bg.ev_fork, 0));
-        score1(bg.stream);
-        score2(bg.side);
-        CUDA_CHECK(cudaEventRecord(bg.ev_join, bg.side));
-        CUDA_CHECK(cudaStreamWaitEvent(bg.stream, bg.ev_join, 0));
+        for (int b = 1; b < branches; ++b) CUDA_CHECK(cudaStreamWaitEvent(bg.side[b - 1], bg.ev_fork, 0));
+        score(0, bg.stream);
+        for (int b = 1; b < branches; ++b) {
+          score(b, bg.side[b - 1]);
+          CUDA_CHECK(cudaEventRecord(bg.ev_join[b - 1], bg.side[b - 1]));
+          CUDA_CHECK(cudaStreamWaitEvent(bg.stream, bg.ev_join[b - 1], 0));
+        }
       } else {
-        score1(bg.stream);
-        score2(bg.stream);
+        score(0, bg.stream);
       }
-      launch_langevin_dev(c.x1, c.x2, c.s1, c.s2, c.mixed, c.nz1, c.nz2, c.dump, bg.dev, c.seed, c.elem_offset, c.nanp,
-                          c.numel, bg.stream);
+      launch_langevin_dev(c.K, c.src, c.mixed, c.noise_stride, c.dump, bg.dev, c.seed, c.elem_offset, c.nanp, c.numel,
+                          bg.stream);
     } catch (...) {
       cudaStreamEndCapture(bg.stream, &graph);
       if (graph) cudaGraphDestroy(graph);
@@ -695,6 +798,55 @@ void run_basis_steps(const BasisCall& c, BasisGraphKey key, bool parallel, bool 
   CUDA_CHECK(cudaEventRecord(bg.ev_out, bg.stream));
   CUDA_CHECK(cudaStreamWaitEvent(s, bg.ev_out, 0));
 }
+
+// T steps with K Glow priors m[k] (c.src.x / n, dump and the scalars filled in by the caller)
+void basis_glow_steps(BasisCall c, GlowModel* const* m, cudaStream_t s) {
+  SourceGroups<GlowModel> g = group_sources(c, m);
+  BasisGraphKey key{};
+  key.kind = 0;
+  for (int k = 0; k < c.K; ++k) key.uid[k] = m[k]->uid();
+  const bool allow_graph = !nn_tc_profile_enabled() && !hbm_profile_enabled();
+  run_basis_steps(c, key, (int)g.models.size(), allow_graph, s,
+                  [&](int b, cudaStream_t st) {
+                    for (int k : g.sources[b])                                 // run_basis_sep.py:174-175
+                      g.models[b]->grad_log_prob(c.src.x[k], const_cast<float*>(c.src.s[k]), nullptr, c.N, st);
+                  },
+                  [&](BasisGraphKey& key) {
+                    for (int k = 0; k < c.K; ++k) key.gen[k] = m[k]->generation();
+                  });
+}
+
+// T steps at noise level sigma_idx with K score networks m[k]
+void basis_ncsn_steps(BasisCall c, NcsnModel* const* m, int sigma_idx, cudaStream_t s) {
+  SourceGroups<NcsnModel> g = group_sources(c, m);
+  const int* idx = m[0]->index_scratch(c.N, sigma_idx, s);                     // run_basis_sep.py:167-168
+  BasisGraphKey key{};
+  key.kind = 1;
+  for (int k = 0; k < c.K; ++k) key.uid[k] = m[k]->uid();
+  const bool allow_graph = !conv_tc_profile_enabled() && !hbm_profile_enabled();
+  run_basis_steps(c, key, (int)g.models.size(), allow_graph, s,
+                  [&](int b, cudaStream_t st) {
+                    for (int k : g.sources[b])                                 // run_basis_sep.py:169-170
+                      g.models[b]->forward(c.src.x[k], idx, const_cast<float*>(c.src.s[k]), c.N, st);
+                  },
+                  [&](BasisGraphKey& key) {
+                    for (int k = 0; k < c.K; ++k) key.gen[k] = m[k]->generation();
+                  });
+}
+
+// Optional injected noise [T, K, ...] / per-step dump [T, K, ...] of a stacked K-source call whose state is x [K, ...].
+const float* stacked_noise(const DLTensor* noise, const TView& x, int T, int dev) {
+  if (!noise) return nullptr;
+  TView v = view_f32(noise, "noise", dev);
+  expect_stacked(v, "noise", {T}, x);
+  return v.f32;
+}
+float* stacked_dump(DLTensor* per_step, const TView& x, int T, int dev) {
+  if (!per_step) return nullptr;
+  TView v = view_f32(per_step, "per_step", dev);
+  expect_stacked(v, "per_step", {T}, x);
+  return v.f32;
+}
 }  // namespace
 
 extern "C" {
@@ -712,36 +864,54 @@ int asep_basis_glow_inner(asep_glow_t m1, asep_glow_t m2, const DLTensor* mixed,
   ASEP_CHECK(batch_of(b, g2, "x2") == N && mx.numel == a.numel, ASEP_ERR_BAD_SHAPE, "x1, x2, mixed must match");
   ASEP_CHECK(g2.device() == dev, ASEP_ERR_BAD_DEVICE, "the two priors live on different devices");
   ASEP_CHECK((noise1 == nullptr) == (noise2 == nullptr), ASEP_ERR_BAD_ARG, "inject both noise tensors or neither");
-  const float *nz1 = nullptr, *nz2 = nullptr;
+  BasisCall call{2, {}, a.numel, mx.f32, nullptr, nullptr, (long long)a.numel, N, T, eta, lambda, noise_scale, seed, step0,
+                 elem_offset};
+  call.src.x[0] = a.f32; call.src.x[1] = b.f32;
   if (noise1) {
     TView na = view_f32(noise1, "noise1", dev), nb = view_f32(noise2, "noise2", dev);
     ASEP_CHECK(na.numel == (int64_t)T * a.numel && nb.numel == na.numel, ASEP_ERR_BAD_SHAPE, "noise must be [T, ...]");
-    nz1 = na.f32; nz2 = nb.f32;
+    call.src.n[0] = na.f32; call.src.n[1] = nb.f32;
   }
-  float* dump = nullptr;
   if (per_step) {
     TView d = view_f32(per_step, "per_step", dev);
     ASEP_CHECK(d.numel == (int64_t)T * 2 * a.numel, ASEP_ERR_BAD_SHAPE, "per_step must be [T, 2, ...]");
-    dump = d.f32;
+    call.dump = d.f32;
   }
-  int* nanp = nullptr;
-  if (nan_count) nanp = static_cast<int*>(view_i32(nan_count, "nan_count", dev).raw);
-  cudaStream_t s = as_stream(stream);
-  // model1 and model2 are just callables in the reference (run_basis_sep.py:166-175): the same prior may serve both
-  // sources, in which case its scratch holds two score tensors
-  const bool same = &g1 == &g2;
-  float* s1 = g1.score_scratch(N, same ? 2 : 1);
-  float* s2 = same ? s1 + a.numel : g2.score_scratch(N);
-  BasisCall call{a.f32, b.f32, s1, s2, mx.f32, nz1, nz2, dump, nanp, (long long)a.numel, N, T, eta, lambda, noise_scale,
-                 seed, step0, elem_offset};
-  BasisGraphKey key{};
-  key.kind = 0;
-  key.m1 = g1.uid(); key.m2 = g2.uid();
-  const bool allow_graph = !nn_tc_profile_enabled() && !hbm_profile_enabled();
-  run_basis_steps(call, key, !same, allow_graph, s,
-                  [&](cudaStream_t st) { g1.grad_log_prob(a.f32, s1, nullptr, N, st); },     // run_basis_sep.py:174-175
-                  [&](cudaStream_t st) { g2.grad_log_prob(b.f32, s2, nullptr, N, st); },
-                  [&](BasisGraphKey& k) { k.g1 = g1.generation(); k.g2 = g2.generation(); });
+  if (nan_count) call.nanp = static_cast<int*>(view_i32(nan_count, "nan_count", dev).raw);
+  GlowModel* const ms[2] = {&g1, &g2};
+  basis_glow_steps(call, ms, as_stream(stream));
+  ASEP_API_END
+}
+
+int asep_basis_glow_inner_k(int K, const asep_glow_t* m, const DLTensor* mixed, DLTensor* x, int T, float eta, float lambda,
+                            float noise_scale, const DLTensor* noise, uint64_t seed, uint64_t step0, uint64_t elem_offset,
+                            DLTensor* per_step, DLTensor* nan_count, void* stream) {
+  ASEP_API_BEGIN
+  check_sources(K);
+  ASEP_CHECK(m != nullptr && T >= 0, ASEP_ERR_BAD_ARG, "NULL model array or negative T");
+  GlowModel* ms[kMaxSources];
+  for (int k = 0; k < K; ++k) {
+    ASEP_CHECK(m[k] != nullptr, ASEP_ERR_BAD_ARG, "NULL handle for source %d", k);
+    ms[k] = m[k]->model.get();
+  }
+  const int dev = ms[0]->device();
+  TView mx = view_f32(mixed, "mixed", dev), xv = view_f32(x, "x", dev);
+  for (int k = 0; k < K; ++k) {
+    batch_of(mx, *ms[k], "mixed");                  // every prior models the data shape of the mixture
+    ASEP_CHECK(ms[k]->device() == dev, ASEP_ERR_BAD_DEVICE, "the priors live on different devices");
+  }
+  expect_stacked(xv, "x", {K}, mx);
+  ASEP_CHECK(mx.numel % 4 == 0, ASEP_ERR_BAD_SHAPE, "the element count of one source (%lld) must be a multiple of 4",
+             (long long)mx.numel);
+  BasisCall call{K, {}, (long long)K * mx.numel, mx.f32, stacked_dump(per_step, xv, T, dev), nullptr, (long long)mx.numel,
+                 (int)mx.shape[0], T, eta, lambda, noise_scale, seed, step0, elem_offset};
+  const float* nz = stacked_noise(noise, xv, T, dev);
+  for (int k = 0; k < K; ++k) {
+    call.src.x[k] = xv.f32 + k * mx.numel;
+    call.src.n[k] = nz ? nz + k * mx.numel : nullptr;
+  }
+  if (nan_count) call.nanp = static_cast<int*>(view_i32(nan_count, "nan_count", dev).raw);
+  basis_glow_steps(call, ms, as_stream(stream));
   ASEP_API_END
 }
 
@@ -924,48 +1094,80 @@ int asep_basis_ncsn_inner(asep_ncsn_t m1, asep_ncsn_t m2, const DLTensor* mixed,
   ASEP_CHECK(sigma_idx >= 0 && sigma_idx < c.num_classes && sigma_idx < c2.num_classes, ASEP_ERR_BAD_ARG,
              "sigma_idx %d out of range (num_classes %d / %d)", sigma_idx, c.num_classes, c2.num_classes);
   ASEP_CHECK((noise1 == nullptr) == (noise2 == nullptr), ASEP_ERR_BAD_ARG, "inject both noise tensors or neither");
-  const float *nz1 = nullptr, *nz2 = nullptr;
+  BasisCall call{2, {}, a.numel, mx.f32, nullptr, nullptr, (long long)a.numel, N, T, eta, lambda, noise_scale, seed, step0,
+                 elem_offset};
+  call.src.x[0] = a.f32; call.src.x[1] = b.f32;
   if (noise1) {
     TView na = view_f32(noise1, "noise1", dev), nb = view_f32(noise2, "noise2", dev);
     ASEP_CHECK(na.numel == (int64_t)T * a.numel && nb.numel == na.numel, ASEP_ERR_BAD_SHAPE, "noise must be [T, ...]");
-    nz1 = na.f32; nz2 = nb.f32;
+    call.src.n[0] = na.f32; call.src.n[1] = nb.f32;
   }
-  float* dump = nullptr;
   if (per_step) {
     TView d = view_f32(per_step, "per_step", dev);
     ASEP_CHECK(d.numel == (int64_t)T * 2 * a.numel, ASEP_ERR_BAD_SHAPE, "per_step must be [T, 2, ...]");
-    dump = d.f32;
+    call.dump = d.f32;
   }
-  int* nanp = nullptr;
-  if (nan_count) nanp = static_cast<int*>(view_i32(nan_count, "nan_count", dev).raw);
-  cudaStream_t s = as_stream(stream);
-  // model1 and model2 are just callables in the reference (run_basis_sep.py:166-175): the same prior may serve both
-  // sources, in which case its scratch holds two score tensors
-  const bool same = &g1 == &g2;
-  float* s1 = g1.score_scratch(N, same ? 2 : 1);
-  float* s2 = same ? s1 + a.numel : g2.score_scratch(N);
-  const int* idx = g1.index_scratch(N, sigma_idx, s);               // run_basis_sep.py:167-168
-  BasisCall call{a.f32, b.f32, s1, s2, mx.f32, nz1, nz2, dump, nanp, (long long)a.numel, N, T, eta, lambda, noise_scale,
-                 seed, step0, elem_offset};
-  BasisGraphKey key{};
-  key.kind = 1;
-  key.m1 = g1.uid(); key.m2 = g2.uid();
-  const bool allow_graph = !conv_tc_profile_enabled() && !hbm_profile_enabled();
-  run_basis_steps(call, key, !same, allow_graph, s,
-                  [&](cudaStream_t st) { g1.forward(a.f32, idx, s1, N, st); },               // run_basis_sep.py:169-170
-                  [&](cudaStream_t st) { g2.forward(b.f32, idx, s2, N, st); },
-                  [&](BasisGraphKey& k) { k.g1 = g1.generation(); k.g2 = g2.generation(); });
+  if (nan_count) call.nanp = static_cast<int*>(view_i32(nan_count, "nan_count", dev).raw);
+  NcsnModel* const ms[2] = {&g1, &g2};
+  basis_ncsn_steps(call, ms, sigma_idx, as_stream(stream));
+  ASEP_API_END
+}
+
+int asep_basis_ncsn_inner_k(int K, const asep_ncsn_t* m, const DLTensor* mixed, DLTensor* x, int sigma_idx, int T, float eta,
+                            float lambda, float noise_scale, const DLTensor* noise, uint64_t seed, uint64_t step0,
+                            uint64_t elem_offset, DLTensor* per_step, DLTensor* nan_count, void* stream) {
+  ASEP_API_BEGIN
+  check_sources(K);
+  ASEP_CHECK(m != nullptr && T >= 0, ASEP_ERR_BAD_ARG, "NULL model array or negative T");
+  NcsnModel* ms[kMaxSources];
+  for (int k = 0; k < K; ++k) {
+    ASEP_CHECK(m[k] != nullptr, ASEP_ERR_BAD_ARG, "NULL handle for source %d", k);
+    ms[k] = m[k]->model.get();
+  }
+  const int dev = ms[0]->device();
+  TView mx = view_f32(mixed, "mixed", dev), xv = view_f32(x, "x", dev);
+  for (int k = 0; k < K; ++k) {
+    const auto& c = ms[k]->cfg();
+    expect_shape(mx, "mixed", {-1, c.H, c.W, c.C});   // every score network models the data shape of the mixture
+    ASEP_CHECK(ms[k]->device() == dev, ASEP_ERR_BAD_DEVICE, "the score networks live on different devices");
+    ASEP_CHECK(sigma_idx >= 0 && sigma_idx < c.num_classes, ASEP_ERR_BAD_ARG, "sigma_idx %d out of range (num_classes %d)",
+               sigma_idx, c.num_classes);
+  }
+  expect_stacked(xv, "x", {K}, mx);
+  ASEP_CHECK(mx.numel % 4 == 0, ASEP_ERR_BAD_SHAPE, "the element count of one source (%lld) must be a multiple of 4",
+             (long long)mx.numel);
+  BasisCall call{K, {}, (long long)K * mx.numel, mx.f32, stacked_dump(per_step, xv, T, dev), nullptr, (long long)mx.numel,
+                 (int)mx.shape[0], T, eta, lambda, noise_scale, seed, step0, elem_offset};
+  const float* nz = stacked_noise(noise, xv, T, dev);
+  for (int k = 0; k < K; ++k) {
+    call.src.x[k] = xv.f32 + k * mx.numel;
+    call.src.n[k] = nz ? nz + k * mx.numel : nullptr;
+  }
+  if (nan_count) call.nanp = static_cast<int*>(view_i32(nan_count, "nan_count", dev).raw);
+  basis_ncsn_steps(call, ms, sigma_idx, as_stream(stream));
   ASEP_API_END
 }
 
 // ------------------------------------------------------------------ whole sigma x T loops on the device
 namespace {
-// snapshot of both states after noise level i into snapshots[i] = [2, N, H, W, C] (x_arr of run_basis_sep.py:243-244)
-void snapshot_states(float* snap, int level, const TView& a, const TView& b, cudaStream_t s) {
+// snapshot of the K states after noise level i into snapshots[i] = [K, N, H, W, C] (x_arr of run_basis_sep.py:243-244)
+void snapshot_states(float* snap, int level, int K, float* const* x, long long numel, cudaStream_t s) {
   if (!snap) return;
-  float* dst = snap + (size_t)level * 2 * a.numel;
-  CUDA_CHECK(cudaMemcpyAsync(dst, a.f32, (size_t)a.numel * sizeof(float), cudaMemcpyDeviceToDevice, s));
-  CUDA_CHECK(cudaMemcpyAsync(dst + a.numel, b.f32, (size_t)a.numel * sizeof(float), cudaMemcpyDeviceToDevice, s));
+  float* dst = snap + (size_t)level * K * numel;
+  for (int k = 0; k < K; ++k)
+    CUDA_CHECK(cudaMemcpyAsync(dst + (size_t)k * numel, x[k], (size_t)numel * sizeof(float), cudaMemcpyDeviceToDevice, s));
+}
+
+// the [L, K, ...] snapshots of a K-source run (or NULL); fills x[k] with the state of every source
+float* run_snapshots(DLTensor* snapshots, const TView& xv, int K, int L, float** x, int dev) {
+  for (int k = 0; k < K; ++k) x[k] = xv.f32 + k * (xv.numel / K);
+  if (!snapshots) return nullptr;
+  TView sv = view_f32(snapshots, "snapshots", dev);
+  ASEP_CHECK(sv.ndim == xv.ndim + 1 && sv.shape[0] == L && sv.numel == (int64_t)L * xv.numel, ASEP_ERR_BAD_SHAPE,
+             "snapshots must be [L, K, N, H, W, C]");
+  for (int j = 0; j < xv.ndim; ++j)
+    ASEP_CHECK(sv.shape[j + 1] == xv.shape[j], ASEP_ERR_BAD_SHAPE, "snapshots must be [L, K, N, H, W, C]");
+  return sv.f32;
 }
 }  // namespace
 
@@ -985,13 +1187,38 @@ int asep_basis_glow_run(const asep_glow_t* m1, const asep_glow_t* m2, int n_mode
     ASEP_CHECK(sv.numel == (int64_t)L * 2 * a.numel, ASEP_ERR_BAD_SHAPE, "snapshots must be [L, 2, N, H, W, C]");
     snap = sv.f32;
   }
+  float* const xs[2] = {a.f32, b.f32};
   for (int i = 0; i < L; ++i) {
     const int k = n_models == 1 ? 0 : i;
     ASEP_CHECK(m1[k] && m2[k], ASEP_ERR_BAD_ARG, "NULL handle at level %d", i);
     const int rc = asep_basis_glow_inner(m1[k], m2[k], mixed, x1, x2, T, eta[i], lambda[i], noise_scale[i], nullptr, nullptr, seed,
                                          (uint64_t)i * (uint64_t)T, elem_offset, nullptr, nan_count, stream);
     if (rc != ASEP_OK) return rc;                      // asep_last_error() holds the inner message
-    snapshot_states(snap, i, a, b, as_stream(stream));
+    snapshot_states(snap, i, 2, xs, a.numel, as_stream(stream));
+  }
+  ASEP_API_END
+}
+
+int asep_basis_glow_run_k(int K, const asep_glow_t* m, int n_models, const DLTensor* mixed, DLTensor* x, int L, int T,
+                          const float* eta, const float* lambda, const float* noise_scale, uint64_t seed, uint64_t elem_offset,
+                          DLTensor* snapshots, DLTensor* nan_count, void* stream) {
+  ASEP_API_BEGIN
+  check_sources(K);
+  ASEP_CHECK(m && eta && lambda && noise_scale, ASEP_ERR_BAD_ARG, "NULL argument");
+  ASEP_CHECK(L >= 1 && T >= 0 && (n_models == 1 || n_models == L), ASEP_ERR_BAD_ARG,
+             "n_models must be 1 (one set of K priors for every level) or L (one set per level)");
+  for (int i = 0; i < n_models * K; ++i) ASEP_CHECK(m[i], ASEP_ERR_BAD_ARG, "NULL handle at level %d, source %d", i / K, i % K);
+  const int dev = m[0]->model->device();
+  TView xv = view_f32(x, "x", dev);
+  ASEP_CHECK(xv.ndim >= 1 && xv.shape[0] == K, ASEP_ERR_BAD_SHAPE, "x must be [K = %d, N, H, W, C]", K);
+  float* xs[kMaxSources];
+  float* snap = run_snapshots(snapshots, xv, K, L, xs, dev);
+  for (int i = 0; i < L; ++i) {
+    const int rc = asep_basis_glow_inner_k(K, m + (size_t)(n_models == 1 ? 0 : i) * K, mixed, x, T, eta[i], lambda[i],
+                                           noise_scale[i], nullptr, seed, (uint64_t)i * (uint64_t)T, elem_offset, nullptr,
+                                           nan_count, stream);
+    if (rc != ASEP_OK) return rc;
+    snapshot_states(snap, i, K, xs, xv.numel / K, as_stream(stream));
   }
   ASEP_API_END
 }
@@ -1010,11 +1237,34 @@ int asep_basis_ncsn_run(asep_ncsn_t m1, asep_ncsn_t m2, const DLTensor* mixed, D
     ASEP_CHECK(sv.numel == (int64_t)L * 2 * a.numel, ASEP_ERR_BAD_SHAPE, "snapshots must be [L, 2, N, H, W, C]");
     snap = sv.f32;
   }
+  float* const xs[2] = {a.f32, b.f32};
   for (int i = 0; i < L; ++i) {
     const int rc = asep_basis_ncsn_inner(m1, m2, mixed, x1, x2, i, T, eta[i], lambda[i], noise_scale[i], nullptr, nullptr, seed,
                                          (uint64_t)i * (uint64_t)T, elem_offset, nullptr, nan_count, stream);
     if (rc != ASEP_OK) return rc;
-    snapshot_states(snap, i, a, b, as_stream(stream));
+    snapshot_states(snap, i, 2, xs, a.numel, as_stream(stream));
+  }
+  ASEP_API_END
+}
+
+int asep_basis_ncsn_run_k(int K, const asep_ncsn_t* m, const DLTensor* mixed, DLTensor* x, int L, int T, const float* eta,
+                          const float* lambda, const float* noise_scale, uint64_t seed, uint64_t elem_offset,
+                          DLTensor* snapshots, DLTensor* nan_count, void* stream) {
+  ASEP_API_BEGIN
+  check_sources(K);
+  ASEP_CHECK(m && eta && lambda && noise_scale, ASEP_ERR_BAD_ARG, "NULL argument");
+  ASEP_CHECK(L >= 1 && T >= 0, ASEP_ERR_BAD_ARG, "bad L / T");
+  for (int k = 0; k < K; ++k) ASEP_CHECK(m[k], ASEP_ERR_BAD_ARG, "NULL handle for source %d", k);
+  const int dev = m[0]->model->device();
+  TView xv = view_f32(x, "x", dev);
+  ASEP_CHECK(xv.ndim >= 1 && xv.shape[0] == K, ASEP_ERR_BAD_SHAPE, "x must be [K = %d, N, H, W, C]", K);
+  float* xs[kMaxSources];
+  float* snap = run_snapshots(snapshots, xv, K, L, xs, dev);
+  for (int i = 0; i < L; ++i) {
+    const int rc = asep_basis_ncsn_inner_k(K, m, mixed, x, i, T, eta[i], lambda[i], noise_scale[i], nullptr, seed,
+                                           (uint64_t)i * (uint64_t)T, elem_offset, nullptr, nan_count, stream);
+    if (rc != ASEP_OK) return rc;
+    snapshot_states(snap, i, K, xs, xv.numel / K, as_stream(stream));
   }
   ASEP_API_END
 }

@@ -70,9 +70,18 @@ void launch_actnorm(const float* x, const float* log_scale, const float* shift, 
 void launch_chanmix(const float* x, const float* w, float* y, long long M, int C, cudaStream_t s);
 
 // ---- langevin.cu
-void launch_langevin(float* x1, float* x2, const float* s1, const float* s2, const float* mixed, const float* n1,
-                     const float* n2, float eta, float lambda, float noise_scale, uint64_t seed, uint64_t step,
-                     uint64_t elem_offset, int* nan_count, long long n, cudaStream_t s);
+// BASIS separates K = 2..kMaxSources sources: the bound keeps the per-element state of the fused update in registers
+// and bounds the side streams of the step graph.
+constexpr int kMaxSources = 8;
+// Per-source pointers of one update, passed by value: states x[k] (updated in place), scores s[k] and injected standard
+// normals n[k] (all NULL for in-kernel Philox noise, source k drawing from stream k + 1).
+struct LangevinSources {
+  float* x[kMaxSources];
+  const float* s[kMaxSources];
+  const float* n[kMaxSources];
+};
+void launch_langevin(int K, const LangevinSources& p, const float* mixed, float eta, float lambda, float noise_scale,
+                     uint64_t seed, uint64_t step, uint64_t elem_offset, int* nan_count, long long n, cudaStream_t s);
 // Device-resident scalars of one Langevin step (see k_langevin<.., kDev>): written by the host before a run of graph
 // replays, advanced (step, t) by the kernel pair itself after every step.
 struct LangevinDev {
@@ -80,11 +89,16 @@ struct LangevinDev {
   unsigned long long step;     // Philox step number of the next update
   unsigned long long t;        // index of the next update inside the injected-noise / dump tensors
 };
-// as launch_langevin with the per-step scalars in *dev; n1/n2/dump are the BASES of the [T, ...] tensors (or NULL)
-void launch_langevin_dev(float* x1, float* x2, const float* s1, const float* s2, const float* mixed, const float* n1,
-                         const float* n2, float* dump, LangevinDev* dev, uint64_t seed, uint64_t elem_offset, int* nan_count,
-                         long long n, cudaStream_t s);
-void launch_mixing_db(const float* x1, const float* x2, float* g, float* w1, float* w2, long long n, cudaStream_t s);
+// as launch_langevin with the per-step scalars in *dev; p.n[k] is the base of source k's injected noise (step t at
+// p.n[k] + t * noise_stride), dump the base of the [T, K, ...] per-step dump (or NULL)
+void launch_langevin_dev(int K, const LangevinSources& p, const float* mixed, long long noise_stride, float* dump,
+                         LangevinDev* dev, uint64_t seed, uint64_t elem_offset, int* nan_count, long long n, cudaStream_t s);
+// g = (10/ln10)(logsumexp_k(x_k ln10/10) - ln K) and w_k = softmax_k of the K inputs x[k]
+struct MixingSources {
+  const float* x[kMaxSources];
+  float* w[kMaxSources];
+};
+void launch_mixing_db(int K, const MixingSources& p, float* g, long long n, cudaStream_t s);
 void launch_philox_normal(float* out, uint64_t seed, uint64_t step, uint64_t stream_id, uint64_t elem_offset,
                           long long n, cudaStream_t s);
 

@@ -91,6 +91,12 @@ def get_song_extract(mix_path, piano_path, violin_path, duration, **kwargs):
     """reference: datasets/data_loader.py:113-180.  Returns (mel_spec, raw_audio, stft_mixture):
     mel_spec = [mix, piano, violin], each float32 [n_extract, n_mels, T, 1]; raw_audio = the three concatenated
     waveforms; stft_mixture complex64 [n_extract, 1 + n_fft/2, T]."""
+    return get_song_extract_k(mix_path, [piano_path, violin_path], duration, **kwargs)
+
+
+def get_song_extract_k(mix_path, source_paths, duration, **kwargs):
+    """get_song_extract for any number of stems: mel_spec = [mix, s_1, ..., s_K] and raw_audio the K + 1 concatenated
+    waveforms, in the order of ``source_paths``."""
     length_sec = kwargs["length_sec"]
     fmin, fmax, sr = kwargs["fmin"], kwargs["fmax"], kwargs["sr"]
     dbmin, dbmax = kwargs["dbmin"], kwargs["dbmax"]
@@ -100,7 +106,7 @@ def get_song_extract(mix_path, piano_path, violin_path, duration, **kwargs):
         raise NotImplementedError("power-scale mel spectrograms (use_dB=False) are not on the separation path of the configs")
     n_extract = int(round(duration / length_sec, 0))
     tracks = []
-    for p in (mix_path, piano_path, violin_path):
+    for p in [mix_path] + list(source_paths):
         frames, _ = load_wav(p, length_sec, sr=sr)
         if frames.shape[0] < 2 + n_extract:
             raise ValueError(f"{p}: {frames.shape[0]} windows of {length_sec} s, {2 + n_extract} needed (the first two are skipped)")

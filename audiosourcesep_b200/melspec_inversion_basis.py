@@ -7,6 +7,7 @@ from __future__ import annotations
 
 import argparse
 import os
+import re
 import time
 import wave
 
@@ -75,27 +76,31 @@ def main(args):
     os.makedirs(out_dir, exist_ok=True)
     if args.algorithm not in ("reuse_phase", "griffin"):
         raise ValueError("method should be griffin or reuse_phase")                 # :197-198
-    x1, x2, gt1, gt2, mix, stft_mixture = (res[k] for k in ("x1", "x2", "gt1", "gt2", "mixed", "stft_mixture"))
-    assert x1.ndim == x2.ndim == stft_mixture.ndim == 3, (x1.shape, x2.shape, stft_mixture.shape)
+    K = sum(1 for k in res.files if re.fullmatch(r"x[0-9]+", k))                   # one x{k} / gt{k} pair per source
+    xs = [res[f"x{k + 1}"] for k in range(K)]
+    gts = [res[f"gt{k + 1}"] for k in range(K)]
+    mix, stft_mixture = res["mixed"], res["stft_mixture"]
+    assert all(x.ndim == 3 for x in xs) and stft_mixture.ndim == 3, ([x.shape for x in xs], stft_mixture.shape)
     if args.method == "whole":                                                     # :164-170: one long spectrogram
         cat = lambda a: np.concatenate(list(a), axis=-1)[None]
-        x1, x2, gt1, gt2, mix, stft_mixture = (cat(a) for a in (x1, x2, gt1, gt2, mix, stft_mixture))
+        xs, gts, mix, stft_mixture = [cat(a) for a in xs], [cat(a) for a in gts], cat(mix), cat(stft_mixture)
     t0 = time.time()
     if args.algorithm == "griffin":                                                # :173-183
         gfn = griffin_inversion_fn(sr, fmin, fmax, n_fft, hop_length, args.scale)
-        x1_inv, x2_inv = gfn([x1, x2])
-        gt1_inv, gt2_inv = gfn([gt1, gt2])
+        x_inv = gfn(xs)
+        gt_inv = gfn(gts)
         mix_inv = gfn([mix])[0]
     else:
         fn = stft_inversion_fn(sr, fmin, fmax, n_fft, hop_length, args.scale, args.wiener_filter)
-        x1_inv, x2_inv = fn(([x1, x2], stft_mixture))
-        gt1_inv, gt2_inv = fn(([gt1, gt2], stft_mixture))
+        x_inv = fn((xs, stft_mixture))
+        gt_inv = fn((gts, stft_mixture))
         mix_inv = fn(([mix], stft_mixture))[0]
     torch.cuda.synchronize()
     print("Inversion duration: {} seconds".format(round(time.time() - t0, 4)))
-    flat = {k: np.concatenate(list(v), axis=-1) for k, v in (("x1_audio", x1_inv), ("x2_audio", x2_inv), ("gt1_audio", gt1_inv),
-                                                              ("gt2_audio", gt2_inv), ("mix_audio", mix_inv))}
-    for name, key in (("sep1", "x1_audio"), ("sep2", "x2_audio"), ("gt1", "gt1_audio"), ("gt2", "gt2_audio"), ("mix", "mix_audio")):
+    items = [(f"x{k + 1}_audio", x_inv[k]) for k in range(K)] + [(f"gt{k + 1}_audio", gt_inv[k]) for k in range(K)]
+    flat = {k: np.concatenate(list(v), axis=-1) for k, v in items + [("mix_audio", mix_inv)]}
+    names = [(f"sep{k + 1}", f"x{k + 1}_audio") for k in range(K)] + [(f"gt{k + 1}", f"gt{k + 1}_audio") for k in range(K)]
+    for name, key in names + [("mix", "mix_audio")]:
         write_wav(os.path.join(out_dir, name + ".wav"), flat[key], sr)
     np.savez(os.path.join(out_dir, "inverse_spectrograms"), **flat)
     return flat

@@ -146,3 +146,92 @@ def basis_run(m1, m2, mixed, x1, x2, T: int, eta, lam, noise_scale, seed: int = 
     else:
         _lib.check(_lib.load().asep_basis_ncsn_run(m1.handle, m2.handle, t[0].ptr, t[1].ptr, t[2].ptr, L, int(T), arr[0], arr[1],
                                                    arr[2], int(seed), int(elem_offset), dsn.ptr, dnan.ptr, _lib.stream_ptr()))
+
+
+# ---- K sources (2 <= K <= 8): stacked [K, ...] states, [T, K, ...] noise / per-step dumps, [L, K, ...] snapshots
+def _state_k(x) -> None:
+    if not (x.is_cuda and x.dtype == torch.float32 and x.is_contiguous()):
+        raise ValueError("x must be a contiguous float32 CUDA tensor [K, ...] (updated in place)")
+
+
+def _handles(models):
+    import ctypes
+    return (ctypes.c_void_p * len(models))(*[m.handle.value for m in models])
+
+
+def mixing_db_k(x):
+    """g(x_1..x_K) and grad_g = softmax_k of a stacked ``x`` [K, ...] (reference: run_basis_sep.py:106-149)."""
+    x = _prep(x)
+    g, w = torch.empty_like(x[0]), torch.empty_like(x)
+    t = [_lib.dl(v) for v in (x, g, w)]
+    _lib.check(_lib.load().asep_mixing_db_k(int(x.shape[0]), *(v.ptr for v in t), _lib.stream_ptr()))
+    return g, w
+
+
+def langevin_step_k(x, score, mixed, eta: float, lam: float, noise_scale: float, noise: Optional[torch.Tensor] = None,
+                    seed: int = 0, step: int = 0, elem_offset: int = 0, nan_count: Optional[torch.Tensor] = None) -> None:
+    """In-place fused update of all K sources of ``x`` [K, ...] (reference: run_basis_sep.py:163-181); ``noise``: NULL
+    (Philox, source k on stream k + 1) or [K, ...] standard normals."""
+    _state_k(x)
+    score, mixed = _prep(score), _prep(mixed)
+    noise = None if noise is None else _prep(noise)
+    t = [_lib.dl(v) for v in (x, score, mixed, noise, nan_count)]
+    _lib.check(_lib.load().asep_langevin_step_k(int(x.shape[0]), t[0].ptr, t[1].ptr, t[2].ptr, t[3].ptr, float(eta),
+                                                float(lam), float(noise_scale), int(seed), int(step), int(elem_offset),
+                                                t[4].ptr, _lib.stream_ptr()))
+
+
+def basis_glow_inner_k(models, mixed, x, T: int, eta: float, lam: float, noise_scale: float, noise=None, seed: int = 0,
+                       step0: int = 0, elem_offset: int = 0, per_step: Optional[torch.Tensor] = None,
+                       nan_count: Optional[torch.Tensor] = None) -> None:
+    """T Langevin steps at one noise level with K Glow priors (``models[k]`` for source k of ``x`` [K, ...])."""
+    _state_k(x)
+    mixed = _prep(mixed)
+    noise = None if noise is None else _prep(noise)
+    t = [_lib.dl(v) for v in (mixed, x, noise, per_step, nan_count)]
+    _lib.check(_lib.load().asep_basis_glow_inner_k(len(models), _handles(models), t[0].ptr, t[1].ptr, int(T), float(eta),
+                                                   float(lam), float(noise_scale), t[2].ptr, int(seed), int(step0),
+                                                   int(elem_offset), t[3].ptr, t[4].ptr, _lib.stream_ptr()))
+
+
+def basis_ncsn_inner_k(models, mixed, x, sigma_idx: int, T: int, eta: float, lam: float, noise_scale: float, noise=None,
+                       seed: int = 0, step0: int = 0, elem_offset: int = 0, per_step: Optional[torch.Tensor] = None,
+                       nan_count: Optional[torch.Tensor] = None) -> None:
+    """T Langevin steps at noise level ``sigma_idx`` with K score networks (``models[k]`` for source k of ``x``)."""
+    _state_k(x)
+    mixed = _prep(mixed)
+    noise = None if noise is None else _prep(noise)
+    t = [_lib.dl(v) for v in (mixed, x, noise, per_step, nan_count)]
+    _lib.check(_lib.load().asep_basis_ncsn_inner_k(len(models), _handles(models), t[0].ptr, t[1].ptr, int(sigma_idx),
+                                                   int(T), float(eta), float(lam), float(noise_scale), t[2].ptr, int(seed),
+                                                   int(step0), int(elem_offset), t[3].ptr, t[4].ptr, _lib.stream_ptr()))
+
+
+def basis_run_k(models, mixed, x, T: int, eta, lam, noise_scale, seed: int = 0, elem_offset: int = 0,
+                snapshots: Optional[torch.Tensor] = None, nan_count: Optional[torch.Tensor] = None) -> None:
+    """The whole sigma x T loop over K sources inside the library (reference: run_basis_sep.py:217-260).  ``models``: K
+    score networks, K Glow priors, or L lists of K Glow priors (one fine-tuned set per noise level); ``snapshots``:
+    NULL or [L, K, ...]."""
+    import ctypes
+    _state_k(x)
+    L = len(eta)
+    arr = [(ctypes.c_float * L)(*[float(v) for v in seq]) for seq in (eta, lam, noise_scale)]
+    mixed = _prep(mixed)
+    t = [_lib.dl(v) for v in (mixed, x, snapshots, nan_count)]
+    per_level = isinstance(models[0], (list, tuple))
+    first = models[0][0] if per_level else models[0]
+    if hasattr(first, "cfg") and hasattr(first.cfg, "K"):                 # Glow priors
+        sets = [list(s) for s in models] if per_level else [list(models)]
+        K = len(sets[0])
+        if any(len(s) != K for s in sets):
+            raise ValueError("every noise level needs the same number of priors")
+        flat = [m for s in sets for m in s]
+        _lib.check(_lib.load().asep_basis_glow_run_k(K, _handles(flat), len(sets), t[0].ptr, t[1].ptr, L, int(T), arr[0],
+                                                     arr[1], arr[2], int(seed), int(elem_offset), t[2].ptr, t[3].ptr,
+                                                     _lib.stream_ptr()))
+    else:
+        if per_level:
+            raise ValueError("per-level model lists are a Glow feature; score networks are conditioned on the level")
+        _lib.check(_lib.load().asep_basis_ncsn_run_k(len(models), _handles(models), t[0].ptr, t[1].ptr, L, int(T), arr[0],
+                                                     arr[1], arr[2], int(seed), int(elem_offset), t[2].ptr, t[3].ptr,
+                                                     _lib.stream_ptr()))

@@ -20,6 +20,11 @@ Differences from the shipped script, all forced by its defects (SURVEY.md App. D
   get_song_extract, as in the reference), from ``<song_dir>/{mix,piano,violin}.npy`` (dB, ``[n,96,64]``), or are generated
   with ``--synthetic``.
 
+Beyond the reference, K = 2..8 sources are separated: one prior per restore directory (``RESTORE1 RESTORE2 [RESTORE ...]``,
+all of one ``model_type``), the stems named by ``--sources`` (``piano,violin`` by default, for K = 2), and
+``results.npz`` / ``results_convergence.npz`` holding ``x1..xK`` (and ``gt1..gtK``).  The loop works on one stacked state
+``[K, n, H, W, 1]`` (basis_inner_loop_k / basis_outer_loop_k); the two-source functions are its K = 2 case.
+
 Segments are independent (SURVEY.md 8(e)): under ``torchrun`` every rank separates a contiguous block of
 segments with noise keyed by the GLOBAL element index, and rank 0 gathers the blocks at the end -- the
 only cross-GPU traffic.
@@ -103,117 +108,150 @@ def mixing_process(args):
     return g, grad_g
 
 
+def basis_inner_loop_k(mixed, x, models, sigma_idx, sigmas, g=None, grad_g=None, post_processing=None, model_type="ncsn",
+                       delta=2e-5, T=100, debug=True, train_summary_writer=None, step=None, noise=None, seed=0,
+                       elem_offset=0, per_step=None, **kwargs):
+    """T fused Langevin updates of K sources at noise level ``sigma_idx`` (reference: run_basis_sep.py:152-214).
+
+    ``x`` [K, n, H, W, 1] is a CUDA tensor updated IN PLACE and returned; ``models[k]`` is the prior of source k.
+    ``noise`` ([T, K, n, H, W, 1] standard normals) injects the draws for parity runs; otherwise Philox noise keyed by
+    (seed, global step, global element index) is generated inside the kernel, source k on stream k + 1."""
+    import torch
+    from . import ops
+    eta, lam, ns = langevin_step_constants(sigmas, sigma_idx, delta)
+    step0 = int(sigma_idx) * int(T)
+    nan = torch.zeros(1, dtype=torch.int32, device=x.device) if debug else None
+    if model_type == "glow":
+        ops.basis_glow_inner_k(models, mixed, x, int(T), float(eta), float(lam), float(ns), noise=noise, seed=seed,
+                               step0=step0, elem_offset=elem_offset, per_step=per_step, nan_count=nan)
+    elif all(hasattr(m, "handle") for m in models):
+        ops.basis_ncsn_inner_k(models, mixed, x, int(sigma_idx), int(T), float(eta), float(lam), float(ns), noise=noise,
+                               seed=seed, step0=step0, elem_offset=elem_offset, per_step=per_step, nan_count=nan)
+    else:                                                              # any callable score model (plug-in seam)
+        n = x.shape[1]
+        idx = torch.full((n,), int(sigma_idx), dtype=torch.int32, device=x.device)
+        for t in range(int(T)):
+            s = torch.stack([m([x[k], idx], training=True) for k, m in enumerate(models)])   # run_basis_sep.py:167-170
+            ops.langevin_step_k(x, s, mixed, float(eta), float(lam), float(ns), noise=None if noise is None else noise[t],
+                                seed=seed, step=step0 + t, elem_offset=elem_offset, nan_count=nan)
+            if per_step is not None:
+                per_step[t].copy_(x)
+    if debug and int(nan.item()) != 0:                                 # the reference's --debug NaN asserts, :183-191
+        raise FloatingPointError(f"NaN in the Langevin state at sigma index {sigma_idx}")
+    return x
+
+
 def basis_inner_loop(mixed, x1, x2, model1, model2, sigma_idx, sigmas, g=None, grad_g=None, post_processing=None,
                      model_type="ncsn", delta=2e-5, T=100, debug=True, train_summary_writer=None, step=None,
                      noise1=None, noise2=None, seed=0, elem_offset=0, per_step=None, **kwargs):
-    """T fused Langevin updates at noise level ``sigma_idx`` (reference: run_basis_sep.py:152-214).
+    """T fused Langevin updates at noise level ``sigma_idx`` (reference: run_basis_sep.py:152-214): basis_inner_loop_k
+    with K = 2.
 
     x1 / x2 are CUDA tensors updated IN PLACE and returned.  ``noise1/noise2`` ([T, n, H, W, 1] standard
     normals) inject the draws for parity runs; otherwise Philox noise keyed by (seed, global step, global
     element index) is generated inside the kernel."""
     import torch
-    from . import ops
-    eta, lam, ns = langevin_step_constants(sigmas, sigma_idx, delta)
-    step0 = int(sigma_idx) * int(T)
-    nan = torch.zeros(1, dtype=torch.int32, device=x1.device) if debug else None
-    if model_type == "glow":
-        ops.basis_glow_inner(model1, model2, mixed, x1, x2, int(T), float(eta), float(lam), float(ns), noise1=noise1,
-                             noise2=noise2, seed=seed, step0=step0, elem_offset=elem_offset, per_step=per_step,
-                             nan_count=nan)
-    elif hasattr(model1, "handle") and hasattr(model2, "handle"):
-        ops.basis_ncsn_inner(model1, model2, mixed, x1, x2, int(sigma_idx), int(T), float(eta), float(lam), float(ns),
-                             noise1=noise1, noise2=noise2, seed=seed, step0=step0, elem_offset=elem_offset,
-                             per_step=per_step, nan_count=nan)
-    else:                                                              # any callable score model (plug-in seam)
-        n = x1.shape[0]
-        idx = torch.full((n,), int(sigma_idx), dtype=torch.int32, device=x1.device)
-        for t in range(int(T)):
-            s1 = model1([x1, idx], training=True)                     # run_basis_sep.py:167-170
-            s2 = model2([x2, idx], training=True)
-            ops.langevin_step(x1, x2, s1, s2, mixed, float(eta), float(lam), float(ns),
-                              n1=None if noise1 is None else noise1[t], n2=None if noise2 is None else noise2[t],
-                              seed=seed, step=step0 + t, elem_offset=elem_offset, nan_count=nan)
-            if per_step is not None:
-                per_step[t, 0].copy_(x1)
-                per_step[t, 1].copy_(x2)
-    if debug and int(nan.item()) != 0:                                 # the reference's --debug NaN asserts, :183-191
-        raise FloatingPointError(f"NaN in the Langevin state at sigma index {sigma_idx}")
+    x = torch.stack([x1, x2])
+    noise = None if noise1 is None else torch.stack([torch.as_tensor(noise1), torch.as_tensor(noise2)], 1)
+    try:
+        basis_inner_loop_k(mixed, x, [model1, model2], sigma_idx, sigmas, model_type=model_type, delta=delta, T=T, debug=debug,
+                           noise=noise, seed=seed, elem_offset=elem_offset, per_step=per_step)
+    finally:
+        x1.copy_(x[0])
+        x2.copy_(x[1])
     return x1, x2
 
 
-def basis_outer_loop(mixed, x1, x2, model1, model2, optimizer, sigmas, ckpt1, ckpt2, args, train_summary_writer=None):
-    """reference: run_basis_sep.py:217-260.  ``ckpt1/ckpt2`` are callables ``sigma -> params dict or None``
-    that supply the per-noise-level Glow weights (the reference restores a checkpoint per sigma, :228-234)."""
-    x_arr = {"x1": [x1.detach().cpu().numpy().copy()], "x2": [x2.detach().cpu().numpy().copy()]}
-    device_loop = (not getattr(args, "host_loop", False) and hasattr(model1, "handle") and hasattr(model2, "handle")
-                   and (args.model_type == "ncsn" or (ckpt1 is None and ckpt2 is None)))
+def basis_outer_loop_k(mixed, x, models, optimizer, sigmas, ckpts, args, train_summary_writer=None):
+    """reference: run_basis_sep.py:217-260 for K sources: ``x`` [K, n, H, W, 1] is updated in place.  ``ckpts[k]`` is a
+    callable ``sigma -> params dict or None`` that supplies the per-noise-level Glow weights of prior k (the reference
+    restores a checkpoint per sigma, :228-234), or None.  Returns (x, x_arr) with x_arr = {"x1": [...], ..., "xK": [...]}."""
+    K = len(models)
+    x_arr = {f"x{k + 1}": [x[k].detach().cpu().numpy().copy()] for k in range(K)}
+    ckpts = list(ckpts) if ckpts is not None else [None] * K
+    device_loop = (not getattr(args, "host_loop", False) and all(hasattr(m, "handle") for m in models)
+                   and (args.model_type == "ncsn" or all(c is None for c in ckpts)))
     if device_loop:
-        # the whole sigma x T loop inside the library (asep_basis_ncsn_run / asep_basis_glow_run): no host round trip
+        # the whole sigma x T loop inside the library (asep_basis_ncsn_run_k / asep_basis_glow_run_k): no host round trip
         # between noise levels, the per-level snapshots are copied on the stream and read once at the end
         import torch
         from . import ops
         L = len(sigmas)
         consts = [langevin_step_constants(sigmas, i, 2e-5) for i in range(L)]
-        snaps = torch.empty((L, 2) + tuple(x1.shape), dtype=torch.float32, device=x1.device)
-        nan = torch.zeros(1, dtype=torch.int32, device=x1.device) if args.debug else None
+        snaps = torch.empty((L,) + tuple(x.shape), dtype=torch.float32, device=x.device)
+        nan = torch.zeros(1, dtype=torch.int32, device=x.device) if args.debug else None
         for sigma_idx, sigma in enumerate(sigmas):
             print("Sigma = {} ({} / {})".format(sigma, sigma_idx + 1, L))
-        ops.basis_run(model1, model2, mixed, x1, x2, int(args.T), [c[0] for c in consts], [c[1] for c in consts],
-                      [c[2] for c in consts], seed=getattr(args, "seed", 0), elem_offset=getattr(args, "elem_offset", 0),
-                      snapshots=snaps, nan_count=nan)
+        ops.basis_run_k(models, mixed, x, int(args.T), [c[0] for c in consts], [c[1] for c in consts], [c[2] for c in consts],
+                        seed=getattr(args, "seed", 0), elem_offset=getattr(args, "elem_offset", 0), snapshots=snaps,
+                        nan_count=nan)
         if args.debug and int(nan.item()) != 0:
             raise FloatingPointError("NaN in the Langevin state")
         host = snaps.cpu().numpy()
         for i in range(L):
-            x_arr["x1"].append(host[i, 0].copy())
-            x_arr["x2"].append(host[i, 1].copy())
+            for k in range(K):
+                x_arr[f"x{k + 1}"].append(host[i, k].copy())
         print("inner loop done")
         print("_" * 100)
-        return x1, x2, x_arr
+        return x, x_arr
     for sigma_idx, sigma in enumerate(sigmas):
         print("Sigma = {} ({} / {})".format(sigma, sigma_idx + 1, len(sigmas)))
         if args.model_type == "glow":
-            for m, ck, tag in ((model1, ckpt1, 1), (model2, ckpt2, 2)):
+            for tag, (m, ck) in enumerate(zip(models, ckpts), start=1):
                 p = ck(float(sigma)) if ck is not None else None
                 if p is not None:
                     m.set_params(p)
                     m.prepare()
                     print("Model {} at noise level {} restored".format(tag, sigma))
-        x1, x2 = basis_inner_loop(mixed, x1, x2, model1, model2, sigma_idx, sigmas, model_type=args.model_type,
-                                  delta=2e-5, T=args.T, debug=args.debug, seed=getattr(args, "seed", 0),
-                                  elem_offset=getattr(args, "elem_offset", 0))
-        x_arr["x1"].append(x1.detach().cpu().numpy().copy())
-        x_arr["x2"].append(x2.detach().cpu().numpy().copy())
+        basis_inner_loop_k(mixed, x, models, sigma_idx, sigmas, model_type=args.model_type, delta=2e-5, T=args.T,
+                           debug=args.debug, seed=getattr(args, "seed", 0), elem_offset=getattr(args, "elem_offset", 0))
+        for k in range(K):
+            x_arr[f"x{k + 1}"].append(x[k].detach().cpu().numpy().copy())
         print("inner loop done")
         print("_" * 100)
+    return x, x_arr
+
+
+def basis_outer_loop(mixed, x1, x2, model1, model2, optimizer, sigmas, ckpt1, ckpt2, args, train_summary_writer=None):
+    """reference: run_basis_sep.py:217-260: basis_outer_loop_k with K = 2.  ``ckpt1/ckpt2`` are callables
+    ``sigma -> params dict or None`` that supply the per-noise-level Glow weights (the reference restores a checkpoint
+    per sigma, :228-234)."""
+    import torch
+    x = torch.stack([x1, x2])
+    try:
+        x, x_arr = basis_outer_loop_k(mixed, x, [model1, model2], optimizer, sigmas, [ckpt1, ckpt2], args, train_summary_writer)
+    finally:
+        x1.copy_(x[0])
+        x2.copy_(x[1])
     return x1, x2, x_arr
 
 
 # --------------------------------------------------------------------------------------- data / weights
 def load_song_patches(args):
-    """(mixed_db, gt1_db, gt2_db, stft_mixture) as float32 [n_mixed, H, W, 1] in dB."""
+    """(mixed_db, [gt_1_db, ..., gt_K_db], stft_mixture) as float32 [n_mixed, H, W, 1] in dB, one ground truth per source
+    (source_names)."""
     from . import synthetic
     n = int(args.n_mixed)
+    names = source_names(args)
     if getattr(args, "synthetic", False) or args.song_dir is None:
         if args.song_dir is None and not getattr(args, "synthetic", False):
             raise ValueError("song_dir is None")                       # run_basis_sep.py:300-301
-        gt1 = synthetic.mel_patches_db(n, 0, args.height, args.width)
-        gt2 = synthetic.mel_patches_db(n, 1, args.height, args.width)
-        mix = synthetic.mixture_db(gt1, gt2)
-        return mix, gt1, gt2, np.zeros((n, 1025, args.width), np.complex64)
+        gts = [synthetic.mel_patches_db(n, k, args.height, args.width) for k in range(len(names))]
+        return synthetic.mixture_db(*gts), gts, np.zeros((n, 1025, args.width), np.complex64)
     d = os.path.abspath(args.song_dir)
     if os.path.exists(os.path.join(d, "mix.wav")):                    # the reference's own input (run_basis_sep.py:342-351)
         from .datasets import data_loader
         spec_params = {"length_sec": 2.04, "dbmin": -100, "dbmax": 20, "fmin": 125, "fmax": 7600, "use_dB": True, "n_fft": 2048,
                        "hop_length": 512, "n_mels": 96, "sr": 16000}
-        mel_spec, _, stft_mixture = data_loader.get_song_extract(os.path.join(d, "mix.wav"), os.path.join(d, "piano.wav"),
-                                                                 os.path.join(d, "violin.wav"), 2.04 * n, **spec_params)
-        mix, gt1, gt2 = (m.cpu().numpy() for m in mel_spec)
+        mel_spec, _, stft_mixture = data_loader.get_song_extract_k(os.path.join(d, "mix.wav"),
+                                                                   [os.path.join(d, nm + ".wav") for nm in names], 2.04 * n,
+                                                                   **spec_params)
+        mix, *gts = (m.cpu().numpy() for m in mel_spec)
         if mix.shape[1:] != (args.height, args.width, 1):
             raise ValueError(f"mel patches of shape {mix.shape[1:]}, the model expects {(args.height, args.width, 1)}")
-        return mix, gt1, gt2, stft_mixture
+        return mix, gts, stft_mixture
     arrs = []
-    for name in ("mix", "piano", "violin"):
+    for name in ["mix"] + names:
         a = np.load(os.path.join(d, name + ".npy")).astype(np.float32)
         if a.ndim == 3:
             a = a[..., None]
@@ -222,7 +260,7 @@ def load_song_patches(args):
         arrs.append(a[:n])
     stft_path = os.path.join(d, "stft_mixture.npy")
     stft = np.load(stft_path)[:n] if os.path.exists(stft_path) else np.zeros((n, 1025, args.width), np.complex64)
-    return arrs[0], arrs[1], arrs[2], stft
+    return arrs[0], arrs[1:], stft
 
 
 def load_weights(directory: str, shapes: Dict[str, tuple]) -> Dict[str, np.ndarray]:
@@ -269,15 +307,17 @@ def glow_precision(args) -> int:
 
 
 def build_models(args, sigmas, device_index: int):
-    """Two priors (reference: run_basis_sep.py:386-397) and their per-sigma weight suppliers."""
+    """One prior per restore directory (reference: run_basis_sep.py:386-397) and their per-sigma weight suppliers:
+    (models, ckpts), both of length K."""
     from . import _lib
     from .flow_models.flow_builder import build_glow
     from .weights import init_glow_params
+    restores = restore_dirs(args)
     if args.model_type == "glow":
         cfg = GlowConfig(H=args.height, W=args.width, C=1, L=args.L, K=args.K, n_filters=args.n_filters,
                          learntop=bool(args.learntop), minval=0.0, maxval=1.0)
         models, ckpts = [], []
-        for i, restore in enumerate((args.RESTORE1, args.RESTORE2)):
+        for i, restore in enumerate(restores):
             if args.random_init is not None:
                 params = init_glow_params(cfg, seed=int(args.random_init) + i, mode="perturbed")
                 ckpts.append(None)
@@ -288,10 +328,10 @@ def build_models(args, sigmas, device_index: int):
             models.append(build_glow(None, [args.height, args.width, 1], L=args.L, K=args.K, n_filters=args.n_filters,
                                      learntop=args.learntop, l2_reg=args.l2_reg, data_type="melspec", minval=0.0,
                                      maxval=1.0, use_logit=False, params=params, precision=glow_precision(args)))
-        return models[0], models[1], ckpts[0], ckpts[1]
+        return models, ckpts
     from .ncsn.utils import get_uncompiled_model, get_uncompiled_model_v2
     builders = []
-    for i, restore in enumerate((args.RESTORE1, args.RESTORE2)):
+    for i, restore in enumerate(restores):
         params = None
         if args.random_init is None:
             from .ncsn.utils import _ncsn_cfg
@@ -303,15 +343,47 @@ def build_models(args, sigmas, device_index: int):
         else:
             builders.append(get_uncompiled_model_v2(args, sigmas=sigmas, name=f"model{i + 1}", params=params,
                                                     seed=None if args.random_init is None else int(args.random_init) + i))
-    return builders[0], builders[1], None, None
+    return builders, [None] * len(builders)
+
+
+# --------------------------------------------------------------------------------------- sources
+MAX_SOURCES = 8                     # the fused update keeps the state of every source in registers (csrc/langevin.cu)
+
+
+def restore_dirs(args) -> List[str]:
+    """The K restore directories, one prior per source: RESTORE1 RESTORE2 [RESTORE ...]."""
+    dirs = [args.RESTORE1, args.RESTORE2] + list(getattr(args, "RESTORE", None) or [])
+    if len(dirs) > MAX_SOURCES:
+        raise ValueError(f"BASIS separates at most {MAX_SOURCES} sources; {len(dirs)} restore directories were given")
+    return dirs
+
+
+def source_names(args) -> List[str]:
+    """Stem names of the K sources (``--sources``): ``<song_dir>/<name>.wav`` or ``.npy``.  The default piano,violin is
+    the reference's two-source layout; with more sources and a song directory, --sources is required."""
+    K = len(restore_dirs(args))
+    spec = getattr(args, "sources", None)
+    if spec is None:
+        if K == 2:
+            return ["piano", "violin"]
+        if args.song_dir is not None and not getattr(args, "synthetic", False):
+            raise ValueError(f"--sources is required to name the {K} stems in --song_dir")
+        return [f"source{k + 1}" for k in range(K)]
+    names = [nm.strip() for nm in spec.split(",")]
+    if len(names) != K or not all(names):
+        raise ValueError(f"--sources names {len(names)} stems ({spec!r}), but there are {K} restore directories")
+    return names
 
 
 # --------------------------------------------------------------------------------------- main
 def build_parser() -> argparse.ArgumentParser:
-    """The reference's flags (run_basis_sep.py:453-523) plus --synthetic / --random_init / --seed."""
+    """The reference's flags (run_basis_sep.py:453-523) plus --synthetic / --random_init / --seed, and K sources:
+    RESTORE1 RESTORE2 [RESTORE ...] with --sources."""
     p = argparse.ArgumentParser(description="BASIS Separatation")
     p.add_argument("RESTORE1", type=str, default=None, help="directory of saved model1")
     p.add_argument("RESTORE2", type=str, default=None, help="directory of saved model2")
+    p.add_argument("RESTORE", type=str, nargs="*", default=[],
+                   help="directories of the priors of sources 3..K (K <= 8): one prior per source")
     p.add_argument("--output", type=str, default="basis_sep")
     p.add_argument("--debug", action="store_true")
     p.add_argument("--dataset", type=str, default="melspec")
@@ -350,6 +422,8 @@ def build_parser() -> argparse.ArgumentParser:
                    help="Glow priors: fp32 | bf16 | fp16 | bf16x2 | fp16x2 | fp16x3 (overrides --fast / --exact)")
     p.add_argument("--exact", action="store_true",
                    help="Glow priors on the fp32 CUDA-core kernels (the on-device checker); score networks: the parity mode")
+    p.add_argument("--sources", type=str, default=None, metavar="NAME,...",
+                   help="stem names of the K sources in --song_dir (<name>.wav or <name>.npy); default piano,violin (K = 2)")
     p.add_argument("--host_loop", action="store_true",
                    help="run the sigma loop on the host (one library call per noise level) instead of asep_basis_*_run")
     return p
@@ -361,7 +435,7 @@ def merge_config(args: argparse.Namespace) -> argparse.Namespace:
         return args
     cfg = vars(get_config(args.config))
     keep = ("dataset", "debug", "output", "song_dir", "inverse", "model_type", "n_mixed", "RESTORE1", "RESTORE2",
-            "synthetic", "random_init", "seed", "config", "fast", "precision", "exact", "host_loop")
+            "synthetic", "random_init", "seed", "config", "fast", "precision", "exact", "host_loop", "RESTORE", "sources")
     merged = dict(vars(args))
     for k, v in cfg.items():
         if k not in keep:
@@ -408,20 +482,19 @@ def main(args) -> Optional[Dict[str, np.ndarray]]:
         sys.stdout = open(os.devnull, "w")
     try:
         t0 = time.time()
-        mix_db, gt1, gt2, stft_mixture = load_song_patches(args)
+        mix_db, gts, stft_mixture = load_song_patches(args)
+        K = len(gts)
         n = mix_db.shape[0]
         lo, hi = shard_range(n, world, rank)
         mixed_full = ((mix_db - args.minval) / (args.maxval - args.minval)).astype(np.float32)   # :355
         rng = np.random.Generator(np.random.PCG64(args.seed))
-        x1_full = rng.uniform(0.0, 1.0, mixed_full.shape).astype(np.float32)                    # :360-361
-        x2_full = rng.uniform(0.0, 1.0, mixed_full.shape).astype(np.float32)
+        x_full = np.stack([rng.uniform(0.0, 1.0, mixed_full.shape).astype(np.float32) for _ in range(K)])   # :360-361
         mixed = torch.as_tensor(mixed_full[lo:hi]).to(dev)
-        x1 = torch.as_tensor(x1_full[lo:hi]).to(dev)
-        x2 = torch.as_tensor(x2_full[lo:hi]).to(dev)
+        x = torch.as_tensor(np.ascontiguousarray(x_full[:, lo:hi])).to(dev)
         args.elem_offset = lo * args.height * args.width
         print("Data Loaded in {} seconds".format(round(time.time() - t0, 3)))
         post_processing = post_processing_fn(args)
-        model1, model2, ckpt1, ckpt2 = build_models(args, sigmas, local_rank)
+        models, ckpts = build_models(args, sigmas, local_rank)
         template = "BASIS Separation \n\t "
         for k, v in vars(args).items():
             template += "{} = {} \n\t ".format(k, v)
@@ -429,24 +502,23 @@ def main(args) -> Optional[Dict[str, np.ndarray]]:
         torch.cuda.synchronize()
         t0 = time.time()
         if hi > lo:
-            x1, x2, x_arr = basis_outer_loop(mixed, x1, x2, model1, model2, None, sigmas, ckpt1, ckpt2, args, None)
+            x, x_arr = basis_outer_loop_k(mixed, x, models, None, sigmas, ckpts, args, None)
         else:
-            x_arr = {"x1": [x1.cpu().numpy()] * (len(sigmas) + 1), "x2": [x2.cpu().numpy()] * (len(sigmas) + 1)}
+            x_arr = {f"x{k + 1}": [x[k].cpu().numpy()] * (len(sigmas) + 1) for k in range(K)}
         torch.cuda.synchronize()
         t1 = time.time()
         print("Duration: {} seconds".format(round(t1 - t0, 3)))
         # final gather: the only cross-GPU traffic (SURVEY.md 8(e))
-        x1_all = gather_segments(x1.cpu().numpy(), n)
-        x2_all = gather_segments(x2.cpu().numpy(), n)
-        conv1 = gather_segments(np.array(x_arr["x1"]), n, axis=1)
-        conv2 = gather_segments(np.array(x_arr["x2"]), n, axis=1)
+        x_all = [gather_segments(x[k].cpu().numpy(), n) for k in range(K)]
+        conv = [gather_segments(np.array(x_arr[f"x{k + 1}"]), n, axis=1) for k in range(K)]
         results = None
         if rank == 0:
-            results = {"x1": post_processing(x1_all.squeeze(-1)), "x2": post_processing(x2_all.squeeze(-1)),
-                       "gt1": gt1.squeeze(-1), "gt2": gt2.squeeze(-1), "mixed": post_processing(mixed_full.squeeze(-1)),
-                       "stft_mixture": stft_mixture}
+            results = {f"x{k + 1}": post_processing(x_all[k].squeeze(-1)) for k in range(K)}
+            results.update({f"gt{k + 1}": gts[k].squeeze(-1) for k in range(K)})
+            results.update({"mixed": post_processing(mixed_full.squeeze(-1)), "stft_mixture": stft_mixture})
             np.savez(os.path.join(out_dir, "results"), **results)                                # :435
-            np.savez(os.path.join(out_dir, "results_convergence"), x1=post_processing(conv1), x2=post_processing(conv2))
+            np.savez(os.path.join(out_dir, "results_convergence"),
+                     **{f"x{k + 1}": post_processing(conv[k]) for k in range(K)})
             results["duration_s"] = t1 - t0
         return results
     finally:

@@ -39,9 +39,13 @@ def normalise(db: np.ndarray) -> np.ndarray:
     return np.ascontiguousarray((db - DB_MIN) / (DB_MAX - DB_MIN), dtype=np.float32)
 
 
-def mixture_db(a_db: np.ndarray, b_db: np.ndarray) -> np.ndarray:
-    """Power-sum mixture of two dB patches, clipped like the data loader does."""
-    p = np.power(10.0, a_db.astype(np.float64) / 10.0) + np.power(10.0, b_db.astype(np.float64) / 10.0)
+def mixture_db(*sources_db: np.ndarray) -> np.ndarray:
+    """Power-sum mixture of two or more dB patches (summed in argument order), clipped like the data loader does."""
+    if len(sources_db) < 2:
+        raise ValueError("a mixture needs at least two sources")
+    p = np.power(10.0, sources_db[0].astype(np.float64) / 10.0)
+    for s in sources_db[1:]:
+        p = p + np.power(10.0, s.astype(np.float64) / 10.0)
     return np.clip(10.0 * np.log10(p), DB_MIN, DB_MAX).astype(np.float32)
 
 

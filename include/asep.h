@@ -176,6 +176,25 @@ int asep_basis_glow_inner(asep_glow_t m1, asep_glow_t m2, const DLTensor* mixed,
                           const DLTensor* noise2, uint64_t seed, uint64_t step0, uint64_t elem_offset,
                           DLTensor* per_step, DLTensor* nan_count, void* stream);
 
+/* ---- BASIS with K sources, 2 <= K <= 8 (any other K fails with ASEP_ERR_BAD_ARG before a launch).  Stacked layout: the
+ * states, scores, injected noise, per-step dumps and snapshots of all K sources are ONE contiguous tensor with the source
+ * axis after the step / level axis: x [K, ...], noise [T, K, ...], per_step [T, K, ...], snapshots [L, K, ...], where
+ * ... is the shape of `mixed`.  The update is the two-source one with g = (10/ln10)(logsumexp_k(x_k ln10/10) - ln K) and
+ * grad g = softmax_k; in-kernel noise of source k (0-based) is Philox stream k + 1, so K = 2 equals the two-source entry
+ * points bit for bit.  The same handle may serve several sources. */
+int asep_mixing_db_k(int K, const DLTensor* x, DLTensor* g, DLTensor* w, void* stream);
+int asep_langevin_step_k(int K, DLTensor* x, const DLTensor* score, const DLTensor* mixed, const DLTensor* noise, float eta,
+                         float lambda, float noise_scale, uint64_t seed, uint64_t step, uint64_t elem_offset,
+                         DLTensor* nan_count, void* stream);
+/* m: K Glow priors, one per source. */
+int asep_basis_glow_inner_k(int K, const asep_glow_t* m, const DLTensor* mixed, DLTensor* x, int T, float eta, float lambda,
+                            float noise_scale, const DLTensor* noise, uint64_t seed, uint64_t step0, uint64_t elem_offset,
+                            DLTensor* per_step, DLTensor* nan_count, void* stream);
+/* m: n_models * K handles, level i using m[(n_models == 1 ? 0 : i) * K + k] for source k. */
+int asep_basis_glow_run_k(int K, const asep_glow_t* m, int n_models, const DLTensor* mixed, DLTensor* x, int L, int T,
+                          const float* eta, const float* lambda, const float* noise_scale, uint64_t seed, uint64_t elem_offset,
+                          DLTensor* snapshots, DLTensor* nan_count, void* stream);
+
 /* ------------------------------------------------------------------ NCSN score networks
  * Replaces ncsn/utils.py:41-64 (get_uncompiled_model / get_uncompiled_model_v2) and the Keras call
  * `model([perturbed_X, sigma_idx], training=True)` on CondRefineNetDilated (ncsn/score_network.py:224-296,
@@ -238,6 +257,13 @@ int asep_basis_glow_run(const asep_glow_t* m1, const asep_glow_t* m2, int n_mode
 int asep_basis_ncsn_run(asep_ncsn_t m1, asep_ncsn_t m2, const DLTensor* mixed, DLTensor* x1, DLTensor* x2, int L, int T,
                         const float* eta, const float* lambda, const float* noise_scale, uint64_t seed, uint64_t elem_offset,
                         DLTensor* snapshots, DLTensor* nan_count, void* stream);
+/* K score networks m[K]; stacked layout and limits of asep_basis_glow_inner_k. */
+int asep_basis_ncsn_inner_k(int K, const asep_ncsn_t* m, const DLTensor* mixed, DLTensor* x, int sigma_idx, int T, float eta,
+                            float lambda, float noise_scale, const DLTensor* noise, uint64_t seed, uint64_t step0,
+                            uint64_t elem_offset, DLTensor* per_step, DLTensor* nan_count, void* stream);
+int asep_basis_ncsn_run_k(int K, const asep_ncsn_t* m, const DLTensor* mixed, DLTensor* x, int L, int T, const float* eta,
+                          const float* lambda, const float* noise_scale, uint64_t seed, uint64_t elem_offset,
+                          DLTensor* snapshots, DLTensor* nan_count, void* stream);
 /* Event timing of the tcgen05 convolution launches of the score networks (same contract as asep_tc_profile). */
 int asep_conv_profile(int on);
 int asep_conv_profile_read(double* total_ms, int64_t* launches, double* flops);
