@@ -134,6 +134,7 @@ _SIGNATURES = {
     "asep_mel_to_stft": [_P, _P, _P, _P, _P, _P, _F, _I, _V],
     "asep_stft_filter": [_P, _P, _P, _I, _V],
     "asep_istft": [_P, _I, _P, _V],
+    "asep_istft_track": [_P, _I, _I, _P, _V],
     "asep_griffinlim_update": [_P, _P, _P, _P, _F, _V],
     "asep_resample": [_P, _P, _P, _P, ctypes.c_double, _I, _P, _V],
     "asep_basis_graphs": [_I],

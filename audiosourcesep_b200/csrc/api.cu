@@ -1446,6 +1446,38 @@ int asep_istft(const DLTensor* stft, int hop, DLTensor* audio, void* stream) {
   ASEP_API_END
 }
 
+int asep_istft_track(const DLTensor* stft, int hop, int overlap_frames, DLTensor* audio, void* stream) {
+  ASEP_API_BEGIN
+  ASEP_CHECK(g_device >= 0, ASEP_ERR_STATE, "asep_init() has not been called");
+  TView sv = view_f32(stft, "stft", g_device), a = view_f32(audio, "audio", g_device);
+  ASEP_CHECK(sv.ndim == 5 && sv.shape[4] == 2 && sv.shape[2] >= 2 && sv.shape[3] >= 2, ASEP_ERR_BAD_SHAPE,
+             "stft must be [S, n_seg, F, T, 2]");
+  ASEP_CHECK(a.ndim == 2 && a.shape[0] == sv.shape[0] && a.shape[1] >= 1, ASEP_ERR_BAD_SHAPE, "audio must be [S, length]");
+  const int S = (int)sv.shape[0], n_seg = (int)sv.shape[1], F = (int)sv.shape[2], T = (int)sv.shape[3], n_fft = 2 * (F - 1);
+  ASEP_CHECK(n_seg >= 1, ASEP_ERR_BAD_SHAPE, "istft_track: no segments");
+  ASEP_CHECK(hop >= 1, ASEP_ERR_BAD_ARG, "hop must be positive");
+  // at most two segments may cover a sample: 2 overlap < V = hop (T - 1); for T = 64 frames, 0 <= overlap_frames <= 31
+  ASEP_CHECK(overlap_frames >= 0 && 2 * overlap_frames < T - 1, ASEP_ERR_BAD_ARG,
+             "istft_track: overlap_frames = %d outside 0..%d for segments of %d frames", overlap_frames, (T - 2) / 2, T);
+  const long long V = (long long)hop * (T - 1), O = (long long)hop * overlap_frames, P = V - O;
+  const long long length = a.shape[1], span = (long long)(n_seg - 1) * P + V;
+  ASEP_CHECK(length <= span, ASEP_ERR_BAD_ARG, "istft_track: %lld samples, but %d segments reconstruct only %lld", length, n_seg,
+             span);
+  ASEP_CHECK((long long)S * n_seg <= 65535, ASEP_ERR_UNSUPPORTED, "istft_track: %d x %d segments are beyond one launch", S,
+             n_seg);
+  cudaStream_t s = as_stream(stream);
+  float* frames = nullptr;
+  CUDA_CHECK(cudaMallocAsync(&frames, (size_t)S * n_seg * T * n_fft * sizeof(float), s));
+  try {
+    launch_istft_track(sv.f32, frames, a.f32, S, n_seg, n_fft, hop, T, (int)O, length, s);
+  } catch (...) {
+    cudaFreeAsync(frames, s);
+    throw;
+  }
+  CUDA_CHECK(cudaFreeAsync(frames, s));
+  ASEP_API_END
+}
+
 // ------------------------------------------------------------------ resampling (resample_kernels.cu)
 int asep_resample(const DLTensor* audio, const DLTensor* time, const DLTensor* win, const DLTensor* delta, double scale, int step,
                   DLTensor* out, void* stream) {

@@ -216,11 +216,9 @@ __global__ void __launch_bounds__(256) k_istft_frames(const float2* __restrict__
   }
 }
 
-__global__ void __launch_bounds__(256) k_overlap_add(const float* __restrict__ frames, float* __restrict__ audio, int n_fft, int hop,
-                                                     int T, long long out_len, long long total) {
-  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= total) return;
-  const long long n = i / out_len, o = i % out_len;
+// sample o of one segment's trimmed iSTFT: windowed frames [T, n_fft] of the segment summed over the (at most n_fft / hop)
+// frames covering it, divided by the window sum of squares, in double
+__device__ __forceinline__ double ola_sample(const float* __restrict__ seg_frames, long long o, int n_fft, int hop, int T) {
   const long long p = o + n_fft / 2;                    // position in the untrimmed signal
   const int t1 = (int)min((long long)T - 1, p / hop);
   const int t0 = p >= n_fft ? (int)((p - n_fft) / hop + 1) : 0;
@@ -229,10 +227,42 @@ __global__ void __launch_bounds__(256) k_overlap_add(const float* __restrict__ f
     const int k = (int)(p - (long long)t * hop);
     if (k < 0 || k >= n_fft) continue;
     const double w = 0.5 - 0.5 * cospi(2.0 * (double)k / (double)n_fft);
-    acc += (double)frames[((size_t)n * T + t) * n_fft + k];
+    acc += (double)seg_frames[(size_t)t * n_fft + k];
     wss += w * w;
   }
-  audio[i] = (float)(wss > 1.1754943508222875e-38 ? acc / wss : acc);
+  return wss > 1.1754943508222875e-38 ? acc / wss : acc;
+}
+
+__global__ void __launch_bounds__(256) k_overlap_add(const float* __restrict__ frames, float* __restrict__ audio, int n_fft, int hop,
+                                                     int T, long long out_len, long long total) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  const long long n = i / out_len, o = i % out_len;
+  audio[i] = (float)ola_sample(frames + (size_t)n * T * n_fft, o, n_fft, hop, T);
+}
+
+// Whole-track overlap-add: frames [S, n_seg, T, n_fft] -> audio [S, length].  Segment g spans track samples
+// [g P, g P + V), V = hop (T - 1), P = V - overlap; 2 overlap < V, so one or two segments cover a sample.  Each covering
+// segment contributes its trimmed iSTFT value u_g (ola_sample) with a cross-fade weight c_g: 1 inside the segment, a linear
+// ramp over the `overlap` samples it shares with a neighbour (none at either end of the track).  out = sum c_g u_g / sum c_g.
+__global__ void __launch_bounds__(256) k_overlap_add_track(const float* __restrict__ frames, float* __restrict__ audio, int n_seg,
+                                                           int n_fft, int hop, int T, int overlap, long long length, long long total) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  const long long s = i / length, n = i % length;
+  const long long V = (long long)hop * (T - 1), P = V - overlap;
+  const int last = (int)min((long long)n_seg - 1, n / P);
+  double num = 0.0, den = 0.0;
+  for (int g = max(0, last - 1); g <= last; ++g) {
+    const long long j = n - (long long)g * P;            // position inside segment g
+    if (j < 0 || j >= V) continue;
+    double c = 1.0;
+    if (g > 0 && j < overlap) c = ((double)j + 0.5) / (double)overlap;                 // fade in after segment g - 1
+    if (g < n_seg - 1 && j >= P) c = ((double)(V - j) - 0.5) / (double)overlap;       // fade out into segment g + 1
+    num += c * ola_sample(frames + ((size_t)s * n_seg + g) * T * n_fft, j, n_fft, hop, T);
+    den += c;
+  }
+  audio[i] = (float)(num / den);
 }
 
 int ilog2(int n) { int l = 0; while ((1 << l) < n) ++l; return l; }
@@ -301,6 +331,22 @@ void launch_istft(const float* stft, float* frames, float* audio, int N, int n_f
   ASEP_LAUNCH_CHECK();
   const long long out_len = (long long)hop * (T - 1), total = out_len * N;
   k_overlap_add<<<cdiv(total, 256), 256, 0, s>>>(frames, audio, n_fft, hop, T, out_len, total);
+  ASEP_LAUNCH_CHECK();
+}
+
+void launch_istft_track(const float* stft, float* frames, float* audio, int S, int n_seg, int n_fft, int hop, int T, int overlap,
+                        long long length, cudaStream_t s) {
+  ASEP_CHECK(n_fft >= 64 && n_fft <= 4096 && (n_fft & (n_fft - 1)) == 0, ASEP_ERR_UNSUPPORTED, "istft_track: n_fft = %d", n_fft);
+  static bool attr = false;
+  if (!attr) {
+    CUDA_CHECK(cudaFuncSetAttribute(k_istft_frames, cudaFuncAttributeMaxDynamicSharedMemorySize, 4096 * (int)sizeof(double2)));
+    attr = true;
+  }
+  k_istft_frames<<<dim3(T, S * n_seg), 256, (size_t)n_fft * sizeof(double2), s>>>(reinterpret_cast<const float2*>(stft), frames,
+                                                                                  twiddles(n_fft), n_fft, ilog2(n_fft), T);
+  ASEP_LAUNCH_CHECK();
+  const long long total = (long long)S * length;
+  k_overlap_add_track<<<cdiv(total, 256), 256, 0, s>>>(frames, audio, n_seg, n_fft, hop, T, overlap, length, total);
   ASEP_LAUNCH_CHECK();
 }
 

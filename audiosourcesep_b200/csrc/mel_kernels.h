@@ -26,5 +26,11 @@ void launch_griffinlim_update(const float* mag, const float* rebuilt, float* tpr
 // stft [N, F, T] complex64 -> audio [N, hop * (T - 1)]: windowed overlap-add of the inverse FFT frames divided by the
 // window sum of squares, n_fft/2 samples trimmed at both ends (librosa.istft, center = True); frames: scratch [N, T, n_fft]
 void launch_istft(const float* stft, float* frames, float* audio, int N, int n_fft, int hop, int T, cudaStream_t s);
+// stft [S, n_seg, F, T] complex64 of overlapping segments of one track (segment g starts at sample g P, P = hop (T-1) -
+// overlap) -> audio [S, length]: each segment's iSTFT value as launch_istft computes it, cross-faded linearly over the
+// `overlap` samples two neighbours share (hard cut when overlap = 0) and written straight into the track; the caller
+// guarantees 0 <= 2 overlap < hop (T-1) and length <= (n_seg-1) P + hop (T-1).  frames: scratch [S, n_seg, T, n_fft]
+void launch_istft_track(const float* stft, float* frames, float* audio, int S, int n_seg, int n_fft, int hop, int T, int overlap,
+                        long long length, cudaStream_t s);
 
 }  // namespace asep

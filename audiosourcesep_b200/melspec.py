@@ -138,6 +138,20 @@ def istft(stft_c: torch.Tensor, hop_length: int = 512) -> torch.Tensor:
     return out
 
 
+def istft_track(stft_c: torch.Tensor, overlap_frames: int, length: int, hop_length: int = 512) -> torch.Tensor:
+    """iSTFT of the overlapping segments of one track, written as the whole track: complex64 [S, n_seg, F, T] -> float32
+    [S, length].  Segment g starts at sample g P, P = hop (T-1) - hop overlap_frames; neighbours are cross-faded linearly
+    over the hop * overlap_frames samples they share (asep_istft_track, restated in oracle/track_oracle.py)."""
+    s = torch.view_as_real(stft_c.contiguous()).contiguous()
+    if s.ndim != 5:
+        raise ValueError(f"istft_track: expected complex [S, n_seg, F, T], got shape {tuple(stft_c.shape)}")
+    _dev(s.device.index)
+    out = torch.empty((s.shape[0], int(length)), dtype=torch.float32, device=s.device)
+    ds, do = _lib.dl(s), _lib.dl(out)
+    _lib.check(_lib.load().asep_istft_track(ds.ptr, int(hop_length), int(overlap_frames), do.ptr, _lib.stream_ptr()))
+    return out
+
+
 def griffinlim(mag: torch.Tensor, n_iter: int = 32, hop_length: int = 512, momentum: float = 0.99, seed: Optional[int] = None) -> torch.Tensor:
     """librosa.griffinlim(S, n_iter=32, hop_length, momentum=0.99, init='random'): STFT magnitudes [N, F, T] -> audio
     [N, hop (T-1)].  Random initial phases (librosa draws them from an unseeded RandomState, so outputs are not

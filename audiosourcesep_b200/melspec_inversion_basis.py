@@ -2,7 +2,8 @@
 (``stft_inversion_fn`` :42-90, ``single_channel_wiener_filter`` :93-119, ``main`` :122-236): reads ``results.npz`` of a
 BASIS run, inverts x1 / x2 / gt1 / gt2 / mixed with the mixture's phase (optionally through the single-channel Wiener
 filter) and writes ``inverse_spectrograms.npz`` + 16-bit wav files.  The transforms run on the GPU (melspec.py).
-``--algorithm griffin`` runs Griffin-Lim (:21-39; 32 iterations, momentum 0.99) on the same STFT / iSTFT kernels."""
+``--algorithm griffin`` runs Griffin-Lim (:21-39; 32 iterations, momentum 0.99) on the same STFT / iSTFT kernels.
+Results of ``run_basis_sep --mix`` (a ``segment_start`` key) are inverted as whole tracks instead (track.invert_track)."""
 from __future__ import annotations
 
 import argparse
@@ -77,6 +78,8 @@ def main(args):
     if args.algorithm not in ("reuse_phase", "griffin"):
         raise ValueError("method should be griffin or reuse_phase")                 # :197-198
     K = sum(1 for k in res.files if re.fullmatch(r"x[0-9]+", k))                   # one x{k} / gt{k} pair per source
+    if "segment_start" in res.files:                                               # a whole track (run_basis_sep --mix)
+        return _main_track(args, res, out_dir, K)
     xs = [res[f"x{k + 1}"] for k in range(K)]
     gts = [res[f"gt{k + 1}"] for k in range(K)]
     mix, stft_mixture = res["mixed"], res["stft_mixture"]
@@ -104,6 +107,22 @@ def main(args):
         write_wav(os.path.join(out_dir, name + ".wav"), flat[key], sr)
     np.savez(os.path.join(out_dir, "inverse_spectrograms"), **flat)
     return flat
+
+
+def _main_track(args, res, out_dir, K):
+    """Results of ``run_basis_sep --mix``: every x{k} is inverted as one full-length track (track.invert_track: segments
+    cross-faded, resampled back to the input's rate and length) and written as sep{k}.wav, with the float32 tracks in
+    separated.npz.  gt{k} keys are not needed; --method does not apply (the track is always inverted whole)."""
+    from . import track
+    if args.algorithm != "reuse_phase":
+        raise ValueError("a whole track is inverted with the mixture's phase (reuse_phase); Griffin-Lim draws random phases per "
+                         "segment, which do not cross-fade coherently")
+    t0 = time.time()
+    tracks = track.invert_results({k: res[k] for k in res.files}, args.wiener_filter)
+    torch.cuda.synchronize()
+    print("Inversion duration: {} seconds".format(round(time.time() - t0, 4)))
+    track.write_tracks(out_dir, [f"sep{k + 1}" for k in range(K)], tracks, int(res["orig_sr"]))
+    return {f"x{k + 1}_audio": tracks[k] for k in range(K)}
 
 
 def build_parser():

@@ -25,6 +25,12 @@ all of one ``model_type``), the stems named by ``--sources`` (``piano,violin`` b
 ``results.npz`` / ``results_convergence.npz`` holding ``x1..xK`` (and ``gt1..gtK``).  The loop works on one stacked state
 ``[K, n, H, W, 1]`` (basis_inner_loop_k / basis_outer_loop_k); the two-source functions are its K = 2 case.
 
+``--mix PATH`` separates a whole recording from its mixture alone (track.py): the wav file is cut into overlapping 2.04 s
+segments (``--overlap_frames``, default 8), nothing skipped or dropped; ``results.npz`` then holds x1..xK / mixed /
+stft_mixture over all segments plus ``segment_start``, ``track_length``, ``orig_sr``, ``orig_length`` and
+``overlap_frames`` (no gt keys), and rank 0 writes ``<output>/<source name>.wav`` at the input's rate and length and
+``separated.npz`` with the float32 tracks.
+
 Segments are independent (SURVEY.md 8(e)): under ``torchrun`` every rank separates a contiguous block of
 segments with noise keyed by the GLOBAL element index, and rank 0 gathers the blocks at the end -- the
 only cross-GPU traffic.
@@ -263,6 +269,18 @@ def load_song_patches(args):
     return arrs[0], arrs[1:], stft
 
 
+def load_mix_patches(args):
+    """Whole-track front end of ``--mix`` (track.py): (mixed_db float32 [n_seg, H, W, 1], stft_mixture complex64
+    [n_seg, 1025, W], segmentation) with segmentation = segment_start, track_length, orig_sr and orig_length."""
+    from . import track
+    x, rate, length = track.read_track(os.path.abspath(args.mix))
+    mel, stft, starts = track.segment_track(x, args.overlap_frames)
+    mix = mel.cpu().numpy()
+    if mix.shape[1:] != (args.height, args.width, 1):
+        raise ValueError(f"mel patches of shape {mix.shape[1:]}, the model expects {(args.height, args.width, 1)}")
+    return mix, stft.cpu().numpy(), {"starts": starts, "track_length": int(x.numel()), "orig_sr": rate, "orig_length": length}
+
+
 def load_weights(directory: str, shapes: Dict[str, tuple]) -> Dict[str, np.ndarray]:
     """Weights of one model: ``<directory>/weights.npz`` (this package's container) or, failing that, the TensorFlow
     checkpoint the reference writes -- ``<directory>/tf_ckpts/ckpt-N`` or ``<directory>/ckpt-N``
@@ -426,7 +444,27 @@ def build_parser() -> argparse.ArgumentParser:
                    help="stem names of the K sources in --song_dir (<name>.wav or <name>.npy); default piano,violin (K = 2)")
     p.add_argument("--host_loop", action="store_true",
                    help="run the sigma loop on the host (one library call per noise level) instead of asep_basis_*_run")
+    p.add_argument("--mix", type=str, default=None, metavar="PATH",
+                   help="separate this whole wav file from the mixture alone (no stems needed): overlapping 2.04 s segments, "
+                        "<output>/<source name>.wav per source at the input's rate and length; --n_mixed is ignored")
+    p.add_argument("--overlap_frames", type=int, default=8,
+                   help="with --mix: STFT frames (512 samples at 16 kHz) two neighbouring segments share and cross-fade "
+                        "over, 0..31 (0: hard cuts)")
+    p.add_argument("--wiener_filter", action="store_true",
+                   help="with --mix: invert through the K-source Wiener filter instead of the mixture's phase")
     return p
+
+
+def check_mix_args(args) -> None:
+    """Flag rules of the whole-track mode (--mix), checked before anything runs on the device: no --song_dir / --synthetic
+    next to it, --overlap_frames in 0..31, and --sources (if given) naming one output per restore directory."""
+    if getattr(args, "mix", None) is None:
+        return
+    if args.song_dir is not None or getattr(args, "synthetic", False):
+        raise ValueError("--mix separates a mixture on its own; it cannot be combined with --song_dir or --synthetic")
+    from .track import check_overlap_frames
+    check_overlap_frames(args.overlap_frames)
+    source_names(args)
 
 
 def merge_config(args: argparse.Namespace) -> argparse.Namespace:
@@ -435,7 +473,8 @@ def merge_config(args: argparse.Namespace) -> argparse.Namespace:
         return args
     cfg = vars(get_config(args.config))
     keep = ("dataset", "debug", "output", "song_dir", "inverse", "model_type", "n_mixed", "RESTORE1", "RESTORE2",
-            "synthetic", "random_init", "seed", "config", "fast", "precision", "exact", "host_loop", "RESTORE", "sources")
+            "synthetic", "random_init", "seed", "config", "fast", "precision", "exact", "host_loop", "RESTORE", "sources", "mix",
+            "overlap_frames", "wiener_filter")
     merged = dict(vars(args))
     for k, v in cfg.items():
         if k not in keep:
@@ -449,6 +488,8 @@ def main(args) -> Optional[Dict[str, np.ndarray]]:
     import torch.distributed as dist
 
     args = merge_config(args)
+    check_mix_args(args)
+    mix_mode = getattr(args, "mix", None) is not None
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -482,8 +523,12 @@ def main(args) -> Optional[Dict[str, np.ndarray]]:
         sys.stdout = open(os.devnull, "w")
     try:
         t0 = time.time()
-        mix_db, gts, stft_mixture = load_song_patches(args)
-        K = len(gts)
+        if mix_mode:
+            mix_db, stft_mixture, seg = load_mix_patches(args)
+            gts, K = None, len(restore_dirs(args))
+        else:
+            mix_db, gts, stft_mixture = load_song_patches(args)
+            K = len(gts)
         n = mix_db.shape[0]
         lo, hi = shard_range(n, world, rank)
         mixed_full = ((mix_db - args.minval) / (args.maxval - args.minval)).astype(np.float32)   # :355
@@ -513,12 +558,25 @@ def main(args) -> Optional[Dict[str, np.ndarray]]:
         conv = [gather_segments(np.array(x_arr[f"x{k + 1}"]), n, axis=1) for k in range(K)]
         results = None
         if rank == 0:
-            results = {f"x{k + 1}": post_processing(x_all[k].squeeze(-1)) for k in range(K)}
-            results.update({f"gt{k + 1}": gts[k].squeeze(-1) for k in range(K)})
-            results.update({"mixed": post_processing(mixed_full.squeeze(-1)), "stft_mixture": stft_mixture})
+            if mix_mode:
+                from . import track
+                results = track.track_results([post_processing(x_all[k].squeeze(-1)) for k in range(K)],
+                                              post_processing(mixed_full.squeeze(-1)), stft_mixture, seg["starts"],
+                                              seg["track_length"], seg["orig_sr"], seg["orig_length"], args.overlap_frames)
+            else:
+                results = {f"x{k + 1}": post_processing(x_all[k].squeeze(-1)) for k in range(K)}
+                results.update({f"gt{k + 1}": gts[k].squeeze(-1) for k in range(K)})
+                results.update({"mixed": post_processing(mixed_full.squeeze(-1)), "stft_mixture": stft_mixture})
             np.savez(os.path.join(out_dir, "results"), **results)                                # :435
             np.savez(os.path.join(out_dir, "results_convergence"),
                      **{f"x{k + 1}": post_processing(conv[k]) for k in range(K)})
+            if mix_mode:                                                 # whole-track back end: one wav per source
+                t2 = time.time()
+                tracks = track.invert_results(results, args.wiener_filter)
+                names = source_names(args)
+                track.write_tracks(out_dir, names, tracks, seg["orig_sr"])
+                print("Inversion duration: {} seconds".format(round(time.time() - t2, 3)))
+                results["separated"] = dict(zip(names, tracks))
             results["duration_s"] = t1 - t0
         return results
     finally:

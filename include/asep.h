@@ -315,6 +315,12 @@ int asep_mel_to_stft(const DLTensor* mel_db, const DLTensor* basis, const DLTens
                      DLTensor* mag, float step, int iters, void* stream);
 int asep_stft_filter(const DLTensor* mag, const DLTensor* stft_mixture, DLTensor* out, int wiener, void* stream);
 int asep_istft(const DLTensor* stft, int hop, DLTensor* audio, void* stream);
+/* Whole-track iSTFT of overlapping segments: stft [S, n_seg, F, T, 2] -> audio [S, length].  Segment g starts at sample g P,
+ * P = V - O, V = hop (T-1) (the span one segment's iSTFT reconstructs), O = hop * overlap_frames.  Every sample is the
+ * per-segment value asep_istft computes, cross-faded linearly over the O samples two neighbours share (hard cut when
+ * overlap_frames = 0, no ramp at either end of the track) and written straight into the track; no per-segment waveform is
+ * stored.  Requires 0 <= 2 overlap_frames < T - 1 (0..31 for T = 64) and length <= (n_seg-1) P + V (ASEP_ERR_BAD_ARG). */
+int asep_istft_track(const DLTensor* stft, int hop, int overlap_frames, DLTensor* audio, void* stream);
 /* One phase update of librosa.griffinlim (momentum variant; melspec_inversion_basis.py:21-39 through
  * librosa.feature.inverse.mel_to_audio): next = mag * unit(rebuilt - momentum/(1+momentum) * tprev); tprev <- rebuilt.
  * mag [...] fp32; rebuilt / tprev / next [..., 2] complex64.  The iteration (istft -> stft -> update) is driven from
