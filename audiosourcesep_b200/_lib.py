@@ -125,6 +125,9 @@ _SIGNATURES = {
     "asep_conv_profile": [_I],
     "asep_conv_profile_read": [ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_int64),
                                ctypes.POINTER(ctypes.c_double)],
+    "asep_conv_tc_image": [_P, _I, _I, _I, _P, _V],
+    "asep_conv_tc_forward": [_P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _V],
+    "asep_conv_wgrad_tc": [_P, _P, _P, _I, _I, _V],
     "asep_crc32c": [ctypes.c_char_p, ctypes.c_uint64, ctypes.c_uint32],
     "asep_bss_eval": [_P, _P, _I, ctypes.c_int64, ctypes.c_int64, ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64),
                       _I, _I, _P, _V],

@@ -10,6 +10,7 @@
 #include "glow_model.h"
 #include "mel_kernels.h"
 #include "ncsn_model.h"
+#include "ncsn_train_kernels.h"
 #include "resample_kernels.h"
 
 namespace asep {
@@ -95,8 +96,8 @@ static TView view_any(const DLTensor* t, const char* what, int device, bool allo
   ASEP_CHECK(t != nullptr, ASEP_ERR_BAD_ARG, "%s: NULL tensor", what);
   ASEP_CHECK(t->ndim >= 0 && t->ndim <= 8, ASEP_ERR_BAD_SHAPE, "%s: unsupported rank %d", what, t->ndim);
   ASEP_CHECK(t->dtype.code == code && t->dtype.bits == bits && t->dtype.lanes == 1, ASEP_ERR_BAD_DTYPE,
-             "%s: expected %s%d, got dtype code %d bits %d", what, code == kDLFloat ? "float" : "int", bits,
-             t->dtype.code, t->dtype.bits);
+             "%s: expected %s%d, got dtype code %d bits %d", what,
+             code == kDLFloat ? "float" : (code == kDLBfloat ? "bfloat" : "int"), bits, t->dtype.code, t->dtype.bits);
   TView v;
   v.ndim = t->ndim;
   for (int i = 0; i < t->ndim; ++i) v.shape[i] = t->shape[i];
@@ -1280,6 +1281,117 @@ int asep_conv_profile_read(double* total_ms, int64_t* launches, double* flops) {
   long long n = 0;
   conv_tc_profile_read(total_ms, &n, flops);
   if (launches) *launches = (int64_t)n;
+  ASEP_API_END
+}
+
+// ---- the tcgen05 convolutions one launch at a time (tests/test_gpu_conv_tc.py): thin wrappers over conv_tc_prepare /
+// launch_build_conv_image, conv_tc_forward and conv_wgrad_tc that check every shape before anything is launched
+static TView view_bf16(const DLTensor* t, const char* what) { return view_any(t, what, g_device, false, kDLBfloat, 16); }
+
+static void expect_numel(const TView& v, const char* what, int64_t n) {
+  ASEP_CHECK(v.numel == n, ASEP_ERR_BAD_SHAPE, "%s: %lld elements, expected %lld", what, (long long)v.numel, (long long)n);
+}
+
+int asep_conv_tc_image(const DLTensor* kernel, int transposed, int lo, int on_device, DLTensor* img, void* stream) {
+  ASEP_API_BEGIN
+  ASEP_CHECK(g_device >= 0, ASEP_ERR_STATE, "asep_init() has not been called");
+  ASEP_CHECK((transposed == 0 || transposed == 1) && (lo == 0 || lo == 1) && (on_device == 0 || on_device == 1),
+             ASEP_ERR_BAD_ARG, "transposed, lo and on_device are 0 or 1");
+  ASEP_CHECK(on_device || (!transposed && !lo), ASEP_ERR_BAD_ARG, "the host builder makes the forward hi image only");
+  TView kv = view_f32(kernel, "kernel", g_device, /*allow_host=*/!on_device);
+  ASEP_CHECK(kv.ndim == 4 && kv.shape[0] == kv.shape[1] && (kv.shape[0] == 1 || kv.shape[0] == 3), ASEP_ERR_BAD_SHAPE,
+             "kernel: expected HWIO [k,k,Cin,Cout] with k = 1 or 3");
+  const int ksize = (int)kv.shape[0], Cin = (int)kv.shape[2], Cout = (int)kv.shape[3];
+  // the contraction extent of the image (Cin, or Cout for the transposed image) is walked in 64-channel panels
+  ASEP_CHECK(Cin > 0 && Cout > 0 && (transposed ? Cout : Cin) % 64 == 0, ASEP_ERR_UNSUPPORTED,
+             "conv image: Cin=%d Cout=%d, the contraction extent must be a multiple of 64", Cin, Cout);
+  TView iv = view_bf16(img, "img");
+  expect_numel(iv, "img", kv.numel);
+  __nv_bfloat16* dst = static_cast<__nv_bfloat16*>(iv.raw);
+  if (on_device) {
+    launch_build_conv_image(kv.f32, dst, ksize * ksize, Cin, Cout, transposed, lo, as_stream(stream));
+  } else {
+    std::vector<float> host((size_t)kv.numel);
+    if (kv.on_device) CUDA_CHECK(cudaMemcpy(host.data(), kv.f32, host.size() * sizeof(float), cudaMemcpyDeviceToHost));
+    else std::memcpy(host.data(), kv.f32, host.size() * sizeof(float));
+    ConvWeightsTC w;
+    conv_tc_prepare(w, host.data(), nullptr, ksize, Cin, Cout, 1);
+    cudaError_t e = cudaMemcpy(dst, w.img, w.bytes, cudaMemcpyDeviceToDevice);
+    conv_tc_release(w);
+    CUDA_CHECK(e);
+  }
+  ASEP_API_END
+}
+
+int asep_conv_tc_forward(const DLTensor* img, const DLTensor* bias, int ksize, int Cin, int Cout, int dil, const DLTensor* x,
+                         const DLTensor* add, const DLTensor* add2, DLTensor* out, DLTensor* stats, DLTensor* out_bf16,
+                         void* stream) {
+  ASEP_API_BEGIN
+  ASEP_CHECK(g_device >= 0, ASEP_ERR_STATE, "asep_init() has not been called");
+  ASEP_CHECK((ksize == 1 || ksize == 3) && dil >= 1, ASEP_ERR_UNSUPPORTED, "conv: kernel size %d (1 or 3), dilation %d",
+             ksize, dil);
+  TView xv = view_bf16(x, "x");
+  ASEP_CHECK(xv.ndim == 4, ASEP_ERR_BAD_SHAPE, "x: expected NHWC [N,H,W,Cin]");
+  expect_shape(xv, "x", {-1, -1, -1, Cin});
+  const int N = (int)xv.shape[0], H = (int)xv.shape[1], W = (int)xv.shape[2];
+  ASEP_CHECK(conv_tc_supported(Cin, Cout, H, W), ASEP_ERR_UNSUPPORTED,
+             "tcgen05 conv: unsupported shape Cin=%d Cout=%d H=%d W=%d", Cin, Cout, H, W);
+  TView iv = view_bf16(img, "img");
+  expect_numel(iv, "img", (int64_t)ksize * ksize * Cin * Cout);
+  TView ov = view_f32(out, "out", g_device);
+  expect_shape(ov, "out", {N, H, W, Cout});
+  const float* addp[2] = {nullptr, nullptr};
+  const DLTensor* adds[2] = {add, add2};
+  for (int i = 0; i < 2; ++i)
+    if (adds[i]) {
+      TView av = view_f32(adds[i], i ? "add2" : "add", g_device);
+      expect_shape(av, i ? "add2" : "add", {N, H, W, Cout});
+      addp[i] = av.f32;
+    }
+  ConvWeightsTC w;                 // borrows the caller's image and bias: never conv_tc_release'd
+  w.img = static_cast<__nv_bfloat16*>(iv.raw);
+  w.bias_owned = false;
+  if (bias) {
+    TView bv = view_f32(bias, "bias", g_device);
+    expect_shape(bv, "bias", {Cout});
+    w.bias = bv.f32;
+  }
+  w.Cin = Cin; w.Cout = Cout; w.ksize = ksize; w.dil = dil;
+  w.bytes = (size_t)iv.numel * sizeof(__nv_bfloat16);
+  double* st = nullptr;
+  if (stats) {
+    TView sv = view_any(stats, "stats", g_device, false, kDLFloat, 64);
+    expect_shape(sv, "stats", {N, Cout, 2});
+    st = static_cast<double*>(sv.raw);
+  }
+  __nv_bfloat16* ob = nullptr;
+  if (out_bf16) {
+    TView bv = view_bf16(out_bf16, "out_bf16");
+    expect_shape(bv, "out_bf16", {N, H, W, Cout});
+    ob = static_cast<__nv_bfloat16*>(bv.raw);
+  }
+  conv_tc_forward(w, static_cast<const __nv_bfloat16*>(xv.raw), addp[0], ov.f32, N, H, W, as_stream(stream), st, ob, addp[1]);
+  ASEP_API_END
+}
+
+int asep_conv_wgrad_tc(const DLTensor* x, const DLTensor* g, DLTensor* dk, int ksize, int dil, void* stream) {
+  ASEP_API_BEGIN
+  ASEP_CHECK(g_device >= 0, ASEP_ERR_STATE, "asep_init() has not been called");
+  ASEP_CHECK((ksize == 1 || ksize == 3) && dil >= 1, ASEP_ERR_UNSUPPORTED, "conv wgrad: kernel size %d (1 or 3), dilation %d",
+             ksize, dil);
+  TView xv = view_bf16(x, "x");
+  ASEP_CHECK(xv.ndim == 4, ASEP_ERR_BAD_SHAPE, "x: expected NHWC [N,H,W,Cin]");
+  const int N = (int)xv.shape[0], H = (int)xv.shape[1], W = (int)xv.shape[2], Cin = (int)xv.shape[3];
+  TView gv = view_bf16(g, "g");
+  ASEP_CHECK(gv.ndim == 4, ASEP_ERR_BAD_SHAPE, "g: expected NHWC [N,H,W,Cout]");
+  expect_shape(gv, "g", {N, H, W, -1});
+  const int Cout = (int)gv.shape[3];
+  TView kv = view_f32(dk, "dk", g_device);
+  expect_shape(kv, "dk", {ksize, ksize, Cin, Cout});
+  ASEP_CHECK(conv_wgrad_tc_supported(Cin, Cout, H, W), ASEP_ERR_UNSUPPORTED,
+             "conv_wgrad_tc: unsupported shape Cin=%d Cout=%d H=%d W=%d", Cin, Cout, H, W);
+  conv_wgrad_tc(static_cast<const __nv_bfloat16*>(xv.raw), static_cast<const __nv_bfloat16*>(gv.raw), kv.f32, N, H, W, Cin,
+                Cout, ksize, dil, as_stream(stream));
   ASEP_API_END
 }
 

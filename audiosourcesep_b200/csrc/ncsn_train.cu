@@ -17,6 +17,12 @@ void NcsnModel::enable_training() {
   if (training_) return;
   ASEP_CHECK(prepared_, ASEP_ERR_STATE, "asep_ncsn_prepare() must be called before asep_ncsn_enable_training()");
   ASEP_CHECK(sigmas_dev_ != nullptr, ASEP_ERR_STATE, "training needs the noise levels (asep_ncsn_set_sigmas)");
+  // the weight gradient tiles 64 pixels where the forward convolution tiles 128 (W = 128 runs inference only): refuse
+  // such a patch here instead of inside the first train_grads
+  ASEP_CHECK(conv_wgrad_tc_supported(cfg_.ngf, cfg_.ngf, cfg_.H, cfg_.W) &&
+                 conv_wgrad_tc_supported(2 * cfg_.ngf, 2 * cfg_.ngf, cfg_.H / 2, cfg_.W / 2),
+             ASEP_ERR_UNSUPPORTED, "patch %dx%d with %d filters is outside the tcgen05 weight-gradient tiling (W <= 64)",
+             cfg_.H, cfg_.W, cfg_.ngf);
   CUDA_CHECK(cudaSetDevice(device_));
   CUDA_CHECK(cudaDeviceSynchronize());
   ++generation_;

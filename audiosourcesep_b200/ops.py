@@ -235,3 +235,55 @@ def basis_run_k(models, mixed, x, T: int, eta, lam, noise_scale, seed: int = 0, 
         _lib.check(_lib.load().asep_basis_ncsn_run_k(len(models), _handles(models), t[0].ptr, t[1].ptr, L, int(T), arr[0],
                                                      arr[1], arr[2], int(seed), int(elem_offset), t[2].ptr, t[3].ptr,
                                                      _lib.stream_ptr()))
+
+
+# ---- the tcgen05 convolutions of the score networks one launch at a time (tests compare each with a float64 reference)
+def _bf16(t: torch.Tensor, what: str) -> torch.Tensor:
+    if t.dtype != torch.bfloat16:
+        raise ValueError(f"{what} must be a bfloat16 tensor (got {t.dtype})")
+    return t.to(torch.device("cuda", _lib.init())).contiguous()
+
+
+def conv_tc_image(kernel, transposed: bool = False, lo: bool = False, on_device: bool = True) -> torch.Tensor:
+    """bf16 SWIZZLE_128B tile image [k*k*Cin*Cout] of the HWIO fp32 ``kernel`` as the device builder of the training step
+    (``on_device``) or the host builder of ``asep_ncsn_prepare`` makes it; ``transposed``: the data-gradient image,
+    ``lo``: the low word of the split-bf16 pair."""
+    k = torch.as_tensor(kernel)
+    k = _prep(k) if on_device else k.float().contiguous()
+    img = torch.empty(k.numel(), dtype=torch.bfloat16, device=torch.device("cuda", _lib.init()))
+    a, b = _lib.dl(k), _lib.dl(img)
+    _lib.check(_lib.load().asep_conv_tc_image(a.ptr, int(transposed), int(lo), int(on_device), b.ptr, _lib.stream_ptr()))
+    return img
+
+
+def conv_tc_forward(img, x, ksize: int, cin: int, cout: int, dil: int = 1, bias=None, add=None, add2=None, out=None,
+                    stats: bool = False, out_bf16: bool = False):
+    """One ``k_conv_tc`` / ``k_conv_tc_sw`` launch: ``out`` [N,H,W,cout] fp32 = conv(x bf16 [N,H,W,cin]) + bias + add +
+    add2.  ``out`` may be passed (and be ``add``: the split-bf16 passes accumulate in place).  Returns (out, stats
+    [N,cout,2] float64 or None, bf16 copy of out or None)."""
+    img, x = _bf16(img, "img"), _bf16(x, "x")
+    if out is None:
+        out = torch.empty(tuple(x.shape[:3]) + (cout,), dtype=torch.float32, device=x.device)
+    elif not (out.is_cuda and out.dtype == torch.float32 and out.is_contiguous()):
+        raise ValueError("out must be a contiguous float32 CUDA tensor")
+    bias = None if bias is None else _prep(bias)
+    if add is not None and add is not out:
+        add = _prep(add)
+    add2 = None if add2 is None else _prep(add2)
+    st = torch.empty((x.shape[0], cout, 2), dtype=torch.float64, device=x.device) if stats else None
+    ob = torch.empty(tuple(x.shape[:3]) + (cout,), dtype=torch.bfloat16, device=x.device) if out_bf16 else None
+    t = [_lib.dl(v) for v in (img, bias, x, add, add2, out, st, ob)]
+    _lib.check(_lib.load().asep_conv_tc_forward(t[0].ptr, t[1].ptr, int(ksize), int(cin), int(cout), int(dil), t[2].ptr,
+                                                t[3].ptr, t[4].ptr, t[5].ptr, t[6].ptr, t[7].ptr, _lib.stream_ptr()))
+    return out, st, ob
+
+
+def conv_wgrad_tc(x, g, dk: torch.Tensor, ksize: int, dil: int = 1) -> torch.Tensor:
+    """One ``k_conv_wgrad_tc`` launch: ``dk`` fp32 [k,k,Cin,Cout] (a contiguous CUDA tensor, updated in place) += the
+    weight gradient of the 'same' convolution for input x bf16 [N,H,W,Cin] and output gradient g bf16 [N,H,W,Cout]."""
+    x, g = _bf16(x, "x"), _bf16(g, "g")
+    if not (dk.is_cuda and dk.dtype == torch.float32 and dk.is_contiguous()):
+        raise ValueError("dk must be a contiguous float32 CUDA tensor (it is accumulated into)")
+    t = [_lib.dl(v) for v in (x, g, dk)]
+    _lib.check(_lib.load().asep_conv_wgrad_tc(t[0].ptr, t[1].ptr, t[2].ptr, int(ksize), int(dil), _lib.stream_ptr()))
+    return dk

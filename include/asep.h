@@ -31,7 +31,7 @@ typedef enum {
   ASEP_OK = 0,
   ASEP_ERR_BAD_ARG = -1,     /* NULL pointer, unknown name, bad enum            */
   ASEP_ERR_BAD_SHAPE = -2,   /* shape contract violated (reference asserts)     */
-  ASEP_ERR_BAD_DTYPE = -3,   /* not float32 (or int32 for sigma_idx)            */
+  ASEP_ERR_BAD_DTYPE = -3,   /* not float32 (or the int32 / bf16 / float64 stated) */
   ASEP_ERR_BAD_LAYOUT = -4,  /* non-contiguous / misaligned                     */
   ASEP_ERR_BAD_DEVICE = -5,  /* tensor not on the handle's CUDA device          */
   ASEP_ERR_CUDA = -6,        /* CUDA runtime / driver error                     */
@@ -229,7 +229,8 @@ int asep_ncsn_forward(asep_ncsn_t h, const DLTensor* x, const DLTensor* sigma_id
  * sigma[idx] * noise; grads [num_trainable] <- d loss / d theta with loss [1] = sum_n 1/2 ||score + noise/sigma_n||^2 *
  * sigma_n^2 / global_batch (the SUM over data-parallel ranks is the reference's compute_average_loss).  The three GEMMs of
  * every convolution (forward, data gradient, weight gradient) run on tcgen05 in the handle's precision mode.
- * adam_step: Keras Adam on the flat vector, then the tile images are rebuilt on the device. */
+ * adam_step: Keras Adam on the flat vector, then the tile images are rebuilt on the device.  enable_training fails with
+ * ASEP_ERR_UNSUPPORTED for patches wider than 64 (the weight gradient tiles 64 pixels; W = 128 runs inference only). */
 int asep_ncsn_enable_training(asep_ncsn_t h);
 int asep_ncsn_num_trainable(asep_ncsn_t h, int64_t* out);
 int asep_ncsn_param_span(asep_ncsn_t h, const char* name, int64_t* offset, int64_t* numel);
@@ -267,6 +268,25 @@ int asep_basis_ncsn_run_k(int K, const asep_ncsn_t* m, const DLTensor* mixed, DL
 /* Event timing of the tcgen05 convolution launches of the score networks (same contract as asep_tc_profile). */
 int asep_conv_profile(int on);
 int asep_conv_profile_read(double* total_ms, int64_t* launches, double* flops);
+/* ---- the tcgen05 convolutions of the score networks one launch at a time, so each can be tested against a float64
+ * reference.  Shapes are checked before anything is launched (ASEP_ERR_BAD_SHAPE / _BAD_DTYPE / _UNSUPPORTED).
+ * asep_conv_tc_image: kernel fp32 HWIO [k,k,Cin,Cout] (k = 1 or 3) -> img bf16 with k*k*Cin*Cout elements, the
+ *   SWIZZLE_128B tile images the convolution streams: per (tap, 64-channel panel) one [rows x 64] block, element (r, c)
+ *   at r*64 + (((c>>3) ^ (r&7))<<3) + (c&7).  transposed = 1: the image of the data gradient, K'[tap][co][ci] =
+ *   K[k*k-1-tap][ci][co]; lo = 1: the low word bf16(v - bf16(v)) of the split-bf16 mode.  on_device = 1 builds it with
+ *   the kernel the training step uses after every optimizer step (kernel on the device), on_device = 0 with the host
+ *   builder of asep_ncsn_prepare (kernel on the host or the device; transposed = lo = 0 only).
+ * asep_conv_tc_forward: out [N,H,W,Cout] fp32 = 'same' stride-1 convolution of x bf16 [N,H,W,Cin] with the image
+ *   + bias [Cout] + add + add2 ([N,H,W,Cout] fp32).  bias, add, add2, stats and out_bf16 may be NULL; add may alias out.
+ *   stats: float64 [N,Cout,2], per-(image, channel) sum and sum of squares of out (zeroed first); out_bf16: bf16 copy of
+ *   out [N,H,W,Cout].  Cout in {128, 192, 256, 384}, Cin a multiple of 64, W dividing 128 and H a multiple of 128/W.
+ * asep_conv_wgrad_tc: dk fp32 [k,k,Cin,Cout] += the weight gradient sum_p x[p + offset(tap)] g[p] of the same
+ *   convolution (it accumulates); x bf16 [N,H,W,Cin], g bf16 [N,H,W,Cout], W dividing 64. */
+int asep_conv_tc_image(const DLTensor* kernel, int transposed, int lo, int on_device, DLTensor* img, void* stream);
+int asep_conv_tc_forward(const DLTensor* img, const DLTensor* bias, int ksize, int Cin, int Cout, int dil, const DLTensor* x,
+                         const DLTensor* add, const DLTensor* add2, DLTensor* out, DLTensor* stats, DLTensor* out_bf16,
+                         void* stream);
+int asep_conv_wgrad_tc(const DLTensor* x, const DLTensor* g, DLTensor* dk, int ksize, int dil, void* stream);
 
 /* CRC-32C (Castagnoli) of a HOST buffer, continuing from `crc` (0 to start): the checksum of the TensorFlow checkpoint
  * (TensorBundle) files tf.train.Checkpoint writes (train_utils.py:62-75), used by audiosourcesep_b200/tf_checkpoint.py. */

@@ -144,3 +144,18 @@ def test_dsm_gradients_at_the_reference_patch_size():
     print(f"[v1 96x64] whole-gradient relative error {flat_err:.3e}, worst tensor {worst[0]:.3e} ({worst[1]}), loss {loss.item():.6f} vs {loss_ref:.6f}")
     assert abs(loss.item() - loss_ref) <= 2e-4 * abs(loss_ref)
     assert flat_err <= 2e-4 and worst[0] <= 1e-3
+
+
+def test_enable_training_rejects_a_patch_the_weight_gradient_does_not_tile():
+    """The forward convolution tiles W up to 128, the weight gradient only up to 64: a W = 128 score network runs
+    inference, and enable_training refuses it up front (ASEP_ERR_UNSUPPORTED) instead of the first train step."""
+    from audiosourcesep_b200 import _lib
+    from audiosourcesep_b200.ncsn.score_model import ScoreModel
+    cfg = NCSNConfig(version="v2", H=8, W=128, ngf=128, num_classes=4, sigma1=1.0, sigmaL=0.01)
+    sig = bo.get_sigmas(cfg.sigma1, cfg.sigmaL, cfg.num_classes, cfg.progression)
+    model = ScoreModel(cfg, init_ncsn_params(cfg, seed=1, mode="perturbed"), sigmas=sig, precision=_lib.PREC_BF16)
+    score = model.score(torch.rand(2, cfg.H, cfg.W, 1), 1)
+    assert bool(torch.isfinite(score).all())
+    with pytest.raises(_lib.AsepError) as e:
+        model.enable_training()
+    assert e.value.code == -9 and "weight-gradient" in str(e.value)
