@@ -91,10 +91,7 @@ _SIGNATURES = {
     "asep_squeeze": [_P, _P, _I, _V],
     "asep_glow_coupling_nn": [_V, _I, _I, _P, _P, _V],
     "asep_glow_coupling_nn_backward": [_V, _I, _I, _P, _P, _P, _V],
-    "asep_langevin_step": [_P, _P, _P, _P, _P, _P, _P, _F, _F, _F, _U64, _U64, _U64, _P, _V],
-    "asep_mixing_db": [_P, _P, _P, _P, _P, _V],
     "asep_philox_normal": [_P, _U64, _U64, _U64, _U64, _V],
-    "asep_basis_glow_inner": [_V, _V, _P, _P, _P, _I, _F, _F, _F, _P, _P, _U64, _U64, _U64, _P, _P, _V],
     "asep_ncsn_create": [ctypes.POINTER(NcsnCfg), ctypes.POINTER(_V)],
     "asep_ncsn_destroy": [_V],
     "asep_ncsn_set_param": [_V, ctypes.c_char_p, _P],
@@ -109,11 +106,6 @@ _SIGNATURES = {
     "asep_ncsn_adam_step": [_V, _P, _F, _F, _F, _F, _V],
     "asep_ncsn_get_flat": [_V, _P, _V],
     "asep_ncsn_set_flat": [_V, _P, _V],
-    "asep_basis_ncsn_inner": [_V, _V, _P, _P, _P, _I, _I, _F, _F, _F, _P, _P, _U64, _U64, _U64, _P, _P, _V],
-    "asep_basis_glow_run": [ctypes.POINTER(_V), ctypes.POINTER(_V), _I, _P, _P, _P, _I, _I, ctypes.POINTER(ctypes.c_float),
-                            ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_float), _U64, _U64, _P, _P, _V],
-    "asep_basis_ncsn_run": [_V, _V, _P, _P, _P, _I, _I, ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_float),
-                            ctypes.POINTER(ctypes.c_float), _U64, _U64, _P, _P, _V],
     "asep_mixing_db_k": [_I, _P, _P, _P, _V],
     "asep_langevin_step_k": [_I, _P, _P, _P, _P, _F, _F, _F, _U64, _U64, _U64, _P, _V],
     "asep_basis_glow_inner_k": [_I, ctypes.POINTER(_V), _P, _P, _I, _F, _F, _F, _P, _U64, _U64, _U64, _P, _P, _V],

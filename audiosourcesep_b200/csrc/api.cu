@@ -542,29 +542,6 @@ static void expect_stacked(const TView& v, const char* what, std::initializer_li
   }
 }
 
-int asep_langevin_step(DLTensor* x1, DLTensor* x2, const DLTensor* s1, const DLTensor* s2, const DLTensor* mixed,
-                       const DLTensor* n1, const DLTensor* n2, float eta, float lambda, float noise_scale,
-                       uint64_t seed, uint64_t step, uint64_t elem_offset, DLTensor* nan_count, void* stream) {
-  ASEP_API_BEGIN
-  TView a = view_f32(x1, "x1", g_device), b = view_f32(x2, "x2", g_device);
-  TView sa = view_f32(s1, "s1", g_device), sb = view_f32(s2, "s2", g_device), mx = view_f32(mixed, "mixed", g_device);
-  ASEP_CHECK(a.numel == b.numel && a.numel == sa.numel && a.numel == sb.numel && a.numel == mx.numel,
-             ASEP_ERR_BAD_SHAPE, "langevin: all tensors must have the same number of elements");
-  ASEP_CHECK((n1 == nullptr) == (n2 == nullptr), ASEP_ERR_BAD_ARG, "inject both noise tensors or neither");
-  LangevinSources p{};
-  p.x[0] = a.f32; p.x[1] = b.f32;
-  p.s[0] = sa.f32; p.s[1] = sb.f32;
-  if (n1) {
-    TView na = view_f32(n1, "n1", g_device), nb = view_f32(n2, "n2", g_device);
-    ASEP_CHECK(na.numel == a.numel && nb.numel == a.numel, ASEP_ERR_BAD_SHAPE, "noise shape mismatch");
-    p.n[0] = na.f32; p.n[1] = nb.f32;
-  }
-  int* nanp = nullptr;
-  if (nan_count) nanp = static_cast<int*>(view_i32(nan_count, "nan_count", g_device).raw);
-  launch_langevin(2, p, mx.f32, eta, lambda, noise_scale, seed, step, elem_offset, nanp, a.numel, as_stream(stream));
-  ASEP_API_END
-}
-
 int asep_langevin_step_k(int K, DLTensor* x, const DLTensor* score, const DLTensor* mixed, const DLTensor* noise, float eta,
                          float lambda, float noise_scale, uint64_t seed, uint64_t step, uint64_t elem_offset,
                          DLTensor* nan_count, void* stream) {
@@ -589,19 +566,6 @@ int asep_langevin_step_k(int K, DLTensor* x, const DLTensor* score, const DLTens
     p.n[k] = noise ? nv.f32 + k * n : nullptr;
   }
   launch_langevin(K, p, mx.f32, eta, lambda, noise_scale, seed, step, elem_offset, nanp, n, as_stream(stream));
-  ASEP_API_END
-}
-
-int asep_mixing_db(const DLTensor* x1, const DLTensor* x2, DLTensor* g, DLTensor* w1, DLTensor* w2, void* stream) {
-  ASEP_API_BEGIN
-  TView a = view_f32(x1, "x1", g_device), b = view_f32(x2, "x2", g_device), gv = view_f32(g, "g", g_device);
-  TView wa = view_f32(w1, "w1", g_device), wb = view_f32(w2, "w2", g_device);
-  ASEP_CHECK(a.numel == b.numel && a.numel == gv.numel && a.numel == wa.numel && a.numel == wb.numel,
-             ASEP_ERR_BAD_SHAPE, "mixing: element counts differ");
-  MixingSources p{};
-  p.x[0] = a.f32; p.x[1] = b.f32;
-  p.w[0] = wa.f32; p.w[1] = wb.f32;
-  launch_mixing_db(2, p, gv.f32, a.numel, as_stream(stream));
   ASEP_API_END
 }
 
@@ -848,41 +812,29 @@ float* stacked_dump(DLTensor* per_step, const TView& x, int T, int dev) {
   expect_stacked(v, "per_step", {T}, x);
   return v.f32;
 }
+
+// The BasisCall of a stacked K-source call on the data shape of `mixed` (mx): state x [K, ...], the optional noise and
+// per-step dump [T, K, ...] and NaN counter.  The checks of the priors against that shape stay with each entry point.
+BasisCall stacked_call(int K, const TView& mx, DLTensor* x, int T, float eta, float lambda, float noise_scale,
+                       const DLTensor* noise, uint64_t seed, uint64_t step0, uint64_t elem_offset, DLTensor* per_step,
+                       DLTensor* nan_count, int dev) {
+  TView xv = view_f32(x, "x", dev);
+  expect_stacked(xv, "x", {K}, mx);
+  ASEP_CHECK(mx.numel % 4 == 0, ASEP_ERR_BAD_SHAPE, "the element count of one source (%lld) must be a multiple of 4",
+             (long long)mx.numel);
+  BasisCall call{K, {}, (long long)K * mx.numel, mx.f32, stacked_dump(per_step, xv, T, dev), nullptr, (long long)mx.numel,
+                 (int)mx.shape[0], T, eta, lambda, noise_scale, seed, step0, elem_offset};
+  const float* nz = stacked_noise(noise, xv, T, dev);
+  for (int k = 0; k < K; ++k) {
+    call.src.x[k] = xv.f32 + k * mx.numel;
+    call.src.n[k] = nz ? nz + k * mx.numel : nullptr;
+  }
+  if (nan_count) call.nanp = static_cast<int*>(view_i32(nan_count, "nan_count", dev).raw);
+  return call;
+}
 }  // namespace
 
 extern "C" {
-
-int asep_basis_glow_inner(asep_glow_t m1, asep_glow_t m2, const DLTensor* mixed, DLTensor* x1, DLTensor* x2, int T,
-                          float eta, float lambda, float noise_scale, const DLTensor* noise1, const DLTensor* noise2,
-                          uint64_t seed, uint64_t step0, uint64_t elem_offset, DLTensor* per_step,
-                          DLTensor* nan_count, void* stream) {
-  ASEP_API_BEGIN
-  ASEP_CHECK(m1 && m2, ASEP_ERR_BAD_ARG, "NULL handle");
-  GlowModel &g1 = *m1->model, &g2 = *m2->model;
-  const int dev = g1.device();
-  TView a = view_f32(x1, "x1", dev), b = view_f32(x2, "x2", dev), mx = view_f32(mixed, "mixed", dev);
-  const int N = batch_of(a, g1, "x1");
-  ASEP_CHECK(batch_of(b, g2, "x2") == N && mx.numel == a.numel, ASEP_ERR_BAD_SHAPE, "x1, x2, mixed must match");
-  ASEP_CHECK(g2.device() == dev, ASEP_ERR_BAD_DEVICE, "the two priors live on different devices");
-  ASEP_CHECK((noise1 == nullptr) == (noise2 == nullptr), ASEP_ERR_BAD_ARG, "inject both noise tensors or neither");
-  BasisCall call{2, {}, a.numel, mx.f32, nullptr, nullptr, (long long)a.numel, N, T, eta, lambda, noise_scale, seed, step0,
-                 elem_offset};
-  call.src.x[0] = a.f32; call.src.x[1] = b.f32;
-  if (noise1) {
-    TView na = view_f32(noise1, "noise1", dev), nb = view_f32(noise2, "noise2", dev);
-    ASEP_CHECK(na.numel == (int64_t)T * a.numel && nb.numel == na.numel, ASEP_ERR_BAD_SHAPE, "noise must be [T, ...]");
-    call.src.n[0] = na.f32; call.src.n[1] = nb.f32;
-  }
-  if (per_step) {
-    TView d = view_f32(per_step, "per_step", dev);
-    ASEP_CHECK(d.numel == (int64_t)T * 2 * a.numel, ASEP_ERR_BAD_SHAPE, "per_step must be [T, 2, ...]");
-    call.dump = d.f32;
-  }
-  if (nan_count) call.nanp = static_cast<int*>(view_i32(nan_count, "nan_count", dev).raw);
-  GlowModel* const ms[2] = {&g1, &g2};
-  basis_glow_steps(call, ms, as_stream(stream));
-  ASEP_API_END
-}
 
 int asep_basis_glow_inner_k(int K, const asep_glow_t* m, const DLTensor* mixed, DLTensor* x, int T, float eta, float lambda,
                             float noise_scale, const DLTensor* noise, uint64_t seed, uint64_t step0, uint64_t elem_offset,
@@ -896,23 +848,13 @@ int asep_basis_glow_inner_k(int K, const asep_glow_t* m, const DLTensor* mixed, 
     ms[k] = m[k]->model.get();
   }
   const int dev = ms[0]->device();
-  TView mx = view_f32(mixed, "mixed", dev), xv = view_f32(x, "x", dev);
+  TView mx = view_f32(mixed, "mixed", dev);
   for (int k = 0; k < K; ++k) {
     batch_of(mx, *ms[k], "mixed");                  // every prior models the data shape of the mixture
     ASEP_CHECK(ms[k]->device() == dev, ASEP_ERR_BAD_DEVICE, "the priors live on different devices");
   }
-  expect_stacked(xv, "x", {K}, mx);
-  ASEP_CHECK(mx.numel % 4 == 0, ASEP_ERR_BAD_SHAPE, "the element count of one source (%lld) must be a multiple of 4",
-             (long long)mx.numel);
-  BasisCall call{K, {}, (long long)K * mx.numel, mx.f32, stacked_dump(per_step, xv, T, dev), nullptr, (long long)mx.numel,
-                 (int)mx.shape[0], T, eta, lambda, noise_scale, seed, step0, elem_offset};
-  const float* nz = stacked_noise(noise, xv, T, dev);
-  for (int k = 0; k < K; ++k) {
-    call.src.x[k] = xv.f32 + k * mx.numel;
-    call.src.n[k] = nz ? nz + k * mx.numel : nullptr;
-  }
-  if (nan_count) call.nanp = static_cast<int*>(view_i32(nan_count, "nan_count", dev).raw);
-  basis_glow_steps(call, ms, as_stream(stream));
+  basis_glow_steps(stacked_call(K, mx, x, T, eta, lambda, noise_scale, noise, seed, step0, elem_offset, per_step, nan_count, dev),
+                   ms, as_stream(stream));
   ASEP_API_END
 }
 
@@ -1074,46 +1016,6 @@ int asep_ncsn_set_flat(asep_ncsn_t h, const DLTensor* theta, void* stream) {
   ASEP_API_END
 }
 
-int asep_basis_ncsn_inner(asep_ncsn_t m1, asep_ncsn_t m2, const DLTensor* mixed, DLTensor* x1, DLTensor* x2,
-                          int sigma_idx, int T, float eta, float lambda, float noise_scale, const DLTensor* noise1,
-                          const DLTensor* noise2, uint64_t seed, uint64_t step0, uint64_t elem_offset,
-                          DLTensor* per_step, DLTensor* nan_count, void* stream) {
-  ASEP_API_BEGIN
-  ASEP_CHECK(m1 && m2, ASEP_ERR_BAD_ARG, "NULL handle");
-  NcsnModel &g1 = *m1->model, &g2 = *m2->model;
-  const int dev = g1.device();
-  const auto& c = g1.cfg();
-  TView a = view_f32(x1, "x1", dev), b = view_f32(x2, "x2", dev), mx = view_f32(mixed, "mixed", dev);
-  expect_shape(a, "x1", {-1, c.H, c.W, c.C});
-  const int N = (int)a.shape[0];
-  expect_shape(b, "x2", {N, c.H, c.W, c.C});
-  ASEP_CHECK(mx.numel == a.numel, ASEP_ERR_BAD_SHAPE, "x1, x2, mixed must match");
-  const auto& c2 = g2.cfg();
-  ASEP_CHECK(c2.H == c.H && c2.W == c.W && c2.C == c.C, ASEP_ERR_BAD_SHAPE,
-             "the two score networks must share the data shape (%dx%dx%d vs %dx%dx%d)", c.H, c.W, c.C, c2.H, c2.W, c2.C);
-  ASEP_CHECK(g2.device() == dev, ASEP_ERR_BAD_DEVICE, "the two score networks live on different devices");
-  ASEP_CHECK(sigma_idx >= 0 && sigma_idx < c.num_classes && sigma_idx < c2.num_classes, ASEP_ERR_BAD_ARG,
-             "sigma_idx %d out of range (num_classes %d / %d)", sigma_idx, c.num_classes, c2.num_classes);
-  ASEP_CHECK((noise1 == nullptr) == (noise2 == nullptr), ASEP_ERR_BAD_ARG, "inject both noise tensors or neither");
-  BasisCall call{2, {}, a.numel, mx.f32, nullptr, nullptr, (long long)a.numel, N, T, eta, lambda, noise_scale, seed, step0,
-                 elem_offset};
-  call.src.x[0] = a.f32; call.src.x[1] = b.f32;
-  if (noise1) {
-    TView na = view_f32(noise1, "noise1", dev), nb = view_f32(noise2, "noise2", dev);
-    ASEP_CHECK(na.numel == (int64_t)T * a.numel && nb.numel == na.numel, ASEP_ERR_BAD_SHAPE, "noise must be [T, ...]");
-    call.src.n[0] = na.f32; call.src.n[1] = nb.f32;
-  }
-  if (per_step) {
-    TView d = view_f32(per_step, "per_step", dev);
-    ASEP_CHECK(d.numel == (int64_t)T * 2 * a.numel, ASEP_ERR_BAD_SHAPE, "per_step must be [T, 2, ...]");
-    call.dump = d.f32;
-  }
-  if (nan_count) call.nanp = static_cast<int*>(view_i32(nan_count, "nan_count", dev).raw);
-  NcsnModel* const ms[2] = {&g1, &g2};
-  basis_ncsn_steps(call, ms, sigma_idx, as_stream(stream));
-  ASEP_API_END
-}
-
 int asep_basis_ncsn_inner_k(int K, const asep_ncsn_t* m, const DLTensor* mixed, DLTensor* x, int sigma_idx, int T, float eta,
                             float lambda, float noise_scale, const DLTensor* noise, uint64_t seed, uint64_t step0,
                             uint64_t elem_offset, DLTensor* per_step, DLTensor* nan_count, void* stream) {
@@ -1126,7 +1028,7 @@ int asep_basis_ncsn_inner_k(int K, const asep_ncsn_t* m, const DLTensor* mixed, 
     ms[k] = m[k]->model.get();
   }
   const int dev = ms[0]->device();
-  TView mx = view_f32(mixed, "mixed", dev), xv = view_f32(x, "x", dev);
+  TView mx = view_f32(mixed, "mixed", dev);
   for (int k = 0; k < K; ++k) {
     const auto& c = ms[k]->cfg();
     expect_shape(mx, "mixed", {-1, c.H, c.W, c.C});   // every score network models the data shape of the mixture
@@ -1134,18 +1036,8 @@ int asep_basis_ncsn_inner_k(int K, const asep_ncsn_t* m, const DLTensor* mixed, 
     ASEP_CHECK(sigma_idx >= 0 && sigma_idx < c.num_classes, ASEP_ERR_BAD_ARG, "sigma_idx %d out of range (num_classes %d)",
                sigma_idx, c.num_classes);
   }
-  expect_stacked(xv, "x", {K}, mx);
-  ASEP_CHECK(mx.numel % 4 == 0, ASEP_ERR_BAD_SHAPE, "the element count of one source (%lld) must be a multiple of 4",
-             (long long)mx.numel);
-  BasisCall call{K, {}, (long long)K * mx.numel, mx.f32, stacked_dump(per_step, xv, T, dev), nullptr, (long long)mx.numel,
-                 (int)mx.shape[0], T, eta, lambda, noise_scale, seed, step0, elem_offset};
-  const float* nz = stacked_noise(noise, xv, T, dev);
-  for (int k = 0; k < K; ++k) {
-    call.src.x[k] = xv.f32 + k * mx.numel;
-    call.src.n[k] = nz ? nz + k * mx.numel : nullptr;
-  }
-  if (nan_count) call.nanp = static_cast<int*>(view_i32(nan_count, "nan_count", dev).raw);
-  basis_ncsn_steps(call, ms, sigma_idx, as_stream(stream));
+  basis_ncsn_steps(stacked_call(K, mx, x, T, eta, lambda, noise_scale, noise, seed, step0, elem_offset, per_step, nan_count, dev),
+                   ms, sigma_idx, as_stream(stream));
   ASEP_API_END
 }
 
@@ -1172,34 +1064,6 @@ float* run_snapshots(DLTensor* snapshots, const TView& xv, int K, int L, float**
 }
 }  // namespace
 
-int asep_basis_glow_run(const asep_glow_t* m1, const asep_glow_t* m2, int n_models, const DLTensor* mixed, DLTensor* x1,
-                        DLTensor* x2, int L, int T, const float* eta, const float* lambda, const float* noise_scale,
-                        uint64_t seed, uint64_t elem_offset, DLTensor* snapshots, DLTensor* nan_count, void* stream) {
-  ASEP_API_BEGIN
-  ASEP_CHECK(m1 && m2 && eta && lambda && noise_scale, ASEP_ERR_BAD_ARG, "NULL argument");
-  ASEP_CHECK(L >= 1 && T >= 0 && (n_models == 1 || n_models == L), ASEP_ERR_BAD_ARG,
-             "n_models must be 1 (one pair of priors for every level) or L (one pair per level)");
-  ASEP_CHECK(m1[0] && m2[0], ASEP_ERR_BAD_ARG, "NULL handle");
-  const int dev = m1[0]->model->device();
-  TView a = view_f32(x1, "x1", dev), b = view_f32(x2, "x2", dev);
-  float* snap = nullptr;
-  if (snapshots) {
-    TView sv = view_f32(snapshots, "snapshots", dev);
-    ASEP_CHECK(sv.numel == (int64_t)L * 2 * a.numel, ASEP_ERR_BAD_SHAPE, "snapshots must be [L, 2, N, H, W, C]");
-    snap = sv.f32;
-  }
-  float* const xs[2] = {a.f32, b.f32};
-  for (int i = 0; i < L; ++i) {
-    const int k = n_models == 1 ? 0 : i;
-    ASEP_CHECK(m1[k] && m2[k], ASEP_ERR_BAD_ARG, "NULL handle at level %d", i);
-    const int rc = asep_basis_glow_inner(m1[k], m2[k], mixed, x1, x2, T, eta[i], lambda[i], noise_scale[i], nullptr, nullptr, seed,
-                                         (uint64_t)i * (uint64_t)T, elem_offset, nullptr, nan_count, stream);
-    if (rc != ASEP_OK) return rc;                      // asep_last_error() holds the inner message
-    snapshot_states(snap, i, 2, xs, a.numel, as_stream(stream));
-  }
-  ASEP_API_END
-}
-
 int asep_basis_glow_run_k(int K, const asep_glow_t* m, int n_models, const DLTensor* mixed, DLTensor* x, int L, int T,
                           const float* eta, const float* lambda, const float* noise_scale, uint64_t seed, uint64_t elem_offset,
                           DLTensor* snapshots, DLTensor* nan_count, void* stream) {
@@ -1218,32 +1082,8 @@ int asep_basis_glow_run_k(int K, const asep_glow_t* m, int n_models, const DLTen
     const int rc = asep_basis_glow_inner_k(K, m + (size_t)(n_models == 1 ? 0 : i) * K, mixed, x, T, eta[i], lambda[i],
                                            noise_scale[i], nullptr, seed, (uint64_t)i * (uint64_t)T, elem_offset, nullptr,
                                            nan_count, stream);
-    if (rc != ASEP_OK) return rc;
+    if (rc != ASEP_OK) return rc;                      // asep_last_error() holds the inner message
     snapshot_states(snap, i, K, xs, xv.numel / K, as_stream(stream));
-  }
-  ASEP_API_END
-}
-
-int asep_basis_ncsn_run(asep_ncsn_t m1, asep_ncsn_t m2, const DLTensor* mixed, DLTensor* x1, DLTensor* x2, int L, int T,
-                        const float* eta, const float* lambda, const float* noise_scale, uint64_t seed, uint64_t elem_offset,
-                        DLTensor* snapshots, DLTensor* nan_count, void* stream) {
-  ASEP_API_BEGIN
-  ASEP_CHECK(m1 && m2 && eta && lambda && noise_scale, ASEP_ERR_BAD_ARG, "NULL argument");
-  ASEP_CHECK(L >= 1 && T >= 0, ASEP_ERR_BAD_ARG, "bad L / T");
-  const int dev = m1->model->device();
-  TView a = view_f32(x1, "x1", dev), b = view_f32(x2, "x2", dev);
-  float* snap = nullptr;
-  if (snapshots) {
-    TView sv = view_f32(snapshots, "snapshots", dev);
-    ASEP_CHECK(sv.numel == (int64_t)L * 2 * a.numel, ASEP_ERR_BAD_SHAPE, "snapshots must be [L, 2, N, H, W, C]");
-    snap = sv.f32;
-  }
-  float* const xs[2] = {a.f32, b.f32};
-  for (int i = 0; i < L; ++i) {
-    const int rc = asep_basis_ncsn_inner(m1, m2, mixed, x1, x2, i, T, eta[i], lambda[i], noise_scale[i], nullptr, nullptr, seed,
-                                         (uint64_t)i * (uint64_t)T, elem_offset, nullptr, nan_count, stream);
-    if (rc != ASEP_OK) return rc;
-    snapshot_states(snap, i, 2, xs, a.numel, as_stream(stream));
   }
   ASEP_API_END
 }

@@ -71,13 +71,18 @@ def anneal_langevin_dynamics(x_mod, data_shape, model, n_samples, sigmas, n_step
     ``x <- x + step * score(x, i) + sqrt(2 step) * N(0,1)``, ``step = step_lr * (sigma_i / sigma_L)^2``.
 
     This is the single-source, lambda = 0 case of the fused BASIS update (SURVEY.md 8(a) row 19): the same
-    kernel runs it with a dummy second source.  ``noise`` ([L, n_steps_each, n, H, W, C] standard normals) injects
-    the draws for parity runs; otherwise Philox noise keyed by (seed, step, element) is generated in the kernel."""
+    kernel runs it with K = 2 and a dummy second source, held with x in one [2, ...] state so that no step stacks them.
+    ``noise`` ([L, n_steps_each, n, H, W, C] standard normals) injects the draws for parity runs; otherwise Philox noise
+    keyed by (seed, step, element) is generated in the kernel."""
     import torch
     from .. import ops
-    x = torch.as_tensor(np.asarray(x_mod) if not torch.is_tensor(x_mod) else x_mod, dtype=torch.float32).cuda().contiguous().clone()
-    dummy = torch.zeros_like(x)
+    x0 = torch.as_tensor(np.asarray(x_mod) if not torch.is_tensor(x_mod) else x_mod, dtype=torch.float32).cuda()
+    state = torch.zeros((2,) + tuple(x0.shape), dtype=torch.float32, device=x0.device)
+    state[0] = x0
+    x, dummy = state[0], state[1]
+    score = torch.zeros_like(state)                      # row 1: the dummy source's score, zero
     zeros = torch.zeros_like(x)
+    injected = None if noise is None else torch.zeros_like(state)   # row 1: the dummy source's draws, zero
     arr = [x.cpu().numpy().copy()] if return_arr else None
     step_no = 0
     for i, sigma in enumerate(sigmas):
@@ -88,10 +93,11 @@ def anneal_langevin_dynamics(x_mod, data_shape, model, n_samples, sigmas, n_step
         step_size = np.float32(np.float64(step_lr) * np.float64(np.float32(ratio * ratio)))
         noise_scale = np.float32(np.sqrt(np.float32(step_size * np.float32(2.0))))
         for s in range(int(n_steps_each)):
-            grad = model([x, labels], training=True)
-            n1 = None if noise is None else torch.as_tensor(noise[i][s], dtype=torch.float32)
-            ops.langevin_step(x, dummy, grad, zeros, zeros, float(step_size), 0.0, float(noise_scale), n1=n1,
-                              n2=None if n1 is None else torch.zeros_like(x), seed=seed, step=step_no)
+            score[0].copy_(model([x, labels], training=True))
+            if injected is not None:
+                injected[0].copy_(torch.as_tensor(noise[i][s], dtype=torch.float32))
+            ops.langevin_step_k(state, score, zeros, float(step_size), 0.0, float(noise_scale), noise=injected, seed=seed,
+                                step=step_no)
             dummy.zero_()
             step_no += 1
         if return_arr:

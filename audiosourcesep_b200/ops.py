@@ -60,29 +60,43 @@ def squeeze(x, inverse: bool = False) -> torch.Tensor:
     return y
 
 
+# ---- two sources: the K = 2 case of the stacked calls below, for callers that hold x1 and x2 as separate tensors
+def _pair(x1, x2) -> torch.Tensor:
+    """The stacked [2, ...] state of ``x1, x2``; the calls copy it back into them (they are updated in place)."""
+    for t in (x1, x2):
+        if not (t.is_cuda and t.dtype == torch.float32 and t.is_contiguous()):
+            raise ValueError("x1/x2 must be contiguous float32 CUDA tensors (updated in place)")
+    if x1.shape != x2.shape:
+        raise ValueError(f"x1 {tuple(x1.shape)} and x2 {tuple(x2.shape)} must have the same shape")
+    return torch.stack([x1, x2])
+
+
+def _unpair(x, x1, x2) -> None:
+    x1.copy_(x[0])
+    x2.copy_(x[1])
+
+
+def _noise_pair(n1, n2, dim: int) -> Optional[torch.Tensor]:
+    """The injected draws of both sources stacked on the source axis ``dim``, or None for in-kernel Philox noise."""
+    if (n1 is None) != (n2 is None):
+        raise ValueError("inject both noise tensors or neither")
+    return None if n1 is None else torch.stack([_prep(n1), _prep(n2)], dim)
+
+
 def mixing_db(x1, x2):
     """g(x1,x2) and grad_g (reference: run_basis_sep.py:131-147)."""
-    x1, x2 = _prep(x1), _prep(x2)
-    g, w1, w2 = torch.empty_like(x1), torch.empty_like(x1), torch.empty_like(x1)
-    t = [_lib.dl(v) for v in (x1, x2, g, w1, w2)]
-    _lib.check(_lib.load().asep_mixing_db(*(v.ptr for v in t), _lib.stream_ptr()))
-    return g, w1, w2
+    g, w = mixing_db_k(torch.stack([_prep(x1), _prep(x2)]))
+    return g, w[0], w[1]
 
 
 def langevin_step(x1, x2, s1, s2, mixed, eta: float, lam: float, noise_scale: float,
                   n1: Optional[torch.Tensor] = None, n2: Optional[torch.Tensor] = None, seed: int = 0,
                   step: int = 0, elem_offset: int = 0, nan_count: Optional[torch.Tensor] = None) -> None:
     """In-place fused update of both sources (reference: run_basis_sep.py:163-181)."""
-    for t in (x1, x2):
-        if not (t.is_cuda and t.dtype == torch.float32 and t.is_contiguous()):
-            raise ValueError("x1/x2 must be contiguous float32 CUDA tensors (updated in place)")
-    s1, s2, mixed = _prep(s1), _prep(s2), _prep(mixed)
-    n1 = None if n1 is None else _prep(n1)
-    n2 = None if n2 is None else _prep(n2)
-    t = [_lib.dl(v) for v in (x1, x2, s1, s2, mixed, n1, n2)]
-    dn = _lib.dl(nan_count)
-    _lib.check(_lib.load().asep_langevin_step(*(v.ptr for v in t), float(eta), float(lam), float(noise_scale),
-                                              int(seed), int(step), int(elem_offset), dn.ptr, _lib.stream_ptr()))
+    noise, x = _noise_pair(n1, n2, 0), _pair(x1, x2)
+    langevin_step_k(x, torch.stack([_prep(s1), _prep(s2)]), mixed, eta, lam, noise_scale, noise=noise, seed=seed, step=step,
+                    elem_offset=elem_offset, nan_count=nan_count)
+    _unpair(x, x1, x2)
 
 
 def philox_normal(shape, seed: int, step: int, stream_id: int, elem_offset: int = 0) -> torch.Tensor:
@@ -97,55 +111,35 @@ def philox_normal(shape, seed: int, step: int, stream_id: int, elem_offset: int 
 def basis_glow_inner(m1, m2, mixed, x1, x2, T: int, eta: float, lam: float, noise_scale: float,
                      noise1=None, noise2=None, seed: int = 0, step0: int = 0, elem_offset: int = 0,
                      per_step: Optional[torch.Tensor] = None, nan_count: Optional[torch.Tensor] = None) -> None:
-    """T Langevin steps at one noise level with two Glow priors, entirely inside the library."""
-    mixed = _prep(mixed)
-    noise1 = None if noise1 is None else _prep(noise1)
-    noise2 = None if noise2 is None else _prep(noise2)
-    t = [_lib.dl(v) for v in (mixed, x1, x2)]
-    dn1, dn2, dps, dnan = _lib.dl(noise1), _lib.dl(noise2), _lib.dl(per_step), _lib.dl(nan_count)
-    _lib.check(_lib.load().asep_basis_glow_inner(m1.handle, m2.handle, t[0].ptr, t[1].ptr, t[2].ptr, int(T),
-                                                 float(eta), float(lam), float(noise_scale), dn1.ptr, dn2.ptr,
-                                                 int(seed), int(step0), int(elem_offset), dps.ptr, dnan.ptr,
-                                                 _lib.stream_ptr()))
+    """T Langevin steps at one noise level with two Glow priors, entirely inside the library.  ``noise1/noise2``: [T, ...]
+    each; ``per_step``: [T, 2, ...]."""
+    noise, x = _noise_pair(noise1, noise2, 1), _pair(x1, x2)
+    basis_glow_inner_k([m1, m2], mixed, x, T, eta, lam, noise_scale, noise=noise, seed=seed, step0=step0,
+                       elem_offset=elem_offset, per_step=per_step, nan_count=nan_count)
+    _unpair(x, x1, x2)
 
 
 def basis_ncsn_inner(m1, m2, mixed, x1, x2, sigma_idx: int, T: int, eta: float, lam: float, noise_scale: float,
                      noise1=None, noise2=None, seed: int = 0, step0: int = 0, elem_offset: int = 0,
                      per_step: Optional[torch.Tensor] = None, nan_count: Optional[torch.Tensor] = None) -> None:
-    """T Langevin steps at noise level ``sigma_idx`` with two NCSN score networks, inside the library."""
-    mixed = _prep(mixed)
-    noise1 = None if noise1 is None else _prep(noise1)
-    noise2 = None if noise2 is None else _prep(noise2)
-    t = [_lib.dl(v) for v in (mixed, x1, x2)]
-    dn1, dn2, dps, dnan = _lib.dl(noise1), _lib.dl(noise2), _lib.dl(per_step), _lib.dl(nan_count)
-    _lib.check(_lib.load().asep_basis_ncsn_inner(m1.handle, m2.handle, t[0].ptr, t[1].ptr, t[2].ptr, int(sigma_idx),
-                                                 int(T), float(eta), float(lam), float(noise_scale), dn1.ptr, dn2.ptr,
-                                                 int(seed), int(step0), int(elem_offset), dps.ptr, dnan.ptr,
-                                                 _lib.stream_ptr()))
+    """T Langevin steps at noise level ``sigma_idx`` with two NCSN score networks, inside the library (arguments as
+    basis_glow_inner)."""
+    noise, x = _noise_pair(noise1, noise2, 1), _pair(x1, x2)
+    basis_ncsn_inner_k([m1, m2], mixed, x, sigma_idx, T, eta, lam, noise_scale, noise=noise, seed=seed, step0=step0,
+                       elem_offset=elem_offset, per_step=per_step, nan_count=nan_count)
+    _unpair(x, x1, x2)
 
 
 def basis_run(m1, m2, mixed, x1, x2, T: int, eta, lam, noise_scale, seed: int = 0, elem_offset: int = 0,
               snapshots: Optional[torch.Tensor] = None, nan_count: Optional[torch.Tensor] = None) -> None:
     """The whole sigma x T loop inside the library (reference: run_basis_sep.py:217-260): ``eta / lam / noise_scale`` are
     length-L sequences of the per-level float32 constants.  ``m1 / m2``: two score networks, two Glow priors, or two
-    length-L lists of Glow priors (one fine-tuned pair per noise level)."""
-    import ctypes
-    L = len(eta)
-    arr = [(ctypes.c_float * L)(*[float(v) for v in seq]) for seq in (eta, lam, noise_scale)]
-    mixed = _prep(mixed)
-    t = [_lib.dl(v) for v in (mixed, x1, x2)]
-    dsn, dnan = _lib.dl(snapshots), _lib.dl(nan_count)
-    first = m1[0] if isinstance(m1, (list, tuple)) else m1
-    if hasattr(first, "cfg") and hasattr(first.cfg, "K"):                 # Glow priors
-        l1 = list(m1) if isinstance(m1, (list, tuple)) else [m1]
-        l2 = list(m2) if isinstance(m2, (list, tuple)) else [m2]
-        h1 = (ctypes.c_void_p * len(l1))(*[m.handle.value for m in l1])
-        h2 = (ctypes.c_void_p * len(l2))(*[m.handle.value for m in l2])
-        _lib.check(_lib.load().asep_basis_glow_run(h1, h2, len(l1), t[0].ptr, t[1].ptr, t[2].ptr, L, int(T), arr[0], arr[1],
-                                                   arr[2], int(seed), int(elem_offset), dsn.ptr, dnan.ptr, _lib.stream_ptr()))
-    else:
-        _lib.check(_lib.load().asep_basis_ncsn_run(m1.handle, m2.handle, t[0].ptr, t[1].ptr, t[2].ptr, L, int(T), arr[0], arr[1],
-                                                   arr[2], int(seed), int(elem_offset), dsn.ptr, dnan.ptr, _lib.stream_ptr()))
+    length-L lists of Glow priors (one fine-tuned pair per noise level); ``snapshots``: None or [L, 2, ...]."""
+    x = _pair(x1, x2)
+    models = [[a, b] for a, b in zip(m1, m2, strict=True)] if isinstance(m1, (list, tuple)) else [m1, m2]
+    basis_run_k(models, mixed, x, T, eta, lam, noise_scale, seed=seed, elem_offset=elem_offset, snapshots=snapshots,
+                nan_count=nan_count)
+    _unpair(x, x1, x2)
 
 
 # ---- K sources (2 <= K <= 8): stacked [K, ...] states, [T, K, ...] noise / per-step dumps, [L, K, ...] snapshots

@@ -153,44 +153,38 @@ int asep_glow_coupling_nn(asep_glow_t h, int block, int step, const DLTensor* st
 int asep_glow_coupling_nn_backward(asep_glow_t h, int block, int step, const DLTensor* state, const DLTensor* gr,
                                    DLTensor* gxb, void* stream);
 
-/* ------------------------------------------------------------------ BASIS Langevin
- * One fused update of run_basis_sep.py:163-181 for both sources (dB mixing, :131-147):
- *   x_k <- x_k + eta*(s_k + lambda*softmax_k*(mixed - g(x1,x2))) + noise_scale*n_k
- * x1,x2 are updated in place from the OLD states.  n1/n2: injected standard normals, or NULL
- * for in-kernel Philox4x32-10 + Box-Muller keyed by (seed, step, global element index).
- * elem_offset = global index of element 0 (segment sharding keeps draws identical for any
- * number of GPUs).  nan_count: optional int32[1] device counter incremented per NaN. */
-int asep_langevin_step(DLTensor* x1, DLTensor* x2, const DLTensor* s1, const DLTensor* s2, const DLTensor* mixed,
-                       const DLTensor* n1, const DLTensor* n2, float eta, float lambda, float noise_scale,
-                       uint64_t seed, uint64_t step, uint64_t elem_offset, DLTensor* nan_count, void* stream);
-/* Mixing function g and its gradient (run_basis_sep.py:131-147), for tests. */
-int asep_mixing_db(const DLTensor* x1, const DLTensor* x2, DLTensor* g, DLTensor* w1, DLTensor* w2, void* stream);
-/* Standard normal draws of the in-kernel generator (for tests / reproducibility audits). */
-int asep_philox_normal(DLTensor* out, uint64_t seed, uint64_t step, uint64_t stream_id, uint64_t elem_offset,
-                       void* stream);
-/* T inner steps at one noise level with two Glow priors (run_basis_sep.py:152-181, model_type
- * 'glow').  noise1/noise2: NULL or [T,N,H,W,C] injected draws; per_step: NULL or
- * [T,2,N,H,W,C] state dump for parity tests. */
-int asep_basis_glow_inner(asep_glow_t m1, asep_glow_t m2, const DLTensor* mixed, DLTensor* x1, DLTensor* x2,
-                          int T, float eta, float lambda, float noise_scale, const DLTensor* noise1,
-                          const DLTensor* noise2, uint64_t seed, uint64_t step0, uint64_t elem_offset,
-                          DLTensor* per_step, DLTensor* nan_count, void* stream);
-
-/* ---- BASIS with K sources, 2 <= K <= 8 (any other K fails with ASEP_ERR_BAD_ARG before a launch).  Stacked layout: the
- * states, scores, injected noise, per-step dumps and snapshots of all K sources are ONE contiguous tensor with the source
- * axis after the step / level axis: x [K, ...], noise [T, K, ...], per_step [T, K, ...], snapshots [L, K, ...], where
- * ... is the shape of `mixed`.  The update is the two-source one with g = (10/ln10)(logsumexp_k(x_k ln10/10) - ln K) and
- * grad g = softmax_k; in-kernel noise of source k (0-based) is Philox stream k + 1, so K = 2 equals the two-source entry
- * points bit for bit.  The same handle may serve several sources. */
-int asep_mixing_db_k(int K, const DLTensor* x, DLTensor* g, DLTensor* w, void* stream);
+/* ------------------------------------------------------------------ BASIS Langevin with K sources, 2 <= K <= 8
+ * One fused update of run_basis_sep.py:163-181 for every source (dB mixing, :106-149):
+ *   x_k <- x_k + eta*(s_k + lambda*w_k*(mixed - g(x_1..x_K))) + noise_scale*n_k
+ * with g = (10/ln10)(logsumexp_k(x_k ln10/10) - ln K) and w_k = d g / d x_k = softmax_k.  Any other K fails with
+ * ASEP_ERR_BAD_ARG before a launch.  Stacked layout: the states, scores, injected noise, per-step dumps and snapshots of
+ * all K sources are ONE contiguous tensor with the source axis after the step / level axis: x [K, ...], score [K, ...],
+ * noise [T, K, ...], per_step [T, K, ...], snapshots [L, K, ...], where ... is the shape of `mixed`; the update needs the
+ * element count of one source to be a multiple of 4.  x is updated in place from the OLD states of all sources.  noise:
+ * injected standard normals, or NULL for in-kernel Philox4x32-10 + Box-Muller keyed by (seed, step, global element index),
+ * source k (0-based) on stream k + 1.  elem_offset = global index of element 0 of one source (segment sharding keeps the
+ * draws identical for any number of GPUs).  nan_count: optional int32[1] device counter incremented per NaN in any
+ * source.  The same handle may serve several sources. */
 int asep_langevin_step_k(int K, DLTensor* x, const DLTensor* score, const DLTensor* mixed, const DLTensor* noise, float eta,
                          float lambda, float noise_scale, uint64_t seed, uint64_t step, uint64_t elem_offset,
                          DLTensor* nan_count, void* stream);
-/* m: K Glow priors, one per source. */
+/* Mixing function g [...] and its gradient w [K, ...] of the states x [K, ...], for tests. */
+int asep_mixing_db_k(int K, const DLTensor* x, DLTensor* g, DLTensor* w, void* stream);
+/* Standard normal draws of the in-kernel generator (for tests / reproducibility audits). */
+int asep_philox_normal(DLTensor* out, uint64_t seed, uint64_t step, uint64_t stream_id, uint64_t elem_offset,
+                       void* stream);
+/* T inner steps, numbered step0 .. step0 + T - 1, at one noise level with K Glow priors m[K], one per source
+ * (run_basis_sep.py:152-181, model_type 'glow').  noise: NULL or the injected draws of every step; per_step: NULL or
+ * the state after every step, for parity tests. */
 int asep_basis_glow_inner_k(int K, const asep_glow_t* m, const DLTensor* mixed, DLTensor* x, int T, float eta, float lambda,
                             float noise_scale, const DLTensor* noise, uint64_t seed, uint64_t step0, uint64_t elem_offset,
                             DLTensor* per_step, DLTensor* nan_count, void* stream);
-/* m: n_models * K handles, level i using m[(n_models == 1 ? 0 : i) * K + k] for source k. */
+/* basis_outer_loop + basis_inner_loop (run_basis_sep.py:217-260, :152-181) entirely inside the library: L noise levels x T
+ * Langevin steps with in-kernel Philox noise (step number = level * T + t, as the Python host numbers them), no host
+ * synchronisation between levels.  eta / lambda / noise_scale: HOST arrays [L] of the float32 constants of :158-164.
+ * snapshots: NULL or device [L, K, N, H, W, C], the raw states after every level (x_arr, :243-244), copied on the
+ * stream.  m: n_models * K handles, level i using m[(n_models == 1 ? 0 : i) * K + k] for source k; n_models = L (the
+ * per-sigma fine-tuned priors the reference restores at :228-234, all resident) or 1 (one set for every level). */
 int asep_basis_glow_run_k(int K, const asep_glow_t* m, int n_models, const DLTensor* mixed, DLTensor* x, int L, int T,
                           const float* eta, const float* lambda, const float* noise_scale, uint64_t seed, uint64_t elem_offset,
                           DLTensor* snapshots, DLTensor* nan_count, void* stream);
@@ -240,28 +234,13 @@ int asep_ncsn_adam_step(asep_ncsn_t h, const DLTensor* grads, float lr, float be
                         void* stream);
 int asep_ncsn_get_flat(asep_ncsn_t h, DLTensor* theta, void* stream);
 int asep_ncsn_set_flat(asep_ncsn_t h, const DLTensor* theta, void* stream);
-/* T inner Langevin steps at noise level sigma_idx with two score networks (run_basis_sep.py:152-181, model_type
- * 'ncsn'); arguments as asep_basis_glow_inner. */
-int asep_basis_ncsn_inner(asep_ncsn_t m1, asep_ncsn_t m2, const DLTensor* mixed, DLTensor* x1, DLTensor* x2,
-                          int sigma_idx, int T, float eta, float lambda, float noise_scale, const DLTensor* noise1,
-                          const DLTensor* noise2, uint64_t seed, uint64_t step0, uint64_t elem_offset,
-                          DLTensor* per_step, DLTensor* nan_count, void* stream);
-/* basis_outer_loop + basis_inner_loop (run_basis_sep.py:217-260, :152-181) entirely inside the library: L noise levels x T
- * Langevin steps with in-kernel Philox noise (step number = level * T + t, as the Python host numbers them), no host
- * synchronisation between levels.  eta / lambda / noise_scale: HOST arrays [L] of the float32 constants of :158-164.
- * snapshots: NULL or device [L, 2, N, H, W, C], the raw states after every level (x_arr, :243-244), copied on the
- * stream.  Glow: m1 / m2 are arrays of n_models handles, n_models = L (the per-sigma fine-tuned priors the reference
- * restores at :228-234, all resident) or 1 (one pair for every level). */
-int asep_basis_glow_run(const asep_glow_t* m1, const asep_glow_t* m2, int n_models, const DLTensor* mixed, DLTensor* x1,
-                        DLTensor* x2, int L, int T, const float* eta, const float* lambda, const float* noise_scale,
-                        uint64_t seed, uint64_t elem_offset, DLTensor* snapshots, DLTensor* nan_count, void* stream);
-int asep_basis_ncsn_run(asep_ncsn_t m1, asep_ncsn_t m2, const DLTensor* mixed, DLTensor* x1, DLTensor* x2, int L, int T,
-                        const float* eta, const float* lambda, const float* noise_scale, uint64_t seed, uint64_t elem_offset,
-                        DLTensor* snapshots, DLTensor* nan_count, void* stream);
-/* K score networks m[K]; stacked layout and limits of asep_basis_glow_inner_k. */
+/* T inner Langevin steps at noise level sigma_idx with K score networks m[K], one per source (run_basis_sep.py:152-181,
+ * model_type 'ncsn'); the other arguments as asep_basis_glow_inner_k. */
 int asep_basis_ncsn_inner_k(int K, const asep_ncsn_t* m, const DLTensor* mixed, DLTensor* x, int sigma_idx, int T, float eta,
                             float lambda, float noise_scale, const DLTensor* noise, uint64_t seed, uint64_t step0,
                             uint64_t elem_offset, DLTensor* per_step, DLTensor* nan_count, void* stream);
+/* The whole sigma x T loop of asep_basis_glow_run_k with K score networks m[K], level i at sigma_idx = i (the networks are
+ * conditioned on the level, so one set serves every level). */
 int asep_basis_ncsn_run_k(int K, const asep_ncsn_t* m, const DLTensor* mixed, DLTensor* x, int L, int T, const float* eta,
                           const float* lambda, const float* noise_scale, uint64_t seed, uint64_t elem_offset,
                           DLTensor* snapshots, DLTensor* nan_count, void* stream);
@@ -358,7 +337,7 @@ int asep_griffinlim_update(const DLTensor* mag, const DLTensor* rebuilt, DLTenso
 int asep_resample(const DLTensor* audio, const DLTensor* time, const DLTensor* win, const DLTensor* delta, double scale, int step,
                   DLTensor* out, void* stream);
 
-/* CUDA-graph replay of whole Langevin steps inside asep_basis_{glow,ncsn}_inner (on by default; steps 2..T of a call
+/* CUDA-graph replay of whole Langevin steps inside asep_basis_{glow,ncsn}_inner_k (on by default; steps 2..T of a call
  * with T >= 3 are replays of one captured step whose per-step scalars live in device memory).  0 = launch every step
  * eagerly (parity tests compare the two), and drop the cached graphs. */
 int asep_basis_graphs(int on);

@@ -310,10 +310,10 @@ def test_bad_arguments_raise_before_any_launch():
     mixed, x0 = _problem(3)
     mx = torch.as_tensor(mixed)
 
-    def rejects(fn):
+    def rejects(fn, error=_lib.AsepError):
         torch.cuda.synchronize()
         n0 = _lib.launch_count()
-        with pytest.raises(_lib.AsepError):
+        with pytest.raises(error):
             fn()
         assert _lib.launch_count() == n0
 
@@ -328,6 +328,13 @@ def test_bad_arguments_raise_before_any_launch():
     rejects(lambda: ops.langevin_step_k(x[:1].contiguous(), torch.zeros((1,) + SHP), mx, 0.0, 0.0, 1.0))
     rejects(lambda: ops.mixing_db_k(torch.zeros((9, 4))))
     rejects(lambda: ops.basis_run_k(models, mx, x, 2, [1e-5], [1.0], [1e-3], snapshots=torch.zeros((2, 3) + SHP, device="cuda")))
+    # the two-source calls: one injected noise tensor without the other, or states of different shapes
+    a, b, s = x[0].clone(), x[1].clone(), torch.zeros(SHP, device="cuda")
+    noise = torch.zeros((2,) + SHP, device="cuda")
+    rejects(lambda: ops.langevin_step(a, b, s, s, mx, 0.0, 0.0, 1.0, n1=s), ValueError)
+    rejects(lambda: ops.basis_glow_inner(models[0], models[1], mx, a, b, 2, 1e-5, 1.0, 1e-3, noise2=noise), ValueError)
+    rejects(lambda: ops.langevin_step(a, b[:2].contiguous(), s, s, mx, 0.0, 0.0, 1.0), ValueError)
+    rejects(lambda: ops.basis_run(models[0], models[1], mx, a[:2].contiguous(), b, 2, [1e-5], [1.0], [1e-3]), ValueError)
 
 
 def test_run_basis_sep_glow_k3_cli_and_sdr(tmp_path):

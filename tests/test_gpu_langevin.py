@@ -159,8 +159,8 @@ def test_same_prior_for_both_sources_keeps_two_score_tensors():
 
 
 def test_device_sigma_loop_equals_the_host_loop():
-    """asep_basis_glow_run (the whole sigma x T loop inside the library, run_basis_sep.py:217-260) gives bit-identical
-    states and per-level snapshots to one asep_basis_glow_inner call per noise level."""
+    """ops.basis_run (the whole sigma x T loop inside the library, run_basis_sep.py:217-260) gives bit-identical
+    states and per-level snapshots to one ops.basis_glow_inner call per noise level."""
     from audiosourcesep_b200 import ops, _lib
     from audiosourcesep_b200.glow import Glow
     cfg = GlowConfig(H=96, W=64, C=1, L=3, K=2, n_filters=512, minval=0.0, maxval=1.0)
@@ -194,7 +194,7 @@ def test_device_sigma_loop_equals_the_host_loop():
 
 @pytest.mark.parametrize("same_handle", [False, True])
 def test_glow_step_graph_replay_equals_eager_launches(same_handle):
-    """Steps 2..T of asep_basis_glow_inner are replays of ONE captured CUDA graph (both scores as parallel branches when
+    """Steps 2..T of ops.basis_glow_inner are replays of ONE captured CUDA graph (both scores as parallel branches when
     the priors are two handles, per-step scalars in device memory): states and the per-step dump must equal those of
     eager launches, for in-kernel Philox noise and across two consecutive calls that reuse the cached graph."""
     from audiosourcesep_b200 import ops, _lib

@@ -180,7 +180,7 @@ def test_score_is_sample_wise_at_the_bench_size(version):
 
 @pytest.mark.parametrize("version", ["v1", "v2"])
 def test_ncsn_step_graph_replay_equals_eager_launches(version):
-    """asep_basis_ncsn_inner replays steps 2..T as one captured CUDA graph (the two score networks as parallel branches):
+    """ops.basis_ncsn_inner replays steps 2..T as one captured CUDA graph (the two score networks as parallel branches):
     same states as eager launches (the instance-norm statistics are accumulated with double atomics, whose order may
     differ in the last bit, hence a 1e-6 bound instead of bit equality)."""
     from audiosourcesep_b200 import ops, _lib
