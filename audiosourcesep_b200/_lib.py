@@ -131,6 +131,8 @@ _SIGNATURES = {
     "asep_istft": [_P, _I, _P, _V],
     "asep_istft_track": [_P, _I, _I, _P, _V],
     "asep_griffinlim_update": [_P, _P, _P, _P, _F, _V],
+    "asep_track_psd": [_P, _I, _I, _I, _I, _I, _I, _I, _P, _V],
+    "asep_mwf": [_P, _P, _I, _P, _V],
     "asep_resample": [_P, _P, _P, _P, ctypes.c_double, _I, _P, _V],
     "asep_basis_graphs": [_I],
     "asep_hbm_profile": [_I],

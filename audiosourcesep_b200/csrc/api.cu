@@ -9,6 +9,7 @@
 #include "bsseval.h"
 #include "glow_model.h"
 #include "mel_kernels.h"
+#include "mwf_kernels.h"
 #include "ncsn_model.h"
 #include "ncsn_train_kernels.h"
 #include "resample_kernels.h"
@@ -1427,6 +1428,49 @@ int asep_istft_track(const DLTensor* stft, int hop, int overlap_frames, DLTensor
     throw;
   }
   CUDA_CHECK(cudaFreeAsync(frames, s));
+  ASEP_API_END
+}
+
+// ------------------------------------------------------------------ multichannel Wiener-mask rendering (mwf_kernels.cu)
+int asep_track_psd(const DLTensor* mag, int hop, int overlap_frames, int bin_lo, int bin_hi, int out_sr, int out_n_fft,
+                   int out_hop, DLTensor* psd, void* stream) {
+  ASEP_API_BEGIN
+  ASEP_CHECK(g_device >= 0, ASEP_ERR_STATE, "asep_init() has not been called");
+  TView m = view_f32(mag, "mag", g_device), o = view_f32(psd, "psd", g_device);
+  ASEP_CHECK(m.ndim == 4 && m.shape[1] >= 1 && m.shape[2] >= 2 && m.shape[3] >= 2, ASEP_ERR_BAD_SHAPE,
+             "track_psd: mag must be [K, n_seg, F, T]");
+  const int K = (int)m.shape[0], n_seg = (int)m.shape[1], F = (int)m.shape[2], T = (int)m.shape[3];
+  ASEP_CHECK(K >= 2 && K <= kMaxSources, ASEP_ERR_BAD_ARG, "track_psd: the number of sources K must be in [2, %d] (got %d)",
+             kMaxSources, K);
+  ASEP_CHECK(hop >= 1 && out_hop >= 1 && out_sr >= 1, ASEP_ERR_BAD_ARG, "track_psd: hop = %d, out_hop = %d, out_sr = %d",
+             hop, out_hop, out_sr);
+  ASEP_CHECK(overlap_frames >= 0 && 2 * overlap_frames < T - 1, ASEP_ERR_BAD_ARG,
+             "track_psd: overlap_frames = %d outside 0..%d for segments of %d frames", overlap_frames, (T - 2) / 2, T);
+  ASEP_CHECK(bin_lo >= 0 && bin_lo <= bin_hi && bin_hi < F, ASEP_ERR_BAD_ARG, "track_psd: bins [%d, %d] outside 0..%d",
+             bin_lo, bin_hi, F - 1);
+  ASEP_CHECK(out_n_fft >= 2 && out_n_fft % 2 == 0, ASEP_ERR_BAD_ARG, "track_psd: out_n_fft = %d", out_n_fft);
+  ASEP_CHECK(o.ndim == 3 && o.shape[0] == K && o.shape[1] == out_n_fft / 2 + 1 && o.shape[2] >= 1, ASEP_ERR_BAD_SHAPE,
+             "track_psd: psd must be [K = %d, out_n_fft/2 + 1 = %d, T_out]", K, out_n_fft / 2 + 1);
+  launch_track_psd(m.f32, o.f32, K, n_seg, F, T, hop, overlap_frames, bin_lo, bin_hi, out_sr, out_n_fft, out_hop,
+                   (int)o.shape[1], (int)o.shape[2], as_stream(stream));
+  ASEP_API_END
+}
+
+int asep_mwf(const DLTensor* psd, const DLTensor* stft_mix, int iterations, DLTensor* out, void* stream) {
+  ASEP_API_BEGIN
+  ASEP_CHECK(g_device >= 0, ASEP_ERR_STATE, "asep_init() has not been called");
+  TView p = view_f32(psd, "psd", g_device), x = view_f32(stft_mix, "stft_mix", g_device), o = view_f32(out, "out", g_device);
+  ASEP_CHECK(p.ndim == 3 && x.ndim == 4 && x.shape[3] == 2, ASEP_ERR_BAD_SHAPE,
+             "mwf: psd must be [K, F, T] and stft_mix [C, F, T, 2]");
+  const int K = (int)p.shape[0], C = (int)x.shape[0], F = (int)p.shape[1], T = (int)p.shape[2];
+  ASEP_CHECK(K >= 2 && K <= kMaxSources, ASEP_ERR_BAD_ARG, "mwf: the number of sources K must be in [2, %d] (got %d)",
+             kMaxSources, K);
+  ASEP_CHECK(C == 1 || C == 2, ASEP_ERR_BAD_ARG, "mwf: %d channels; 1 or 2 are supported", C);
+  ASEP_CHECK(iterations >= 0 && iterations <= kMwfMaxIterations, ASEP_ERR_BAD_ARG, "mwf: iterations = %d outside 0..%d",
+             iterations, kMwfMaxIterations);
+  expect_shape(x, "stft_mix", {C, F, T, 2});
+  expect_shape(o, "out", {K, C, F, T, 2});
+  launch_mwf(p.f32, x.f32, o.f32, K, C, F, T, iterations, as_stream(stream));
   ASEP_API_END
 }
 

@@ -41,9 +41,10 @@ def _riff_chunks(path: str):
     return fmt, data
 
 
-def read_wav_mono(path: str):
-    """wav -> (float32 mono, rate), scaled as soundfile reads it: PCM of 8 bits ((u - 128) / 128), 16 bits (/ 2^15),
-    24 bits (/ 2^23) or 32 bits (/ 2^31); 32-bit IEEE float as stored.  Channels are averaged."""
+def read_wav(path: str):
+    """wav -> (float32 [C, L], rate), scaled as soundfile reads it: PCM of 8 bits ((u - 128) / 128), 16 bits (/ 2^15),
+    24 bits (/ 2^23) or 32 bits (/ 2^31); 32-bit IEEE float as stored.  The array is a channel-major view of the
+    interleaved samples."""
     fmt, raw = _riff_chunks(path)
     tag, nch, rate, _, block_align, bits = struct.unpack("<HHIIHH", fmt[:16])
     if tag == _WAVE_FORMAT_EXTENSIBLE:
@@ -69,9 +70,16 @@ def read_wav_mono(path: str):
     else:
         kind = {_WAVE_FORMAT_PCM: "PCM", _WAVE_FORMAT_IEEE_FLOAT: "IEEE float"}.get(tag, f"format tag 0x{tag:04x}")
         raise ValueError(f"{path}: unsupported wav format: {kind}, {bits} bits per sample")
-    if nch > 1:
-        a = a.reshape(-1, nch).mean(axis=1)
-    return a, rate
+    return a.reshape(-1, nch).T, rate
+
+
+def read_wav_mono(path: str):
+    """wav -> (float32 [L], rate): read_wav with the channels averaged."""
+    x, rate = read_wav(path)
+    a = x.T                                                # the interleaved [L, C] frames
+    if a.shape[1] > 1:
+        return a.mean(axis=1), rate
+    return a.reshape(-1), rate
 
 
 def load_wav(path, length_sec, sr=None):

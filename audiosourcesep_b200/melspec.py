@@ -128,6 +128,37 @@ def stft_filter(mags: torch.Tensor, stft_mixture: torch.Tensor, wiener_filter: b
     return torch.view_as_complex(out)
 
 
+def band_edges(sr=16000, n_fft=2048, n_mels=96, fmin=125.0, fmax=7600.0):
+    """(bin_lo, bin_hi): the first and last STFT bins that some mel filter covers."""
+    cover = np.flatnonzero((mel_filters(sr, n_fft, n_mels, fmin, fmax) > 0).any(axis=0))
+    return int(cover[0]), int(cover[-1])
+
+
+def track_psd(mags: torch.Tensor, overlap_frames: int, bin_lo: int, bin_hi: int, out_sr: int, out_n_fft: int, out_hop: int,
+              frames: int, hop_length: int = 512) -> torch.Tensor:
+    """mags [K, n_seg, F, T] (16 kHz segment magnitudes) -> float32 [K, out_n_fft/2 + 1, frames]: the sources' track powers
+    mapped onto the output STFT grid (asep_track_psd; restated in oracle/mwf_oracle.py:track_psd)."""
+    m = mags.contiguous().float()
+    _dev(m.device.index)
+    out = torch.empty((m.shape[0], int(out_n_fft) // 2 + 1, int(frames)), dtype=torch.float32, device=m.device)
+    dm, do = _lib.dl(m), _lib.dl(out)
+    _lib.check(_lib.load().asep_track_psd(dm.ptr, int(hop_length), int(overlap_frames), int(bin_lo), int(bin_hi), int(out_sr),
+                                          int(out_n_fft), int(out_hop), do.ptr, _lib.stream_ptr()))
+    return out
+
+
+def mwf(psd: torch.Tensor, stft_mixture: torch.Tensor, iterations: int = 1) -> torch.Tensor:
+    """psd [K, F, T] (power), stft_mixture complex64 [C, F, T] -> complex64 [K, C, F, T]: the multichannel Wiener filter
+    with ``iterations`` EM steps and mixture consistency (asep_mwf; restated in oracle/mwf_oracle.py:mwf)."""
+    p = psd.contiguous().float()
+    x = torch.view_as_real(stft_mixture.contiguous()).contiguous()
+    _dev(p.device.index)
+    out = torch.empty((p.shape[0],) + tuple(x.shape), dtype=torch.float32, device=p.device)
+    dp, dx, do = _lib.dl(p), _lib.dl(x), _lib.dl(out)
+    _lib.check(_lib.load().asep_mwf(dp.ptr, dx.ptr, int(iterations), do.ptr, _lib.stream_ptr()))
+    return torch.view_as_complex(out)
+
+
 def istft(stft_c: torch.Tensor, hop_length: int = 512) -> torch.Tensor:
     """librosa.istft(hop_length, window='hann', center=True): complex64 [N, F, T] -> float32 [N, hop (T-1)]."""
     s = torch.view_as_real(stft_c.contiguous()).contiguous()

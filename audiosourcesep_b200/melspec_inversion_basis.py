@@ -3,7 +3,8 @@
 BASIS run, inverts x1 / x2 / gt1 / gt2 / mixed with the mixture's phase (optionally through the single-channel Wiener
 filter) and writes ``inverse_spectrograms.npz`` + 16-bit wav files.  The transforms run on the GPU (melspec.py).
 ``--algorithm griffin`` runs Griffin-Lim (:21-39; 32 iterations, momentum 0.99) on the same STFT / iSTFT kernels.
-Results of ``run_basis_sep --mix`` (a ``segment_start`` key) are inverted as whole tracks instead (track.invert_track)."""
+Results of ``run_basis_sep --mix`` (a ``segment_start`` key) are inverted as whole tracks instead (track.invert_track),
+or, with ``--render mask --mix PATH``, rendered as multichannel Wiener masks on that recording (track.render_results)."""
 from __future__ import annotations
 
 import argparse
@@ -62,22 +63,33 @@ def griffin_inversion_fn(sr=16000, fmin=125, fmax=7600, n_fft=2048, hop_length=5
 
 
 def write_wav(path: str, data: np.ndarray, samplerate: int) -> None:
+    """16-bit PCM wav of ``data``: [L] (mono) or [C, L] (C channels)."""
     pcm = np.clip(np.asarray(data, dtype=np.float64), -1.0, 1.0 - 1.0 / 32768.0)
+    channels = 1 if pcm.ndim == 1 else pcm.shape[0]
     with wave.open(path, "wb") as w:
-        w.setnchannels(1)
+        w.setnchannels(channels)
         w.setsampwidth(2)
         w.setframerate(int(samplerate))
-        w.writeframes((pcm * 32768.0).astype("<i2").tobytes())
+        w.writeframes((pcm.T.reshape(-1) * 32768.0).astype("<i2").tobytes())
 
 
 def main(args):
     sr, fmin, fmax, n_fft, hop_length = 16000, 125, 7600, 2048, 512
     res = np.load(os.path.join(args.basis_results, "results.npz"))
-    out_dir = args.output or os.path.join(args.basis_results, "inverse_" + args.algorithm + "_" + args.method + ("_wiener_filter" if args.wiener_filter else ""))
+    render = getattr(args, "render", "mel")
+    if render == "mask":
+        check_mask_args(args, "segment_start" in res.files)
+        out_dir = args.output or os.path.join(args.basis_results, "inverse_mask")
+    elif args.mix is not None or args.mwf_iterations is not None:
+        raise ValueError("--mix and --mwf_iterations belong to --render mask")
+    else:
+        out_dir = args.output or os.path.join(args.basis_results, "inverse_" + args.algorithm + "_" + args.method + ("_wiener_filter" if args.wiener_filter else ""))
     os.makedirs(out_dir, exist_ok=True)
     if args.algorithm not in ("reuse_phase", "griffin"):
         raise ValueError("method should be griffin or reuse_phase")                 # :197-198
     K = sum(1 for k in res.files if re.fullmatch(r"x[0-9]+", k))                   # one x{k} / gt{k} pair per source
+    if render == "mask":
+        return _main_mask(args, res, out_dir, K)
     if "segment_start" in res.files:                                               # a whole track (run_basis_sep --mix)
         return _main_track(args, res, out_dir, K)
     xs = [res[f"x{k + 1}"] for k in range(K)]
@@ -125,6 +137,31 @@ def _main_track(args, res, out_dir, K):
     return {f"x{k + 1}_audio": tracks[k] for k in range(K)}
 
 
+def check_mask_args(args, whole_track: bool) -> None:
+    """--render mask re-renders a whole-track results directory from the recording it was separated from (--mix)."""
+    if not whole_track:
+        raise ValueError("--render mask needs the results of run_basis_sep --mix (a whole track)")
+    if args.mix is None:
+        raise ValueError("--render mask needs --mix PATH, the recording the results were separated from")
+    if args.wiener_filter or args.algorithm != "reuse_phase":
+        raise ValueError("--render mask is a Wiener filter of its own; --wiener_filter and --algorithm do not apply")
+    if args.mwf_iterations is not None:
+        from .track import check_mwf_iterations
+        check_mwf_iterations(args.mwf_iterations)
+
+
+def _main_mask(args, res, out_dir, K):
+    """Mask rendering of a whole track (track.render_results): sep{k}.wav with the recording's channels, rate and length,
+    and the float32 tracks [C, L] in separated.npz."""
+    from . import track
+    t0 = time.time()
+    n_iter = 1 if args.mwf_iterations is None else args.mwf_iterations
+    tracks = track.render_results({k: res[k] for k in res.files}, args.mix, n_iter)
+    print("Rendering duration: {} seconds".format(round(time.time() - t0, 4)))
+    track.write_tracks(out_dir, [f"sep{k + 1}" for k in range(K)], tracks, int(res["orig_sr"]))
+    return {f"x{k + 1}_audio": tracks[k] for k in range(K)}
+
+
 def build_parser():
     p = argparse.ArgumentParser(description="Spectrograms Inversion")
     p.add_argument("basis_results", type=str)
@@ -134,6 +171,12 @@ def build_parser():
     p.add_argument("--scale", type=str, default="dB")
     p.add_argument("--wiener_filter", action="store_true")
     p.add_argument("--debug", action="store_true")
+    p.add_argument("--render", choices=("mel", "mask"), default="mel",
+                   help="whole tracks only: mel (default) inverts the separated mel spectrograms at 16 kHz; mask renders "
+                        "them as multichannel Wiener masks on the recording given by --mix (its channels, rate and band)")
+    p.add_argument("--mix", type=str, default=None, metavar="PATH", help="with --render mask: the separated recording")
+    p.add_argument("--mwf_iterations", type=int, default=None, metavar="N",
+                   help="with --render mask: EM iterations of the Wiener filter, 0..10 (default 1)")
     return p
 
 

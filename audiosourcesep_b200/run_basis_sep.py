@@ -29,7 +29,8 @@ all of one ``model_type``), the stems named by ``--sources`` (``piano,violin`` b
 segments (``--overlap_frames``, default 8), nothing skipped or dropped; ``results.npz`` then holds x1..xK / mixed /
 stft_mixture over all segments plus ``segment_start``, ``track_length``, ``orig_sr``, ``orig_length`` and
 ``overlap_frames`` (no gt keys), and rank 0 writes ``<output>/<source name>.wav`` at the input's rate and length and
-``separated.npz`` with the float32 tracks.
+``separated.npz`` with the float32 tracks.  ``--render mask [--mwf_iterations N]`` makes those stems as multichannel Wiener
+masks on the recording itself instead (track.render_track): they keep its channels and full band and sum to it.
 
 Segments are independent (SURVEY.md 8(e)): under ``torchrun`` every rank separates a contiguous block of
 segments with noise keyed by the GLOBAL element index, and rank 0 gathers the blocks at the end -- the
@@ -452,12 +453,31 @@ def build_parser() -> argparse.ArgumentParser:
                         "over, 0..31 (0: hard cuts)")
     p.add_argument("--wiener_filter", action="store_true",
                    help="with --mix: invert through the K-source Wiener filter instead of the mixture's phase")
+    p.add_argument("--render", choices=("mel", "mask"), default="mel",
+                   help="with --mix: how the stems are made from the separated mel spectrograms.  mel (default): inverted at "
+                        "16 kHz (mono, 133 Hz .. 7.6 kHz) and resampled; mask: multichannel Wiener masks applied to the "
+                        "recording itself (its channels, rate and full band; the stems sum to it)")
+    p.add_argument("--mwf_iterations", type=int, default=None, metavar="N",
+                   help="with --render mask: EM iterations of the multichannel Wiener filter, 0..10 (default 1)")
     return p
 
 
 def check_mix_args(args) -> None:
     """Flag rules of the whole-track mode (--mix), checked before anything runs on the device: no --song_dir / --synthetic
-    next to it, --overlap_frames in 0..31, and --sources (if given) naming one output per restore directory."""
+    next to it, --overlap_frames in 0..31, --sources (if given) naming one output per restore directory, and --render mask
+    only with --mix, without --wiener_filter, with --mwf_iterations in 0..10 (which belongs to --render mask alone)."""
+    render = getattr(args, "render", "mel")
+    iterations = getattr(args, "mwf_iterations", None)
+    if render == "mask":
+        if getattr(args, "mix", None) is None:
+            raise ValueError("--render mask renders a whole recording: it needs --mix")
+        if args.wiener_filter:
+            raise ValueError("--render mask is a multichannel Wiener filter of its own; --wiener_filter does not apply")
+        if iterations is not None:
+            from .track import check_mwf_iterations
+            check_mwf_iterations(iterations)
+    elif iterations is not None:
+        raise ValueError("--mwf_iterations belongs to --render mask")
     if getattr(args, "mix", None) is None:
         return
     if args.song_dir is not None or getattr(args, "synthetic", False):
@@ -474,7 +494,7 @@ def merge_config(args: argparse.Namespace) -> argparse.Namespace:
     cfg = vars(get_config(args.config))
     keep = ("dataset", "debug", "output", "song_dir", "inverse", "model_type", "n_mixed", "RESTORE1", "RESTORE2",
             "synthetic", "random_init", "seed", "config", "fast", "precision", "exact", "host_loop", "RESTORE", "sources", "mix",
-            "overlap_frames", "wiener_filter")
+            "overlap_frames", "wiener_filter", "render", "mwf_iterations")
     merged = dict(vars(args))
     for k, v in cfg.items():
         if k not in keep:
@@ -487,6 +507,7 @@ def main(args) -> Optional[Dict[str, np.ndarray]]:
     import torch
     import torch.distributed as dist
 
+    from . import track
     args = merge_config(args)
     check_mix_args(args)
     mix_mode = getattr(args, "mix", None) is not None
@@ -524,6 +545,8 @@ def main(args) -> Optional[Dict[str, np.ndarray]]:
     try:
         t0 = time.time()
         if mix_mode:
+            mask = getattr(args, "render", "mel") == "mask"
+            audio = track.read_track_channels(os.path.abspath(args.mix)) if mask else None     # > 2 channels fail here
             mix_db, stft_mixture, seg = load_mix_patches(args)
             gts, K = None, len(restore_dirs(args))
         else:
@@ -559,7 +582,6 @@ def main(args) -> Optional[Dict[str, np.ndarray]]:
         results = None
         if rank == 0:
             if mix_mode:
-                from . import track
                 results = track.track_results([post_processing(x_all[k].squeeze(-1)) for k in range(K)],
                                               post_processing(mixed_full.squeeze(-1)), stft_mixture, seg["starts"],
                                               seg["track_length"], seg["orig_sr"], seg["orig_length"], args.overlap_frames)
@@ -572,7 +594,11 @@ def main(args) -> Optional[Dict[str, np.ndarray]]:
                      **{f"x{k + 1}": post_processing(conv[k]) for k in range(K)})
             if mix_mode:                                                 # whole-track back end: one wav per source
                 t2 = time.time()
-                tracks = track.invert_results(results, args.wiener_filter)
+                if mask:
+                    n_iter = 1 if args.mwf_iterations is None else args.mwf_iterations
+                    tracks = track.render_results(results, os.path.abspath(args.mix), n_iter, audio)
+                else:
+                    tracks = track.invert_results(results, args.wiener_filter)
                 names = source_names(args)
                 track.write_tracks(out_dir, names, tracks, seg["orig_sr"])
                 print("Inversion duration: {} seconds".format(round(time.time() - t2, 3)))

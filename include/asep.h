@@ -327,6 +327,26 @@ int asep_istft_track(const DLTensor* stft, int hop, int overlap_frames, DLTensor
 int asep_griffinlim_update(const DLTensor* mag, const DLTensor* rebuilt, DLTensor* tprev, DLTensor* next, float momentum,
                            void* stream);
 
+/* ------------------------------------------------------------------ multichannel Wiener-mask rendering of a whole track
+ * Renders the K sources' STFT magnitudes of a whole-track separation (16 kHz mel grid, asep_mel_to_stft) as stems of the
+ * ORIGINAL recording: at its own rate and channel count, full band, summing to it (restated in oracle/mwf_oracle.py).
+ * asep_track_psd: mag [K, n_seg, F, T] (segment g starts at 16 kHz track frame g (T - 1 - overlap_frames); F = 1025,
+ *   T = 64, hop = 512 for the shipped grid) -> psd [K, out_n_fft/2 + 1, T_out], the source powers on the output STFT grid:
+ *   segments sharing a frame blend mag^2 with the cross-fade weight asep_istft_track gives the frame's centre sample;
+ *   output frame u maps to the fractional 16 kHz frame out_hop u 16000 / (out_sr hop) (clamped to the track), output bin b
+ *   to the fractional 16 kHz bin b out_sr (2 (F - 1)) / (out_n_fft 16000), clamped to [bin_lo, bin_hi] (the bins the mel
+ *   filters cover, so out-of-band content takes the gains of the nearest covered bin); bilinear in power.  K outside 2..8,
+ *   0 <= 2 overlap_frames < T - 1 violated or bins outside 0 <= bin_lo <= bin_hi < F: ASEP_ERR_BAD_ARG before a launch.
+ * asep_mwf: psd [K, F, T] and the mixture's stft_mix [C, F, T, 2] -> out [K, C, F, T, 2]: the multichannel Wiener filter
+ *   with `iterations` EM steps (norbert's expectation_maximization; eps = 1e-10, per-frequency C x C spatial covariances
+ *   R_k), the residual x - sum_k y_k shared equally among the sources after every step, so the stems sum to the mixture.
+ *   One CTA per frequency row streams it iterations + 1 times (float64 per-bin algebra, fixed-order reductions: bitwise
+ *   reproducible).  K outside 2..8, C outside {1, 2} or iterations outside 0..10: ASEP_ERR_BAD_ARG; shapes that do not
+ *   match: ASEP_ERR_BAD_SHAPE; both before a launch. */
+int asep_track_psd(const DLTensor* mag, int hop, int overlap_frames, int bin_lo, int bin_hi, int out_sr, int out_n_fft,
+                   int out_hop, DLTensor* psd, void* stream);
+int asep_mwf(const DLTensor* psd, const DLTensor* stft_mix, int iterations, DLTensor* out, void* stream);
+
 /* ------------------------------------------------------------------ resampling
  * Replaces the resampler of librosa.load(path, sr=16000) (datasets/preprocessing.py:9-26; librosa's default
  * res_type='kaiser_best' = resampy.resample): audio [N, L_in] fp32 -> out [N, L_out] fp32.  time [L_out] float64 is
