@@ -91,6 +91,8 @@ _SIGNATURES = {
     "asep_squeeze": [_P, _P, _I, _V],
     "asep_glow_coupling_nn": [_V, _I, _I, _P, _P, _V],
     "asep_glow_coupling_nn_backward": [_V, _I, _I, _P, _P, _P, _V],
+    "asep_glow_coupling_tc": [_V, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _V],
+    "asep_glow_wgrad_tc": [_P, _P, _I, _P, _V],
     "asep_philox_normal": [_P, _U64, _U64, _U64, _U64, _V],
     "asep_ncsn_create": [ctypes.POINTER(NcsnCfg), ctypes.POINTER(_V)],
     "asep_ncsn_destroy": [_V],

@@ -1236,6 +1236,91 @@ int asep_conv_wgrad_tc(const DLTensor* x, const DLTensor* g, DLTensor* dk, int k
   ASEP_API_END
 }
 
+// ---- the tcgen05 coupling network of the Glow prior one launch at a time (tests/test_gpu_coupling_tc.py): thin wrappers
+// over nn_tc_* / nn_tcx_* and wgrad_tc that check every argument before anything is launched
+int asep_glow_coupling_tc(asep_glow_t h, int block, int step, int backward, const DLTensor* src, DLTensor* mask1,
+                          DLTensor* mask2, DLTensor* dump1, DLTensor* dump2, DLTensor* G, DLTensor* out, void* stream) {
+  ASEP_API_BEGIN
+  ASEP_CHECK(h, ASEP_ERR_BAD_ARG, "NULL handle");
+  GlowModel& m = *h->model;
+  ASEP_CHECK(backward == 0 || backward == 1, ASEP_ERR_BAD_ARG, "backward is 0 or 1");
+  ASEP_CHECK(block >= 0 && block < m.cfg().L && step >= 0 && step < m.cfg().K, ASEP_ERR_BAD_ARG,
+             "block %d / step %d out of range (%d blocks, %d steps)", block, step, m.cfg().L, m.cfg().K);
+  const NNWeightsTC& w = m.tc_weights(block, step);
+  ASEP_CHECK(m.is_tc(), ASEP_ERR_UNSUPPORTED, "the handle is prepared in a CUDA-core precision: no tcgen05 coupling network");
+  const bool tcx = m.is_tcx();
+  ASEP_CHECK(!tcx || (dump1 == nullptr && dump2 == nullptr), ASEP_ERR_UNSUPPORTED,
+             "the split-precision kernels write no activation copies");
+  ASEP_CHECK(backward ? (mask1 != nullptr && mask2 != nullptr) : ((mask1 == nullptr) == (mask2 == nullptr)), ASEP_ERR_BAD_ARG,
+             backward ? "the data gradient reads both ReLU masks" : "the forward writes both ReLU masks or neither");
+  const Level& lv = m.level(block);
+  const int dev = m.device();
+  TView sv = view_f32(src, "src", dev);
+  expect_shape(sv, "src", {-1, lv.H, lv.W, lv.C});
+  const int N = (int)sv.shape[0];
+  const long long M = (long long)N * lv.H * lv.W;
+  uint32_t* mk[2] = {nullptr, nullptr};
+  DLTensor* masks[2] = {mask1, mask2};
+  for (int i = 0; i < 2; ++i)
+    if (masks[i]) {
+      TView v = view_i32(masks[i], i ? "mask2" : "mask1", dev);
+      expect_shape(v, i ? "mask2" : "mask1", {M, kTcF / 32});
+      mk[i] = reinterpret_cast<uint32_t*>(v.raw);
+    }
+  __nv_bfloat16* dp[2] = {nullptr, nullptr};
+  DLTensor* dumps[2] = {dump1, dump2};
+  for (int i = 0; i < 2; ++i)
+    if (dumps[i]) {
+      TView v = view_any(dumps[i], i ? "dump2" : "dump1", dev, false, kDLBfloat, 16);
+      expect_shape(v, i ? "dump2" : "dump1", {M, kTcF});
+      dp[i] = static_cast<__nv_bfloat16*>(v.raw);
+    }
+  const int n3p = backward ? w.bwd.n3p : w.fwd.n3p;
+  TView gv = view_f32(G, "G", dev);
+  expect_shape(gv, "G", {tcx ? 2 : 1, (M + 127) / 128 * 128 * n3p});
+  float* op = nullptr;
+  if (out) {
+    TView ov = view_f32(out, "out", dev);
+    expect_shape(ov, "out", {N, lv.H, lv.W, backward ? lv.C / 2 : lv.C});
+    op = ov.f32;
+  }
+  NNScratchTC sc;
+  sc.G = gv.f32;
+  const cudaStream_t s = as_stream(stream);
+  if (tcx) {
+    if (backward) nn_tcx_backward(w, sc, sv.f32, mk[0], mk[1], op, N, lv.H, lv.W, lv.C, s);
+    else nn_tcx_forward(w, sc, sv.f32, op, mk[0], mk[1], N, lv.H, lv.W, lv.C, s);
+  } else {
+    if (backward) nn_tc_backward(w, sc, sv.f32, mk[0], mk[1], op, N, lv.H, lv.W, lv.C, s, dp[0], dp[1]);
+    else nn_tc_forward(w, sc, sv.f32, op, mk[0], mk[1], N, lv.H, lv.W, lv.C, s, dp[0], dp[1]);
+  }
+  ASEP_API_END
+}
+
+int asep_glow_wgrad_tc(const DLTensor* A, const DLTensor* B, int n_valid, DLTensor* out, void* stream) {
+  ASEP_API_BEGIN
+  ASEP_CHECK(g_device >= 0, ASEP_ERR_STATE, "asep_init() has not been called");
+  TView av = view_bf16(A, "A");
+  ASEP_CHECK(av.ndim == 2, ASEP_ERR_BAD_SHAPE, "A: expected [P, %d]", kTcF);
+  expect_shape(av, "A", {-1, kTcF});
+  const long long P = av.shape[0];
+  TView bv = view_bf16(B, "B");
+  ASEP_CHECK(bv.ndim == 2, ASEP_ERR_BAD_SHAPE, "B: expected [P, ldb]");
+  expect_shape(bv, "B", {P, -1});
+  const int ldb = (int)bv.shape[1];
+  ASEP_CHECK(ldb > 0 && ldb % 64 == 0 && (ldb <= 256 || ldb % 256 == 0), ASEP_ERR_UNSUPPORTED,
+             "wgrad_tc: ldb = %d, a multiple of 64 up to 256 and of 256 above", ldb);
+  ASEP_CHECK(n_valid >= 1 && n_valid <= ldb, ASEP_ERR_BAD_ARG, "n_valid = %d outside 1..ldb = %d", n_valid, ldb);
+  TView ov = view_f32(out, "out", g_device);
+  ASEP_CHECK(ov.ndim == 2, ASEP_ERR_BAD_SHAPE, "out: expected [%d, ldo]", kTcF);
+  expect_shape(ov, "out", {kTcF, -1});
+  const int ldo = (int)ov.shape[1];
+  ASEP_CHECK(ldo >= n_valid, ASEP_ERR_BAD_SHAPE, "out: %d columns, n_valid = %d", ldo, n_valid);
+  wgrad_tc(static_cast<const __nv_bfloat16*>(av.raw), static_cast<const __nv_bfloat16*>(bv.raw), ldb, n_valid, ov.f32, ldo,
+           P, as_stream(stream));
+  ASEP_API_END
+}
+
 // CRC-32C (Castagnoli), slicing-by-8, host only: checksums of the TensorFlow checkpoint interchange
 // (audiosourcesep_b200/tf_checkpoint.py; the TensorBundle format stores a masked crc32c per tensor and per index block).
 uint32_t asep_crc32c(const void* data, uint64_t n, uint32_t crc) {

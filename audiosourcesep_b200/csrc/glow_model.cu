@@ -325,8 +325,13 @@ void GlowModel::prepare(int precision) {
   ASEP_CHECK(!(training_ && tcx_mode), ASEP_ERR_UNSUPPORTED,
              "the split-precision modes have no weight-gradient path: train in ASEP_PREC_BF16 / FP16 / FP32");
   const int F = cfg_.n_filters;
-  if (tc_mode)
+  if (tc_mode) {
     ASEP_CHECK(F == kTcF, ASEP_ERR_UNSUPPORTED, "the tcgen05 modes need n_filters = %d (got %d)", kTcF, F);
+    for (int b = 0; b < cfg_.L; ++b)
+      ASEP_CHECK(nn_tc_supported(levels_[b].C), ASEP_ERR_UNSUPPORTED,
+                 "the tcgen05 coupling kernels are built for level widths 4, 8 and 16 (block %d has %d channels)", b,
+                 levels_[b].C);
+  }
   CUDA_CHECK(cudaSetDevice(device_));
   invalidate_graphs();                       // the per-step constants and tile images below are re-allocated
   refresh_dirty_ = true;                     // ... and so are the pointers in the device-side refresh table

@@ -91,6 +91,13 @@ class GlowModel {
   const Level& level(int b) const { return levels_[b]; }
   int latent_dims() const { return Dl_; }
   int precision() const { return precision_; }
+  bool is_tcx() const { return precision_ == ASEP_PREC_BF16X2 || precision_ == ASEP_PREC_FP16X2 || precision_ == ASEP_PREC_FP16X3; }   // split-precision tcgen05
+  bool is_tc() const { return precision_ == ASEP_PREC_BF16 || precision_ == ASEP_PREC_FP16 || is_tcx(); }   // tcgen05 modes
+  // prepared tile images and constants of the tensor-core coupling network of (block, step) (asep_glow_coupling_tc)
+  const NNWeightsTC& tc_weights(int b, int k) const {
+    require_prepared();
+    return steps_[(size_t)b * cfg_.K + k].wtc;
+  }
   // identity of the device allocations a captured graph of this model's kernels would bake in: a process-unique id of
   // the handle and a counter that advances whenever the workspace, the per-step constants or the tile images move
   long long uid() const { return uid_; }
@@ -206,8 +213,6 @@ class GlowModel {
   std::vector<StepDerived> steps_;
   bool prepared_ = false;
   int precision_ = ASEP_PREC_FP32;
-  bool is_tcx() const { return precision_ == ASEP_PREC_BF16X2 || precision_ == ASEP_PREC_FP16X2 || precision_ == ASEP_PREC_FP16X3; }   // split-precision tcgen05
-  bool is_tc() const { return precision_ == ASEP_PREC_BF16 || precision_ == ASEP_PREC_FP16 || is_tcx(); }   // tcgen05 modes
   DeviceArena arena_;
   Work work_;
   float* score_buf_ = nullptr;

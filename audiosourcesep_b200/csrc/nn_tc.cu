@@ -467,6 +467,8 @@ bool run_tc(TCParams prm, cudaStream_t s) {   // returns true when G was written
     ASEP_CHECK(prm.k1_panels * kPanelBytes + ((kTileM * prm.n3p * 4 + 1023) & ~1023) <= kARegionBytes, ASEP_ERR_UNSUPPORTED,
                "coupling network shape outside the tcgen05 kernel (stage-1 panels %d, stage-3 columns %d)", prm.k1_panels, prm.n3p);
     ASEP_CHECK(prm.M < (1ll << 31), ASEP_ERR_UNSUPPORTED, "more than 2^31 pixels in one coupling-network launch");
+    ASEP_CHECK(stage1_width_supported(prm.src_ch, kBwd), ASEP_ERR_UNSUPPORTED,
+               "coupling network input width %d outside the tcgen05 kernel", prm.src_ch);
     const long long tiles = (prm.M + kTileM - 1) / kTileM;
     const int grid = (int)std::min<long long>(tiles, g_num_sms);
     prm.tiles_per_cta_round = grid;

@@ -9,6 +9,10 @@ namespace asep {
 
 constexpr int kTcF = 512;   // hidden width the tcgen05 kernel is built for (configs/melspec_glow.yml:10)
 
+// Level widths C the tcgen05 coupling kernels are built for: their stage-1 operand builders handle C/2 (forward) and
+// C (data gradient) source channels in {2, 4, 8, 16} only, and the stage-3 outputs of C = 32 do not fit the staging area.
+inline bool nn_tc_supported(int C) { return C == 4 || C == 8 || C == 16; }
+
 struct TCStageSet {
   __nv_bfloat16* img = nullptr;  // weight tile images in consumption order (device)
   int k1_steps = 0;              // K=16 MMA steps of stage 1

@@ -48,6 +48,12 @@ struct TCParams {
   int num_rounds;
 };
 
+// source widths the stage-1 operand builders are instantiated for: the register path takes <= 8 channels (1, 2, 4, 8;
+// any other width would be built as 4), the rebuild path 16 (data gradient of C = 16 only)
+inline bool stage1_width_supported(int src_ch, bool bwd) {
+  return src_ch == 1 || src_ch == 2 || src_ch == 4 || src_ch == 8 || (bwd && src_ch == 16);
+}
+
 // byte offset of element (row, k) inside the 128-row A region made of 64-wide SWIZZLE_128B panels
 __device__ __forceinline__ uint32_t a_offset(int row, int k) {
   return (uint32_t)((k >> 6) * kPanelBytes + row * 128 + ((((k & 63) >> 3) ^ (row & 7)) << 4) + ((k & 7) << 1));

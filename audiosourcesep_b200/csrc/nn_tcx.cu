@@ -439,7 +439,7 @@ void run_tcx(TCParams prm, double flops, cudaStream_t s) {
   prm.tiles_per_cta_round = grid;
   prm.num_rounds = (int)((tiles + grid - 1) / grid);
   prm.part_stride = tiles * kTileM * (long long)prm.n3p;
-  ASEP_CHECK(prm.src_ch == 1 || prm.src_ch == 2 || prm.src_ch == 4 || prm.src_ch == 8 || (kBwd && prm.src_ch == 16), ASEP_ERR_UNSUPPORTED,
+  ASEP_CHECK(stage1_width_supported(prm.src_ch, kBwd), ASEP_ERR_UNSUPPORTED,
              "coupling network input width %d outside the tcgen05 kernel", prm.src_ch);
   if constexpr (kBwd) {
     if (prm.src_ch <= 8) launch_tcx<true, false, false, true>(prm, grid, flops, s);

@@ -281,3 +281,23 @@ def conv_wgrad_tc(x, g, dk: torch.Tensor, ksize: int, dil: int = 1) -> torch.Ten
     t = [_lib.dl(v) for v in (x, g, dk)]
     _lib.check(_lib.load().asep_conv_wgrad_tc(t[0].ptr, t[1].ptr, t[2].ptr, int(ksize), int(dil), _lib.stream_ptr()))
     return dk
+
+
+# ---- the tcgen05 coupling network of the Glow prior one launch at a time (tests compare each with a float64 reference)
+def glow_coupling_tc(glow, block: int, step: int, backward: bool, src, G, mask1=None, mask2=None, dump1=None, dump2=None,
+                     out=None) -> None:
+    """One ``k_nn_tc4`` / ``k_nn_tcx`` launch with the prepared weights of (block, step) of ``glow`` (a ``Glow`` in a
+    tensor-core precision), on caller tensors that are passed as they are: the library checks every one before the
+    launch (layouts in include/asep.h).  src fp32 [N,Hb,Wb,Cb]; G fp32 [nparts, ceil(M/128)*128*n3p]; mask1 / mask2 int32
+    [M,16] (outputs of the forward, inputs of the backward); dump1 / dump2 bf16 [M,512]; out fp32 r [N,Hb,Wb,Cb] or gxb
+    [N,Hb,Wb,Cb/2]."""
+    t = [_lib.dl(v) for v in (src, mask1, mask2, dump1, dump2, G, out)]
+    _lib.check(_lib.load().asep_glow_coupling_tc(glow.handle, int(block), int(step), int(backward), t[0].ptr, t[1].ptr,
+                                                 t[2].ptr, t[3].ptr, t[4].ptr, t[5].ptr, t[6].ptr, _lib.stream_ptr()))
+
+
+def glow_wgrad_tc(A, B, n_valid: int, out) -> None:
+    """One ``k_wgrad_tc`` launch: ``out`` fp32 [512, ldo] += A^T B for the columns < n_valid, A bf16 [P,512], B bf16
+    [P,ldb] (passed as they are; the library checks them)."""
+    t = [_lib.dl(v) for v in (A, B, out)]
+    _lib.check(_lib.load().asep_glow_wgrad_tc(t[0].ptr, t[1].ptr, int(n_valid), t[2].ptr, _lib.stream_ptr()))

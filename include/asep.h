@@ -152,6 +152,24 @@ int asep_glow_coupling_nn(asep_glow_t h, int block, int step, const DLTensor* st
 /* Data gradient of the same network: gr [N,Hb,Wb,Cb] -> gxb [N,Hb,Wb,Cb/2]. */
 int asep_glow_coupling_nn_backward(asep_glow_t h, int block, int step, const DLTensor* state, const DLTensor* gr,
                                    DLTensor* gxb, void* stream);
+/* ---- the tcgen05 coupling network one launch at a time, so each can be tested against a float64 reference.  Every
+ * argument is checked before anything is launched.
+ * asep_glow_coupling_tc: one k_nn_tc4 (ASEP_PREC_BF16 / FP16) or k_nn_tcx (BF16X2 / FP16X2 / FP16X3) launch with the
+ *   prepared weights of (block, step) of a handle prepared in a tensor-core precision (else ASEP_ERR_UNSUPPORTED).
+ *   src float32 [N,Hb,Wb,Cb]: the state (forward; the network reads channels Cb/2..Cb-1) or dL/dr (backward = 1).
+ *   mask1, mask2 int32 [M,16] (M = N*Hb*Wb): the ReLU bit masks of p1 / p2, word ch*8 + panel covering hidden columns
+ *   [64*panel + 32*ch, +32) (bit i = column + i); written by the forward when given (both or neither), read by the
+ *   backward (both required: ASEP_ERR_BAD_ARG).  dump1, dump2 bf16 [M,512] (may be NULL; one-product modes only, else
+ *   ASEP_ERR_UNSUPPORTED): forward relu(p1), relu(p2); backward dL/dp2, dL/dp1.  G float32 [nparts, ceil(M/128)*128*n3p]:
+ *   the per-tap stage-3 outputs, tile by tile [n3p/4][128 rows][4] (nparts = 2 K-split parts in the split-precision
+ *   modes, else 1; n3p = pad16(9*Cb) forward, pad16(9*Cb/2) backward).  out (may be NULL): the col2im of G, r
+ *   [N,Hb,Wb,Cb] (forward) or gxb [N,Hb,Wb,Cb/2] (backward).  Block or step out of range: ASEP_ERR_BAD_ARG.
+ * asep_glow_wgrad_tc: out fp32 [512, ldo] += A^T B over the P rows for columns < n_valid (it accumulates; the others are
+ *   not touched); A bf16 [P,512], B bf16 [P,ldb] with ldb a multiple of 64, and of 256 above 256 (else
+ *   ASEP_ERR_UNSUPPORTED), 1 <= n_valid <= min(ldb, ldo).  The weight-gradient GEMM of the tensor-core training step. */
+int asep_glow_coupling_tc(asep_glow_t h, int block, int step, int backward, const DLTensor* src, DLTensor* mask1,
+                          DLTensor* mask2, DLTensor* dump1, DLTensor* dump2, DLTensor* G, DLTensor* out, void* stream);
+int asep_glow_wgrad_tc(const DLTensor* A, const DLTensor* B, int n_valid, DLTensor* out, void* stream);
 
 /* ------------------------------------------------------------------ BASIS Langevin with K sources, 2 <= K <= 8
  * One fused update of run_basis_sep.py:163-181 for every source (dB mixing, :106-149):
